@@ -98,7 +98,17 @@ def parse_args():
     ap.add_argument("--streams", type=int, default=2, help="sub-swarms per GPU, each advanced on its own CUDA stream (multidronesim_b200.SwarmStreams): "
                                                            "the tail wave of one sub-swarm's launch is filled by the next launch of another; 1 = one launch per step")
     ap.add_argument("--dtype", default="f32", choices=["f32", "f64"])
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to DIR/<name>.npy: obs_log.npy = "
+                                                          "the observation after each control step of that launch [T, n, 8, 20] for a fixed, seeded "
+                                                          "sample of n <= 2048 of (rank 0's) environments in ascending order (T = fuse unless the log "
+                                                          "of one environment exceeds the 48 MB budget; then its last T steps), rollout_stats.npy = "
+                                                          "the statistics of the timed steps (MDS_STAT_*, float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
+    return args
 
 
 # ----------------------------------------------------------------------------------------------
@@ -338,6 +348,27 @@ def fp_peak(mds, sms, clocks, use_f64):
                                         f"microbenchmark read {measured:.1f} TFLOP/s, below 95 % of it)")
 
 
+DUMP_ENVS, DUMP_BYTES = 2048, 48 << 20  # --dump-outputs: environments sampled from the swarm, and the byte budget of their observation log
+
+
+def dump_outputs(out_dir, rings, stats):
+    """--dump-outputs: the observation log of the last launch (``rings``: one [F, E_p, N, 20] tensor per sub-swarm, in env order) for a
+    sample of environments drawn with a fixed seed, so that the same arguments select the same environments in every run, and the
+    statistics of the timed steps"""
+    import numpy as np
+    import torch
+    F, _, N, C = rings[0].shape
+    offsets = np.cumsum([0] + [r.shape[1] for r in rings])
+    slot_bytes = N * C * rings[0].element_size()
+    T = min(F, DUMP_BYTES // slot_bytes)  # the last T control steps of one environment fit the budget (all of them unless F is huge)
+    n = max(1, min(int(offsets[-1]), DUMP_ENVS, DUMP_BYTES // (T * slot_bytes)))
+    envs = np.sort(np.random.default_rng(0).choice(int(offsets[-1]), n, replace=False))
+    parts = [r[F - T:, torch.as_tensor(envs[(envs >= b0) & (envs < b1)] - b0, device=r.device)] for r, b0, b1 in zip(rings, offsets[:-1], offsets[1:])]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "obs_log.npy"), torch.cat(parts, dim=1).cpu().numpy())
+    np.save(os.path.join(out_dir, "rollout_stats.npy"), stats.cpu().numpy())
+
+
 def time_launches(torch, fn, reps, swarm=None):
     """CUDA-event time of ``reps`` calls of ``fn`` on the current stream; with ``swarm`` (SwarmStreams) the sub-swarm streams are
     forked after the first event and joined before the second, as in the headline's timed region"""
@@ -392,10 +423,10 @@ def run_gpu_arm(args):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    def timed_swarm(n_envs, env_offset, clk=None):
+    def timed_swarm(n_envs, env_offset, clk=None, dump_dir=None):
         """settle + warm up + time K bench steps of an n_envs-environment swarm cut into P_STREAMS sub-swarms; every control step's
         observation is materialised in HBM (per sub-swarm a ring of F log slots, reused by each launch), as the reference's loop
-        does (observations.append(obs)): a drone-step includes its 80 B observation write"""
+        does (observations.append(obs)): a drone-step includes its 80 B observation write.  ``dump_dir``: dump_outputs() after timing"""
         swarm, subs = scenarios.cbf_swarm_streams(n_envs, P_STREAMS, N, order=CBF_ORDER, dtype=dtype, device=dev, env_offset=env_offset)
         rings = [torch.empty(F, s_["env"].NUM_ENVS, N, 20, device=dev, dtype=dtype) for s_ in subs]
         step = lambda: swarm.run(F, obs_logs=rings, log_every=1)
@@ -416,6 +447,8 @@ def run_gpu_arm(args):
         e1.record(cur)
         torch.cuda.synchronize()
         w1 = time.perf_counter()
+        if dump_dir:
+            dump_outputs(dump_dir, rings, swarm.stats())
         barrier()
         if not all(r.plan() == 6 for r in swarm.rollouts):
             raise SystemExit("bench.py assumes the K-steps-in-one-launch plan")
@@ -423,7 +456,7 @@ def run_gpu_arm(args):
 
     # ---- device-resident headline -------------------------------------------------------------
     with ClockSampler(local_rank) as clk:  # sampling starts with the settle phase: nvidia-smi needs ~0.2 s to deliver its first line
-        ms, t_wall0, t_wall1, stats_rank = timed_swarm(E, rank * E)
+        ms, t_wall0, t_wall1, stats_rank = timed_swarm(E, rank * E, dump_dir=args.dump_outputs if rank == 0 else None)
         time.sleep(0.12)  # let the sample that covers the end of the region arrive
     ms_max = max_over_ranks(ms)
     value = world * D * F * K / (ms_max * 1e-3)

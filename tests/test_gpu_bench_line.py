@@ -5,7 +5,10 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
+
+from multidronesim_b200._lib import STAT_NAMES
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REQUIRED = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline", "dtype", "data",
@@ -21,8 +24,12 @@ def run(args):
 
 
 @pytest.mark.gpu
-def test_gpu_arm_line():
-    d = run(["--envs", "2048", "--steps", "3", "--warmup", "3", "--fuse", "8", "--settle", "16", "--e2e-steps", "4", "--cpu-seconds", "1"])
+def test_gpu_arm_line(tmp_path):
+    d = run(["--envs", "2048", "--steps", "3", "--warmup", "3", "--fuse", "8", "--settle", "16", "--e2e-steps", "4", "--cpu-seconds", "1",
+             "--dump-outputs", str(tmp_path)])
+    obs_log, st = np.load(tmp_path / "obs_log.npy"), np.load(tmp_path / "rollout_stats.npy")
+    assert obs_log.shape == (8, 2048, 8, 20) and obs_log.dtype == np.float32 and np.isfinite(obs_log).all()   # every env fits the sample
+    assert st.dtype == np.float64 and st.tolist() == [d["rollout_stats"][k] for k in STAT_NAMES]
     assert REQUIRED <= set(d), REQUIRED - set(d)
     assert d["value"] > 0 and d["n_gpus"] == 1 and d["steps"] == 3 and d["gpu_launches"] == 3 * 2 and d["dtype"] == "f32"   # two sub-swarm streams, one launch each per step
     assert d["rollout_stats"]["drone_steps"] == 2048 * 8 * 8 * 3
@@ -45,6 +52,28 @@ def test_gpu_arm_line():
     assert set(cf) == {"C2_4096", "C3_o2_16384", "C4_65536_f64", "C5_f64"}
     for k, v in cf.items():
         assert v["value"] > 0 and 0 < v["roofline"]["frac"] < 1.5 and "clocks" in v, k
+
+
+def test_dump_outputs_samples_and_crops(monkeypatch, tmp_path):
+    """bench.dump_outputs on host tensors: a seeded sample of environments drawn across two sub-swarm logs, and the last
+    control steps only when one environment's log exceeds the byte budget"""
+    import torch
+    import bench
+    F, sizes = 6, (9, 14)
+    rings = [torch.randn(F, e, 8, 20, generator=torch.Generator().manual_seed(p)) for p, e in enumerate(sizes)]
+    whole = torch.cat(rings, dim=1).numpy()
+    stats = torch.arange(8, dtype=torch.float64)
+    slot = 8 * 20 * 4
+    for n_envs, budget, T in ((5, 1 << 20, F), (23, 1 << 20, F), (4, 4 * slot, 4)):
+        monkeypatch.setattr(bench, "DUMP_ENVS", n_envs)
+        monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+        bench.dump_outputs(str(tmp_path), rings, stats)
+        n = min(n_envs, budget // (T * slot))
+        envs = np.sort(np.random.default_rng(0).choice(sum(sizes), n, replace=False))
+        got = np.load(tmp_path / "obs_log.npy")
+        assert got.shape == (T, n, 8, 20) and np.array_equal(got, whole[F - T:, envs]), (n_envs, budget)
+        assert np.array_equal(np.load(tmp_path / "rollout_stats.npy"), stats.numpy())
+        assert n == 1 or ((envs < sizes[0]).any() and (envs >= sizes[0]).any())   # the sample spans both sub-swarms
 
 
 def test_reference_arm_line():

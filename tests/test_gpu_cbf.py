@@ -120,7 +120,7 @@ def test_anchor_and_status_codes(lib_built):
 
 
 @pytest.mark.parametrize("order,dtype,tol", [(2, torch.float64, 1e-9), (3, torch.float64, 1e-9), (3, torch.float32, 1e-4)])
-def test_cylinder_obstacles_vs_oracle(golden, order, dtype, tol, lib_built):
+def test_cylinder_obstacles_vs_oracle(golden, order, dtype, tol, lib_built, tmp_path):
     """Builder extension (the reference has spheres only; parity unpinned): a sphere and a vertical cylinder
     (obstacles.Cylinder -> negative radius) in one obstacle set; device rows and QP answers against oracle/cbf.py."""
     import multidronesim_b200 as mds
@@ -154,7 +154,7 @@ def test_cylinder_obstacles_vs_oracle(golden, order, dtype, tol, lib_built):
     assert solved >= (1 if order == 2 else 2)   # order-2 rows vanish at ez = 0: most random order-2 cases are infeasible
     import os
     from multidronesim_b200.obstacles import generate_cylinder
-    path = generate_cylinder(0.15, 3.0)
+    path = generate_cylinder(0.15, 3.0, folder=str(tmp_path))
     assert os.path.isfile(path) and 'cylinder radius="0.15" length="3.0"' in open(path).read()
 
 

@@ -117,20 +117,16 @@ def test_cf2x_needs_the_x_frame_mixer():
 # What the reference tree DOES hold about the env step: its continuous rigid-body model (model/dynamics.py:83-106) and its
 # hover linearisation (model/linearized.py:52-79).  Upstream's explicit DYN update (restated in oracle/aviary.py from the
 # published algorithm; gym-pybullet-drones itself is absent) must be a first-order integrator OF that model: its difference
-# quotients converge to dynamics() as dt -> 0, and their Jacobian at hover is (A, B).  Skipped where the reference's
-# packages cannot be imported.
+# quotients converge to dynamics() as dt -> 0, and their Jacobian at hover is (A, B).  What the reference's model
+# computes comes from tests/golden/models.npz (oracle/make_golden.golden_models, run on the reference's own classes).
 # ---------------------------------------------------------------------------------------------------------------
-def _reference_or_skip():
-    from oracle import ref_pipeline
-    if ref_pipeline.reference_root() is None:
-        pytest.skip("reference packages not available (python -m oracle.build_ref)")
-    return ref_pipeline.load_reference()
-
-
-def _fd_xdot(model, pos, quat, vel, w_body, rpm, dt_hz):
-    """((v_new - v) / dt, (w_new - w) / dt, (p_new - p) / dt, R(q_new), R(q)) of ONE explicit Physics.DYN update at 1 / dt_hz"""
+def _fd_xdot(model, pos, quat, vel, w_body, rpm, dt_hz, J=None):
+    """((v_new - v) / dt, (w_new - w) / dt, (p_new - p) / dt, R(q_new), R(q)) of ONE explicit Physics.DYN update at 1 / dt_hz,
+    with the inertia ``J`` in place of the drone model's if given"""
     from oracle.aviary import quat_to_matrix
     env = OracleCtrlAviary(model, 1, physics=Physics.DYN, pyb_freq=dt_hz, ctrl_freq=dt_hz)
+    if J is not None:
+        env.J, env.J_INV = np.array(J, float), np.linalg.inv(J)
     env.set_state(pos, quat, vel, w_body, last_rpm=rpm)
     R0 = quat_to_matrix(env.quat[0])
     env.step(np.asarray(rpm, float).reshape(1, 4))
@@ -139,49 +135,38 @@ def _fd_xdot(model, pos, quat, vel, w_body, rpm, dt_hz):
 
 
 @pytest.mark.parametrize("model", [DroneModel.CF2P])
-def test_dyn_step_converges_to_the_reference_dynamics(model):
+def test_dyn_step_converges_to_the_reference_dynamics(golden, model):
     """(state(t + dt) - state(t)) / dt of the restated Physics.DYN step -> QuadrotorDynamics.dynamics (model/dynamics.py:83-106,
-    with the env's mass / inertia injected and inputs from the reference's own action_to_input) as dt -> 0: first-order
-    convergence at random states, to 1e-6 relative at dt = 1e-7 s."""
-    ref = _reference_or_skip()
-    from scipy.spatial.transform import Rotation
-    rng = np.random.default_rng(5)
-    env = OracleCtrlAviary(model, 1, physics=Physics.DYN)
-    qd = ref.model.QuadrotorDynamics(240)
-    qd.load_env_params(env)
-    qd.J = np.array(env.J, float)           # load_env_params keeps the Hummingbird inertia (quirk B22): inject the env's
-    qd.J_inv = np.linalg.inv(qd.J)
-    worst = {}
-    for trial in range(12):
-        rpy = rng.uniform(-0.6, 0.6, 3)
-        quat = Rotation.from_euler("xyz", rpy).as_quat()
-        pos, vel, w = rng.uniform(-1, 1, 3) + [0, 0, 2], rng.normal(0, 1, 3), rng.normal(0, 2, 3)
-        rpm = rng.uniform(9440.3, env.MAX_RPM, 4)
-        u = ref.conv.action_to_input(env, rpm.copy())                    # PLUS-frame mixer == the CF2P allocation of the DYN update
-        R = Rotation.from_quat(quat).as_matrix()
-        want = qd.dynamics(0.0, np.hstack([pos, R.flatten(), vel, w]), u)  # (x_dot, w, v_dot, w_dot)
+    inputs from the reference's own action_to_input) as dt -> 0: first-order convergence at the 128 stored random states, to
+    1e-6 relative at dt = 1e-7 s.  The stored xdot was computed with the inertia load_env_params leaves in place (the Hummingbird's,
+    quirk B22), so the env step runs with that inertia here."""
+    g = golden["models"]
+    J = np.diag(g["J_dynamics"])
+    for k, (o, want) in enumerate(zip(g["obs"], g["xdot_nonlinear"])):
+        # stored in linear order (w, w_dot, v_dot, x_dot) (utils/model_conversions.py:124-135), with obs[13:16] as the body rates;
+        # the DYN update does not depend on position, so every state is lifted 3 m to keep it clear of the ground
+        pos, quat, vel, w, rpm = o[0:3] + [0, 0, 3], o[3:7], o[10:13], o[13:16], o[16:20]
         errs = []
         for hz in (1e4, 1e5, 1e6, 1e7):
-            vdot, wdot, pdot, R1, R0 = _fd_xdot(model, pos, quat, vel, w, rpm, hz)
-            scale = 1.0 + np.abs(want[6:12]).max()
-            e = max(np.abs(vdot - want[6:9]).max(), np.abs(wdot - want[9:12]).max()) / scale
+            vdot, wdot, pdot, R1, R0 = _fd_xdot(model, pos, quat, vel, w, rpm, hz, J=J)
+            scale = 1.0 + np.abs(want[3:9]).max()
+            e = max(np.abs(vdot - want[6:9]).max(), np.abs(wdot - want[3:6]).max()) / scale
             # position uses the NEW velocity (semi-implicit): p_dot -> v; attitude: (R1 - R0) / dt -> R hat(w)
-            e = max(e, np.abs(pdot - want[0:3]).max() / (1 + np.abs(vel).max()))
-            Rdot = R0 @ qd.hat_map(w)
+            e = max(e, np.abs(pdot - want[9:12]).max() / (1 + np.abs(vel).max()))
+            Rdot = R0 @ np.array([[0, -w[2], w[1]], [w[2], 0, -w[0]], [-w[1], w[0], 0]])
             e = max(e, np.abs((R1 - R0) * hz - Rdot).max() / (1 + np.abs(Rdot).max()))
             errs.append(e)
-        worst[trial] = errs
-        assert errs[-1] < 1e-5, (trial, errs)
-        assert errs[1] < 0.2 * errs[0] + 1e-9 and errs[2] < 0.2 * errs[1] + 1e-9, (trial, errs)   # O(dt)
+        assert errs[-1] < 1e-5, (k, errs)
+        assert errs[1] < 0.2 * errs[0] + 1e-9 and errs[2] < 0.2 * errs[1] + 1e-9, (k, errs)   # O(dt)
 
 
-def test_dyn_step_hover_jacobian_is_the_reference_linear_model():
+def test_dyn_step_hover_jacobian_is_the_reference_linear_model(golden):
     """Jacobian of the DYN difference quotient at hover, in the reference's linear-model coordinates x = [rpy, w, v, p],
-    u = [f, tau] (utils/model_conversions.py:20-58,69-83), equals LinearizedModel's A and B (model/linearized.py:52-79)."""
-    ref = _reference_or_skip()
+    u = [f, tau] (utils/model_conversions.py:20-58,69-83), equals LinearizedModel's A and B (model/linearized.py:52-79), as
+    stored for the CF2P in tests/golden/models.npz."""
     from scipy.spatial.transform import Rotation
     env = OracleCtrlAviary(DroneModel.CF2P, 1, physics=Physics.DYN)
-    lin = ref.model.LinearizedModel(env)
+    A_ref, B_ref = golden["models"]["torque12_A"], golden["models"]["torque12_B"]
     hz, eps = 1e7, 1e-4
     mixer = np.array([[1, 1, 1, 1], [0, env.L, 0, -env.L], [-env.L, 0, env.L, 0], [-env.KM / env.KF, env.KM / env.KF, -env.KM / env.KF, env.KM / env.KF]])
 
@@ -201,5 +186,5 @@ def test_dyn_step_hover_jacobian_is_the_reference_linear_model():
     A = np.array([(xdot(x0 + eps * np.eye(12)[k], u0) - xdot(x0 - eps * np.eye(12)[k], u0)) / (2 * eps) for k in range(12)]).T
     du = np.array([1e-3 * env.M * env.G, 1e-6, 1e-6, 1e-7])
     B = np.array([(xdot(x0, u0 + du[k] * np.eye(4)[k]) - xdot(x0, u0 - du[k] * np.eye(4)[k])) / (2 * du[k]) for k in range(4)]).T
-    assert np.abs(A - lin.A).max() < 1e-5 * (1 + np.abs(lin.A).max()), np.abs(A - lin.A).max()
-    assert np.abs(B - lin.B).max() < 1e-5 * (1 + np.abs(lin.B).max()), np.abs((B - lin.B) / (1 + np.abs(lin.B))).max()
+    assert np.abs(A - A_ref).max() < 1e-5 * (1 + np.abs(A_ref).max()), np.abs(A - A_ref).max()
+    assert np.abs(B - B_ref).max() < 1e-5 * (1 + np.abs(B_ref).max()), np.abs((B - B_ref) / (1 + np.abs(B_ref))).max()
