@@ -180,6 +180,10 @@ typedef struct MdsRolloutCfg {
   double obstacles[MDS_MAX_OBSTACLES * 4]; /* cx, cy, cz, r (r < 0: vertical cylinder of radius |r|) */
   const void* lqr_gain_planes_dev; /* optional, LQR controllers: a gain per drone, [4*dim][D] planes of Real (DecentralizedLQR*.K,
                                       simulations/CBFTest.py:319-321 `--controller dlqr`); NULL = MdsLqrGains.K for every drone */
+  int traj_period;     /* 0 = one trajectory descriptor per drone (no assumption); N (the drone count) = every environment flies
+                          the references of environment 0: specs_dev[d] equals specs_dev[d mod N] for every drone d.  The caller
+                          guarantees it; plan 6 then evaluates each reference once per block and step instead of once per drone
+                          (fp32, N = 8, LQR_OMEGA / LQR_YANK; the results are the same bits) */
 } MdsRolloutCfg;
 
 /* ---- library ------------------------------------------------------------------ */

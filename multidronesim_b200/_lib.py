@@ -80,7 +80,7 @@ class RlsCfg(C.Structure):
 class RolloutCfg(C.Structure):
     _fields_ = [("ctrl", C.c_int), ("use_cbf", C.c_int), ("num_obstacles", C.c_int),
                 ("write_obs_every", C.c_int), ("stages", C.c_int), ("obstacles", C.c_double * (MAX_OBSTACLES * 4)),
-                ("lqr_gain_planes_dev", C.c_void_p)]
+                ("lqr_gain_planes_dev", C.c_void_p), ("traj_period", C.c_int)]
 
 
 # numpy dtypes of the device-side trajectory tables (must match the C structs)

@@ -738,6 +738,7 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   }
   MDS_REQUIRE(!(cfg->write_obs_every > 0) || obs_log, "rollout: obs_log buffer missing");
   MDS_REQUIRE(cfg->write_obs_every <= 32767, "rollout: write_obs_every must be <= 32767");
+  MDS_REQUIRE(cfg->traj_period == 0 || cfg->traj_period == N, "rollout: traj_period must be 0 or the drone count N");
   const int NP = next_pow2(N), threads = R.use_cbf ? cbf_block_threads<Real>(NP, N, R.n_obs) : MDS_BLOCK, epb = threads / NP;
   const int blocks = (E + epb - 1) / epb;
   size_t smem = R.use_cbf ? cbf_smem_bytes<Real>(threads, NP, N, R.n_obs) : 32;
@@ -759,7 +760,8 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
     return obs;
   };
   cudaError_t attr_err = cudaSuccess;
-  RolloutLaunch<Real> RL{Pd, R, G, L, C, Dg, Ds, Sd, Pi, specs, segs, action, fext, obs, obs_log, stats, E, N, NP, blocks, threads, phys_spec_of(*prm), smem, cs};
+  RolloutLaunch<Real> RL{Pd, R, G, L, C, Dg, Ds, Sd, Pi, specs, segs, action, fext, obs, obs_log, stats, E, N, NP, blocks, threads, phys_spec_of(*prm), smem, cs,
+                         cfg->traj_period};
   auto keep = [&](cudaError_t e) { if (e != cudaSuccess) attr_err = e; };
   // the loop kernel packs two rare-event counters into 16 bits each: longer runs go out as several launches (whole log periods each)
   auto launch_loop = [&]() {

@@ -562,18 +562,22 @@ struct StepStats {
 // instruction cache: 55 % of the stall samples were "no instruction").
 // PDK: a gain per drone (Rc.lqr_planes) instead of LqrP's; SPEC: compile-time parameter switches (PhysSpec); R_out (optional)
 // receives the rotation matrix of the observation's attitude when the inner loop built it (HAS_PID controllers).
-template <typename Real, int CTRL, bool USE_CBF, bool PDK = false, int SPEC = 0, int NT = 0>
+// REFTAB: the reference is read from ref_slot (a slot of rollout_loop_kernel's reference table) instead of evaluated from
+// (spec, segs, t), which are then unused.
+template <typename Real, int CTRL, bool USE_CBF, bool PDK = false, int SPEC = 0, int NT = 0, bool REFTAB = false>
 MDS_DEV void ctrl_body(const DroneP<Real>& P, const RolloutP<Real>& Rc, const GeoP<Real>& G, const LqrP<Real>& L, const CbfP<Real>& C,
                        const DslP<Real>& Dg, const DslStateP<Real>& dst, const CbfSmem<Real>& S, const PidP<Real>& pid,
                        const typename TrajSpecT<Real>::spec& spec,
                        const typename TrajSpecT<Real>::seg* __restrict__ segs, const Obs<Real>& o, const GroupMap& g, int N, int NP,
-                       double t, Real rpm[4], StepStats& ss, int pid_idx, M3<Real>* R_out = nullptr) {
+                       double t, Real rpm[4], StepStats& ss, int pid_idx, M3<Real>* R_out = nullptr,
+                       const typename Vec4T<Real>::type* ref_slot = nullptr) {
   constexpr bool HAS_PID = (CTRL == MDS_CTRL_LQR_OMEGA || CTRL == MDS_CTRL_LQR_YANK);
   constexpr int ORD = CTRL == MDS_CTRL_LQR_OMEGA ? 2 : 3;  // rollout_impl pairs the order-2 filter with LQR_OMEGA, order 3 with LQR_YANK
   Real u[4] = {Real(0), Real(0), Real(0), Real(0)};
   Ref<Real> ref;
   if (g.valid) {
-    ref = eval_traj<Real>(spec, segs, t);
+    if constexpr (REFTAB) ref = load_ref<Real>(ref_slot);
+    else ref = eval_traj<Real>(spec, segs, t);
     ss.err = (float)norm(o.p - ref.p);
     if (CTRL == MDS_CTRL_GEOMETRIC) {
       geometric_input(P, G, o, ref, u);
@@ -766,13 +770,38 @@ __global__ void __launch_bounds__(MDS_BLOCK, sizeof(Real) == 4 ? MDS_FUSED_MINB 
   if (stats) stats_block_reduce<USE_CBF>(stats, g.valid ? 1 : 0, ss, ss.err);
 }
 
+// Reference table of rollout_loop_kernel<..., REFTAB = true>: the references of MDS_REF_STEPS consecutive control steps for
+// the NT drones of an environment, slot (j, n) = 3 words at 3 (j NT + n).  A power of two (the step loop picks the row by a
+// mask); 32 steps x 8 drones = 12 KB in fp32.
+#ifndef MDS_REF_STEPS
+#define MDS_REF_STEPS 32
+#endif
+// Fills rows [0, steps) with the references of steps k0 + j of drones [0, NT) of environment 0 -- of every environment when the
+// trajectory set repeats with period NT -- one slot per thread of the block.  The time is formed exactly as the per-drone path
+// forms it (t0 + (double)k * dt_ctrl), so the slots hold the same bits as eval_traj there.  Out of line: the fp64 time and
+// phase arithmetic stays out of the step loop's instruction stream.
+template <typename Real, int NT>
+__device__ __noinline__ void build_ref_table(typename Vec4T<Real>::type* tab, const typename TrajSpecT<Real>::spec* __restrict__ specs,
+                                             const typename TrajSpecT<Real>::seg* __restrict__ segs, double t0, double dt_ctrl, int k0, int steps) {
+  for (int i = threadIdx.x; i < steps * NT; i += blockDim.x) {
+    const int j = i / NT, n = i - j * NT;
+    const typename TrajSpecT<Real>::spec sp = specs[n];
+    store_ref<Real>(tab + 3 * i, eval_traj<Real>(sp, segs, t0 + (double)(k0 + j) * dt_ctrl));
+  }
+}
+
 // K control steps in ONE launch.  Environments never interact, and everything that couples the drones of an
 // environment (downwash, CBF rows, QP) is exchanged inside its lane group, so a group can run its env forward on its
 // own: the observation and the body rates stay in registers from step to step, HBM sees the initial load, the log slots
 // that are due and the final store.  No launch per step, no grid-wide barrier.
 // SPEC: compile-time parameter switches (PhysSpec); K <= 32767 (rollout_impl splits longer runs): the rare-event counters
 // share one register.
-template <typename Real, int CTRL, bool USE_CBF, int NT, int SPEC>
+// REFTAB (fp32, compile-time N, rate-PID controllers; the host selects it when every environment flies the same N references,
+// MdsRolloutCfg.traj_period): the block evaluates the references of the next MDS_REF_STEPS steps once into a shared-memory
+// table and the lanes read their slot, instead of every lane evaluating its own drone's reference every step (fp64 time and
+// phase, sincos, a 48-byte descriptor staged per thread).  The table is refilled every MDS_REF_STEPS steps between two block
+// barriers; K <= MDS_REF_STEPS (the swarm workloads' 24-step launches) fills it once, before the loop.
+template <typename Real, int CTRL, bool USE_CBF, int NT, int SPEC, bool REFTAB = false>
 __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loop_kernel(DroneP<Real> P, RolloutP<Real> Rc, GeoP<Real> G, LqrP<Real> L, CbfP<Real> C,
                                                                   DslP<Real> Dg, DslStateP<Real> dst, StateP<Real> st, PidP<Real> pid,
                                                                   const typename TrajSpecT<Real>::spec* __restrict__ specs,
@@ -789,7 +818,8 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
   // fp32 stages the per-step read-mostly data (trajectory descriptor, rate-PID state) in shared memory for the launch;
   // fp64 does not: with the CBF stage's 91 KB that would leave one resident block per SM instead of two (0.41 vs 0.31 ms)
   constexpr bool STAGE = sizeof(Real) == 4;
-  __shared__ __align__(16) typename TrajSpecT<Real>::spec sm_spec[STAGE ? loop_block<Real>() : 1];
+  __shared__ __align__(16) typename TrajSpecT<Real>::spec sm_spec[(STAGE && !REFTAB) ? loop_block<Real>() : 1];
+  __shared__ R4 sm_ref[REFTAB ? 3 * MDS_REF_STEPS * NT : 1];
   constexpr bool HAS_PID = (CTRL == MDS_CTRL_LQR_OMEGA || CTRL == MDS_CTRL_LQR_YANK);
   __shared__ R4 sm_pid_a[(STAGE && HAS_PID) ? loop_block<Real>() : 1];
   __shared__ typename Vec2T<Real>::type sm_pid_b[(STAGE && HAS_PID) ? loop_block<Real>() : 1];
@@ -810,10 +840,13 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
 #else
   constexpr bool FULLW = false;
 #endif
+  static_assert(!REFTAB || (FULLW && NT * MDS_REF_STEPS <= 8 * 32 && (MDS_REF_STEPS & (MDS_REF_STEPS - 1)) == 0),
+                "the reference table needs the full-warp instantiation and at most 12 KB of shared memory");
   const bool live = g.env_valid;
   if (FULLW) {
     const int first_env = g.e - (int)((threadIdx.x & 31) / NP);  // lane group 0 of this warp
-    g.env_valid = first_env < E;
+    // REFTAB: warps past the last environment re-run it too, so that every warp of the block reaches the table's barriers
+    g.env_valid = REFTAB || first_env < E;
     if (g.env_valid && !live) { g.e = E - 1; g.d = g.e * N + g.n; }
     g.cmask = 0xffffffffu;
   }
@@ -825,26 +858,39 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
     // automatic it would live in local memory (LDL, L1-missing under this kernel's local footprint): stage it in
     // shared memory instead (12-word lane stride: 128-bit reads are conflict-free per quarter warp).
     typename TrajSpecT<Real>::spec spec_reg;
-    typename TrajSpecT<Real>::spec& spec = STAGE ? sm_spec[threadIdx.x] : spec_reg;
+    typename TrajSpecT<Real>::spec& spec = (STAGE && !REFTAB) ? sm_spec[threadIdx.x] : spec_reg;
     spec.kind = MDS_TRAJ_WAIT;
     V3<Real> fx_reg = {Real(0), Real(0), Real(0)};  // constant world-frame force on this drone (wind), if any
     const bool has_fx = fext != nullptr;
     if (g.valid) {
       o = load_obs(obs, g.d);
-      spec = specs[g.d];
+      if (!REFTAB) spec = specs[g.d];
       wb = {st.pos_wx[g.d].w, st.vel_wy[g.d].w, st.wz[g.d]};
       if (has_fx && !STAGE) fx_reg = {fext[3 * g.d], fext[3 * g.d + 1], fext[3 * g.d + 2]};
       if (STAGE && HAS_PID) { sm_pid_a[threadIdx.x] = pid.a[g.d]; sm_pid_b[threadIdx.x] = pid.b[g.d]; }
+    }
+    if constexpr (REFTAB) {
+      build_ref_table<Real, NT>(sm_ref, specs, segs, t0, dt_ctrl, 0, min(K, MDS_REF_STEPS));
+      __syncthreads();
     }
     Real rpm[4] = {Real(0), Real(0), Real(0), Real(0)};
     const size_t obs_elems = (size_t)E * N * MDS_OBS_DIM;
     int log_countdown = Rc.write_obs_every;  // steps until the next log slot is due (no division in the loop)
     Real* log_slot = obs_log;
     for (int k = 0; k < K; ++k) {
+      const int row = k & (MDS_REF_STEPS - 1);
+      if constexpr (REFTAB) {
+        if (k > 0 && row == 0) {  // every lane has read the table's last row
+          __syncthreads();
+          build_ref_table<Real, NT>(sm_ref, specs, segs, t0, dt_ctrl, k, min(K - k, MDS_REF_STEPS));
+          __syncthreads();
+        }
+      }
       StepStats ss = {0.f, 1e30f, 0, 0, 0, 0};
       M3<Real> R;
-      ctrl_body<Real, CTRL, USE_CBF, (NT < 0), SPEC, NT>(P, Rc, G, L, C, Dg, dst, S, pid_s, spec, segs, o, g, N, NP, t0 + (double)k * dt_ctrl, rpm, ss,
-                                                     STAGE ? (int)threadIdx.x : g.d, HAS_PID ? &R : nullptr);  // the host plans form t exactly like this
+      ctrl_body<Real, CTRL, USE_CBF, (NT < 0), SPEC, NT, REFTAB>(P, Rc, G, L, C, Dg, dst, S, pid_s, spec, segs, o, g, N, NP, t0 + (double)k * dt_ctrl,
+                                                             rpm, ss, STAGE ? (int)threadIdx.x : g.d, HAS_PID ? &R : nullptr,  // the host plans form t exactly like this
+                                                             REFTAB ? sm_ref + 3 * (row * NT + g.n) : nullptr);
       acc.err += ss.err; max_err = fmaxf(max_err, ss.err); acc.min_h = fminf(acc.min_h, ss.min_h);
       acc.qp_solves += ss.qp_solves; acc.qp_iters += ss.qp_iters; acc.qp_infeas += ss.qp_infeas + (ss.qp_cap << 16);
       Drone<Real> s;

@@ -26,6 +26,7 @@ template <typename Real> struct RolloutLaunch {
   int spec;  // PhysSpec instantiation the parameter block qualifies for (0 = none: run-time switches)
   size_t smem;
   cudaStream_t cs;
+  int traj_period;  // MdsRolloutCfg.traj_period: 0, or N when every environment flies the references of environment 0
 };
 
 // Each returns the error of the shared-memory opt-in (cudaSuccess when it was not needed); launch errors are

@@ -39,6 +39,11 @@ struct LoopLauncher {
     auto kern = pdk ? rollout_loop_kernel<Real, CT, CB, (PDKC ? -1 : 0), 0>
                     : (a.spec == 1 ? ((a.N == 8) ? rollout_loop_kernel<Real, CT, CB, 8, 1> : rollout_loop_kernel<Real, CT, CB, 0, 1>)
                                    : ((a.N == 8) ? rollout_loop_kernel<Real, CT, CB, 8, 0> : rollout_loop_kernel<Real, CT, CB, 0, 0>));
+    // every environment flies the same 8 references: the instantiation that evaluates them once per block into a table
+    if constexpr (sizeof(Real) == 4 && (CT == MDS_CTRL_LQR_OMEGA || CT == MDS_CTRL_LQR_YANK)) {
+      if (!pdk && a.N == 8 && a.traj_period == 8)
+        kern = a.spec == 1 ? rollout_loop_kernel<Real, CT, CB, 8, 1, true> : rollout_loop_kernel<Real, CT, CB, 8, 0, true>;
+    }
     err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)a.smem);
     kern<<<a.blocks, a.threads, a.smem, a.cs>>>(a.Pd, a.R, a.G, a.L, a.C, a.Dg, a.Ds, a.Sd, a.Pi, a.specs, a.segs, a.action, a.fext, a.obs, a.obs_log,
                                                  a.stats, t0, dt_ctrl, K, a.E, a.N, a.NP);

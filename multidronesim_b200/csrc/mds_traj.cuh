@@ -172,4 +172,20 @@ MDS_DEV Ref<Real> eval_traj(const typename TrajSpecT<Real>::spec& sp, const type
   return eval_traj_table<Real>(table_spec, segs, t);
 }
 
+// A reference sample in three 128-bit words (11 Reals + 1 pad): (p, v.x) (v.y, v.z, a.x, a.y) (a.z, yaw, yaw_rate, -)
+template <typename Real> MDS_DEV void store_ref(typename Vec4T<Real>::type* w, const Ref<Real>& r) {
+  typename Vec4T<Real>::type w0, w1, w2;
+  w0.x = r.p.x; w0.y = r.p.y; w0.z = r.p.z; w0.w = r.v.x;
+  w1.x = r.v.y; w1.y = r.v.z; w1.z = r.a.x; w1.w = r.a.y;
+  w2.x = r.a.z; w2.y = r.yaw; w2.z = r.yaw_rate; w2.w = Real(0);
+  w[0] = w0; w[1] = w1; w[2] = w2;
+}
+template <typename Real> MDS_DEV Ref<Real> load_ref(const typename Vec4T<Real>::type* w) {
+  const typename Vec4T<Real>::type w0 = w[0], w1 = w[1], w2 = w[2];
+  Ref<Real> r;
+  r.p = {w0.x, w0.y, w0.z}; r.v = {w0.w, w1.x, w1.y}; r.a = {w1.z, w1.w, w2.x};
+  r.yaw = w2.y; r.yaw_rate = w2.z;
+  return r;
+}
+
 }  // namespace mds

@@ -18,11 +18,15 @@ from .control.dlqr import _DecentralizedBase
 
 
 class FusedRollout:
-    def __init__(self, env, trajs, controller, qp_tracker=None, obstacles=None):
+    def __init__(self, env, trajs, controller, qp_tracker=None, obstacles=None, ref_table=True):
         """env: BatchedCtrlAviary; trajs: TrajectorySet (one per drone); controller: GeometricControl |
         LQRController | LQROmegaController | LQRYankOmegaController; qp_tracker: DroneQPTracker or None;
-        obstacles: tensor/list [N_obs, 4] = cx, cy, cz, r (shared by all envs)."""
+        obstacles: tensor/list [N_obs, 4] = cx, cy, cz, r (shared by all envs).
+        ref_table: when every environment flies the same trajectories (``trajs.env_period == N``), let the kernel
+        evaluate each reference once per block and step (MdsRolloutCfg.traj_period; same results).  False (or the attribute
+        of the same name) keeps the per-drone evaluation."""
         self.env, self.trajs, self.controller, self.qp = env, trajs, controller, qp_tracker
+        self.ref_table = ref_table
         if trajs.num != env.NUM_TOTAL:
             raise ValueError("need one trajectory per drone")
         cfg = _lib.RolloutCfg()
@@ -86,6 +90,8 @@ class FusedRollout:
         t_call = t0 + env.CTRL_TIMESTEP if stages == 5 else t0  # 5: the controller runs after the physics step
         self.cfg.stages = int(stages)
         self.cfg.write_obs_every = int(log_every) if obs_log is not None else 0
+        N = env.NUM_DRONES
+        self.cfg.traj_period = N if (self.ref_table and self.trajs.env_period == N) else 0
         if obs_log is not None:
             _lib.require_cuda(obs_log, "obs_log", env.dtype)
             if obs_log.numel() < (K // max(1, log_every)) * env.NUM_TOTAL * _lib.OBS_DIM:

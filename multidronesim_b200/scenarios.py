@@ -90,7 +90,7 @@ def cbf_swarm(num_envs, num_drones=8, order=3, dtype=torch.float32, device="cuda
         trk = DroneQPTracker(cbf, order=2, num_robots=N, xdim=9, env=env)
     params = np.zeros((N, 7))
     params[:, 0], params[:, 1], params[:, 2:5], params[:, 5], params[:, 6] = 1.0, omega, center, 0.0, phase
-    trajs = TrajectorySet.from_arrays(_lib.TRAJ_LEMNISCATE, np.tile(params, (E, 1)), device=device, dtype=dtype)
+    trajs = TrajectorySet.from_arrays(_lib.TRAJ_LEMNISCATE, np.tile(params, (E, 1)), device=device, dtype=dtype, drones_per_env=N)
     obstacles = [list(o) for o in SWARM_OBSTACLES] if obstacle else None
     rollout = FusedRollout(env, trajs, ctrl, trk, obstacles)
     return dict(env=env, ctrl=ctrl, cbf=cbf, tracker=trk, trajs=trajs, obstacles=obstacles, rollout=rollout, init=init)

@@ -176,7 +176,11 @@ class RotateTrajectory(TrajectoryBase):
 
 class TrajectorySet:
     """One trajectory per drone, packed for the device.  ``trajs`` is a list of D = E*N
-    descriptions, or N descriptions repeated over ``num_envs`` environments."""
+    descriptions, or N descriptions repeated over ``num_envs`` environments.
+
+    ``env_period`` is N when every environment flies the same N trajectories (descriptor d equals descriptor d mod N), else 0.
+    ``FusedRollout`` passes it to the kernel, which then evaluates each reference once per block instead of once per drone.
+    Assigning ``specs`` clears it; code that edits the ``specs`` tensor in place must set it to 0 itself."""
 
     def __init__(self, trajs, num_envs=1, device="cuda", dtype=torch.float32):
         _lib.load_library()
@@ -211,18 +215,29 @@ class TrajectorySet:
                 seg_arr[k]["rot"][:] = rot
         if num_envs > 1:
             specs = np.tile(specs, num_envs)
-        self._finish(specs, seg_arr)
+        self._finish(specs, seg_arr, n_unique)
 
-    def _finish(self, specs, seg_arr):
+    def _finish(self, specs, seg_arr, env_period):
         self.num = len(specs)
         self.specs = torch.from_numpy(specs.view(np.uint8).copy()).to(self.device)
         self.segs = torch.from_numpy(seg_arr.view(np.uint8).copy()).to(self.device)
         self.ref = torch.zeros(self.num, _lib.REF_DIM, device=self.device, dtype=self.dtype)
+        self.env_period = env_period
+
+    @property
+    def specs(self):
+        return self._specs
+
+    @specs.setter
+    def specs(self, value):
+        self._specs = value
+        self.env_period = 0  # new descriptors are not known to repeat per environment
 
     @classmethod
-    def from_arrays(cls, kind, params, device="cuda", dtype=torch.float32):
+    def from_arrays(cls, kind, params, device="cuda", dtype=torch.float32, drones_per_env=None):
         """Vectorised constructor for large swarms: ``kind`` int or [D] array of MDS_TRAJ_*,
-        ``params`` [D, <=8] (layout of include/mds_b200.h)."""
+        ``params`` [D, <=8] (layout of include/mds_b200.h).  With ``drones_per_env`` = N the descriptors are
+        checked for repeating per environment (``env_period``)."""
         self = cls.__new__(cls)
         _lib.load_library()
         self.device, self.dtype = torch.device(device), dtype
@@ -231,7 +246,11 @@ class TrajectorySet:
         specs = np.zeros(params.shape[0], dtype=_lib.traj_spec_dtype(real))
         specs["kind"] = kind
         specs["p"][:, :params.shape[1]] = params
-        self._finish(specs, np.zeros(1, dtype=_lib.traj_seg_dtype(real)))
+        period = 0
+        if drones_per_env and len(specs) % int(drones_per_env) == 0:
+            envs = specs.view(np.uint8).reshape(len(specs) // int(drones_per_env), -1)  # one row of bytes per environment
+            period = int(drones_per_env) if bool((envs == envs[0]).all()) else 0
+        self._finish(specs, np.zeros(1, dtype=_lib.traj_seg_dtype(real)), period)
         return self
 
     def eval(self, t, out=None):
