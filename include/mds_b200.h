@@ -166,17 +166,11 @@ typedef struct MdsRolloutCfg {
                           0      whole steps, plan chosen by mds_rollout_plan(E, N) (currently always 6)
                           6      all K steps in ONE launch: observation and body rates stay in registers from step to
                                  step (environments are independent and a lane group owns its environment)
-                          7      the same K steps from a device-side work queue: a persistent grid whose warps pull
-                                 (warp-tile of environments, chunk of steps) tasks; a tile's state goes through HBM between
-                                 its chunks.  Same results as 6 to rounding; not for MDS_CTRL_DSLPID.  Measured equal to 6
-                                 at large E and not better at small E (DESIGN.md 8), so 0 never selects it.
-                          3      whole steps, fused: ctrl | K-1 x [physics + ctrl in one launch] | physics
                           4      whole steps as two launches each (controller kernel, physics kernel)
                           1      controller kernel only (action_dev <- controller stack at obs_dev; env does not advance)
                           2      physics kernel only (env advances under action_dev)
-                          5      K fused launches: physics under the current action_dev, then the controller at
-                                 t0 + k dt_ctrl on the new observation (t0 = time AFTER the first physics step)
-                          1, 2 and 5 let a caller replay a rollout launch by launch with its own CUDA events. */
+                          A call with 1 then a call with 2 (K = 1 each) is one step of plan 4: repeated K times, they let
+                          a caller replay a rollout launch by launch with its own CUDA events.  Any other value is an error. */
   double obstacles[MDS_MAX_OBSTACLES * 4]; /* cx, cy, cz, r (r < 0: vertical cylinder of radius |r|) */
   const void* lqr_gain_planes_dev; /* optional, LQR controllers: a gain per drone, [4*dim][D] planes of Real (DecentralizedLQR*.K,
                                       simulations/CBFTest.py:319-321 `--controller dlqr`); NULL = MdsLqrGains.K for every drone */
@@ -297,7 +291,7 @@ int mds_xdot_nonlinear_f64(const MdsDroneParams* prm, double jx, double jy, doub
 /* ---- K-step rollout.  Default plan: ONE launch for all K control steps -- every lane group runs its own environment
  * forward (reference -> tracking controller -> CBF-QP -> inner loop -> physics sub-steps) with the observation and
  * the body rates in registers; HBM sees the initial load, the PID state, the log slots that are due and the final
- * store.  Other plans (MdsRolloutCfg.stages): one fused launch per step, two launches per step, single kernels.
+ * store.  Other plans (MdsRolloutCfg.stages): two launches per step, single kernels.
  * Everything is enqueued on `stream` with no host synchronisation.
  * obs_dev [D*20] in/out (observation before the first / after the last step); action_dev [D*4] scratch;
  * ext_force_dev optional [D*3] constant world-frame force per drone (wind, EnvGeometric.py:463-467);

@@ -667,17 +667,6 @@ static int xdot_nonlinear_impl(const MdsDroneParams* prm, double jx, double jy, 
 }
 extern "C" int mds_rollout_plan(int E, int N);
 extern "C" int mds_device_info(int* sm_count, int* cc_major, int* cc_minor, int* l2_bytes);
-static int cached_sm_count() {
-  static int sm_of_device[MDS_MAX_DEVICES];
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= MDS_MAX_DEVICES) return 0;
-  if (sm_of_device[dev] == 0) {
-    int sms = 0;
-    if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return 0;
-    sm_of_device[dev] = sms;
-  }
-  return sm_of_device[dev];
-}
 // PhysSpec<1> (mds_common.cuh): the swarm configuration of the reference's CBF mains, compiled without its mode switches
 static int phys_spec_of(const MdsDroneParams& p) {
   return (p.physics == MDS_PHYSICS_DYN_GND_DRAG_DW && p.drone_model == MDS_DRONE_CF2P && p.substeps == 1 && !p.renormalize_quat && p.ground_clamp &&
@@ -691,13 +680,13 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   MDS_REQUIRE(prm && cfg && st.pos_wx && st.quat && st.vel_wy && st.rpm && st.wz && specs && obs && action, "rollout: null pointer");
   MDS_REQUIRE(E > 0 && N > 0 && N <= MDS_MAX_DRONES_PER_ENV && K > 0, "rollout: bad E, N or K");
   MDS_REQUIRE(cfg->ctrl >= MDS_CTRL_GEOMETRIC && cfg->ctrl <= MDS_CTRL_DSLPID, "rollout: unknown controller");
-  MDS_REQUIRE(cfg->stages >= 0 && cfg->stages <= 7, "rollout: stages must be 0..7");
+  MDS_REQUIRE(cfg->stages == 0 || cfg->stages == 1 || cfg->stages == 2 || cfg->stages == 4 || cfg->stages == 6,
+              "rollout: stages must be 0, 1, 2, 4 or 6");
   RolloutP<Real> R;
   memset(&R, 0, sizeof(R));
   R.ctrl = cfg->ctrl; R.use_cbf = cfg->use_cbf; R.n_obs = cfg->num_obstacles; R.write_obs_every = cfg->write_obs_every;
   R.lqr_planes = (const Real*)cfg->lqr_gain_planes_dev; R.lqr_D = E * N;
   MDS_REQUIRE(!R.lqr_planes || lqr_variant_ok(cfg->ctrl), "rollout: per-drone gains need an LQR controller");
-  MDS_REQUIRE(!R.lqr_planes || (cfg->stages != 3 && cfg->stages != 5), "rollout: per-drone gains run in launch plans 6 / 7 (default), 4, 1 and 2");
   GeoP<Real> G;
   memset(&G, 0, sizeof(G));
   LqrP<Real> L;
@@ -747,14 +736,9 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   const StateP<Real> Sd = to_dev<Real>(st);
   const PidP<Real> Pi = to_dev<Real>(pid);
   const size_t obs_elems = (size_t)E * N * MDS_OBS_DIM;
-  // launch plan.  stages 0: mds_rollout_plan(E, N) (= 6, K steps in one launch); 3: the whole step, fused wherever a physics step is
-  // followed by a controller step (ctrl | K-1 x [physics + ctrl] | physics); 4: two launches (ctrl, physics) per step;
-  // 1: controller kernel only; 2: physics kernel only; 5: K fused launches [physics under the current action
-  // buffer + controller at t0 + k dt] -- with 1 and 2 it lets a caller replay a rollout launch by launch.
-  int mode = cfg->stages == 0 ? mds_rollout_plan(E, N) : cfg->stages;
-  // the queue plan re-reads a tile's state after another SM wrote it; the DSL PID state goes through plain (L1-cached) loads
-  if (mode == 7 && cfg->stages == 0 && (cfg->ctrl == MDS_CTRL_DSLPID || NP > 32)) mode = 6;
-  MDS_REQUIRE(!(mode == 7 && (cfg->ctrl == MDS_CTRL_DSLPID || NP > 32)), "rollout: plan 7 does not take the DSL PID controller");
+  // launch plan.  stages 0: mds_rollout_plan(E, N) (= 6, K steps in one launch); 4: two launches (ctrl, physics) per step;
+  // 1: controller kernel only; 2: physics kernel only -- 1 then 2 per step lets a caller replay a rollout launch by launch.
+  const int mode = cfg->stages == 0 ? mds_rollout_plan(E, N) : cfg->stages;
   auto obs_slot = [&](int j) -> Real* {  // where the observation after physics step j (1-based) goes
     if (R.write_obs_every > 0 && (j % R.write_obs_every) == 0) return obs_log + (size_t)(j / R.write_obs_every - 1) * obs_elems;
     return obs;
@@ -767,7 +751,6 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   auto launch_loop = [&]() {
     RolloutLaunch<Real> RLL = RL;  // the loop kernel has its own block size (MDS_LOOP_BLOCK)
     RLL.threads = R.use_cbf ? cbf_block_threads<Real>(NP, N, R.n_obs, loop_block<Real>()) : loop_block<Real>();
-    if (const char* force = getenv("MDS_LOOP_THREADS")) { const int t = atoi(force); if (t >= 32 && t <= RLL.threads && t % 32 == 0) RLL.threads = t; }  // experiment knob
     if (RLL.threads < NP) RLL.threads = NP;
     const int epb_l = RLL.threads / NP;
     RLL.blocks = (E + epb_l - 1) / epb_l;
@@ -781,47 +764,10 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
       keep(launch_loop_kernel<Real>(part, t0 + k0 * prm->dt_ctrl, prm->dt_ctrl, K - k0 < chunk ? K - k0 : chunk));
     }
   };
-  // plan 7: the same K steps from a device-side work queue (rollout_queue_kernel): a persistent grid whose warps pull
-  // (warp-tile of environments, chunk of steps) tasks; the queue lives in stream-ordered memory for the duration of the call
-  cudaError_t queue_err = cudaSuccess;
-  auto launch_queue = [&]() {
-    RolloutLaunch<Real> RLQ = RL;
-    RLQ.threads = R.use_cbf ? cbf_block_threads<Real>(NP, N, R.n_obs, loop_block<Real>()) : loop_block<Real>();
-    if (RLQ.threads < 32) RLQ.threads = 32;
-    RLQ.smem = R.use_cbf ? cbf_smem_bytes<Real>(RLQ.threads, NP, N, R.n_obs) : 32;
-    int per_sm = 0;
-    const int sms = cached_sm_count();  // cudaGetDeviceProperties costs milliseconds: once per device
-    if (sms <= 0) { queue_err = cudaErrorUnknown; return; }
-    RolloutQueue q{nullptr, nullptr, 0, 0, 0};
-    keep(launch_queue_kernel<Real>(RLQ, t0, prm->dt_ctrl, K, q, sms, true, &per_sm));
-    if (attr_err != cudaSuccess || per_sm < 1) { if (attr_err == cudaSuccess) queue_err = cudaErrorLaunchOutOfResources; return; }
-    const int envs_per_tile = 32 / NP, warps_per_block = RLQ.threads / 32;
-    q.tiles = (E + envs_per_tile - 1) / envs_per_tile;
-    int grid = sms * per_sm;
-    if (grid > (q.tiles + warps_per_block - 1) / warps_per_block) grid = (q.tiles + warps_per_block - 1) / warps_per_block;
-    const long long slots = (long long)grid * warps_per_block;
-    // ~8 tasks per resident warp: enough slack for the queue to even out the tail, few enough that the per-chunk state
-    // round trip through HBM (~350 B per drone) stays small against the chunk's steps
-    long long chunks = (8 * slots + q.tiles - 1) / q.tiles;
-    if (const char* force = getenv("MDS_QUEUE_CHUNKS")) chunks = atoi(force);  // experiment knob (tools/exp_queue.py)
-    if (chunks < 1) chunks = 1;
-    if (chunks > K) chunks = K;
-    q.chunk_steps = (int)((K + chunks - 1) / chunks);
-    q.chunks = (K + q.chunk_steps - 1) / q.chunk_steps;
-    int* mem = nullptr;
-    queue_err = cudaMallocAsync((void**)&mem, (size_t)(q.tiles + 1) * sizeof(int), cs);
-    if (queue_err != cudaSuccess) return;
-    queue_err = cudaMemsetAsync(mem, 0, (size_t)(q.tiles + 1) * sizeof(int), cs);
-    q.head = mem; q.progress = mem + 1;
-    RLQ.blocks = grid;
-    if (queue_err == cudaSuccess) keep(launch_queue_kernel<Real>(RLQ, t0, prm->dt_ctrl, K, q, sms, false, &per_sm));
-    cudaError_t fe = cudaFreeAsync(mem, cs);
-    if (queue_err == cudaSuccess) queue_err = fe;
-  };
-  bool first_ctrl = true, first_fused = true;
-  auto launch_ctrl = [&](bool fused, double t, Real* obs_ptr) {
-    if (fused) { keep(launch_fused_kernel<Real>(RL, t, obs_ptr, first_fused)); first_fused = false; }
-    else { keep(launch_ctrl_kernel<Real>(RL, t, obs_ptr, first_ctrl)); first_ctrl = false; }
+  bool first_ctrl = true;
+  auto launch_ctrl = [&](double t, Real* obs_ptr) {
+    keep(launch_ctrl_kernel<Real>(RL, t, obs_ptr, first_ctrl));
+    first_ctrl = false;
   };
   auto launch_phys = [&](Real* obs_out) {
     if (N == 8) physics_step_kernel<Real, 8><<<blocks, threads, 0, cs>>>(Pd, Sd, action, fext, obs_out, E, N, NP);
@@ -830,27 +776,17 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   const double dt = prm->dt_ctrl;
   Real* obs_last = obs;  // buffer holding the newest observation
   if (mode == 1) {
-    for (int k = 0; k < K; ++k) launch_ctrl(false, t0 + k * dt, obs);
+    for (int k = 0; k < K; ++k) launch_ctrl(t0 + k * dt, obs);
   } else if (mode == 2) {
     for (int k = 0; k < K; ++k) { obs_last = obs_slot(k + 1); launch_phys(obs_last); }
   } else if (mode == 4) {
     for (int k = 0; k < K; ++k) {
-      launch_ctrl(false, t0 + k * dt, obs_last);
+      launch_ctrl(t0 + k * dt, obs_last);
       obs_last = obs_slot(k + 1);
       launch_phys(obs_last);
     }
-  } else if (mode == 5) {
-    for (int k = 0; k < K; ++k) { obs_last = obs_slot(k + 1); launch_ctrl(true, t0 + k * dt, obs_last); }
-  } else if (mode == 6) {
-    launch_loop();  // writes the final observation to `obs` itself
-  } else if (mode == 7) {
-    launch_queue();
-    if (queue_err != cudaSuccess) return cuda_fail("rollout: work queue", queue_err);
   } else {
-    launch_ctrl(false, t0, obs);
-    for (int k = 1; k < K; ++k) { obs_last = obs_slot(k); launch_ctrl(true, t0 + k * dt, obs_last); }
-    obs_last = obs_slot(K);
-    launch_phys(obs_last);
+    launch_loop();  // writes the final observation to `obs` itself
   }
   if (attr_err != cudaSuccess) return cuda_fail("rollout: shared memory opt-in failed", attr_err);
   if (obs_last != obs) {
@@ -910,9 +846,9 @@ int mds_stream_synchronize(void* stream) {
   return MDS_OK;
 }
 // Measured on B200 (tools/exp_plans.py, tools/exp_c2.py): the K-steps-in-one-launch plan (6) is the fastest at every
-// size and precision -- C2 4096 envs 1.8 us per step vs 8.3 (fused) / 11.3 (two launches); C5 1M drones fp32 0.127 ms
-// vs 0.140 / 0.132; fp64 0.305 ms vs 0.50 / 0.44 -- so stages == 0 always selects it.  3 and 4 remain for callers
-// that want the observation materialised in HBM after every step, 1 / 2 / 5 for launch-by-launch replays.
+// size and precision -- C2 4096 envs 1.8 us per step vs 8.3 (one fused launch per step, a plan since removed) / 11.3 (two
+// launches); C5 1M drones fp32 0.127 ms vs 0.140 / 0.132; fp64 0.305 ms vs 0.50 / 0.44 -- so stages == 0 always selects it.
+// 4 remains as the per-call reference with the observation in HBM after every step, 1 / 2 for launch-by-launch replays.
 int mds_rollout_plan(int E, int N) { (void)E; (void)N; return 6; }
 int mds_cbf_num_rows(int order, int N, int n_obs) { return N * (N - 1) / 2 + 8 * N + (order == 3 ? 2 * N : 0) + N * n_obs; }
 

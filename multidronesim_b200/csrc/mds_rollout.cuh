@@ -1,5 +1,5 @@
-// mds_rollout.cuh -- the lane-group machinery and the three heavy kernels of the fused control step
-// (ctrl_step_kernel, step_fused_kernel, rollout_loop_kernel) + physics_step_kernel.  Header so that every
+// mds_rollout.cuh -- the lane-group machinery and the two heavy kernels of the fused control step
+// (ctrl_step_kernel, rollout_loop_kernel) + physics_step_kernel.  Header so that every
 // (precision, kernel kind) pair compiles in its own translation unit (mds_rollout_tu.cu; `make -j`).
 #pragma once
 #include <cuda_runtime.h>
@@ -32,9 +32,6 @@ using namespace mds;
 #endif
 // threads per block of the loop kernels for a precision
 template <typename Real> constexpr int loop_block() { return sizeof(Real) == 4 ? MDS_LOOP_BLOCK : MDS_LOOP_BLOCK_F64; }
-#ifndef MDS_FUSED_MINB
-#define MDS_FUSED_MINB 4
-#endif
 #ifndef MDS_PHYS_MINB
 #define MDS_PHYS_MINB 5
 #endif
@@ -735,41 +732,6 @@ __global__ void __launch_bounds__(MDS_BLOCK, MDS_CTRL_PERSISTENT ? 2 : (sizeof(R
   if (stats) stats_block_reduce<USE_CBF>(stats, n_done, acc, max_err);
 }
 
-// One launch per control step inside a rollout: the env advances under the PREVIOUS step's action, and the
-// controller stack runs on the new observation while it is still in registers (the observation is written for the
-// caller / the log but never read back; the action buffer is read and rewritten by the same thread).  Blocks of
-// one grid are in different phases (HBM-heavy physics, issue-heavy controller), which overlap on an SM.
-template <typename Real, int CTRL, bool USE_CBF, int NT>
-__global__ void __launch_bounds__(MDS_BLOCK, sizeof(Real) == 4 ? MDS_FUSED_MINB : 2) step_fused_kernel(DroneP<Real> P, RolloutP<Real> Rc, GeoP<Real> G, LqrP<Real> L, CbfP<Real> C,
-                                                                DslP<Real> Dg, DslStateP<Real> dst, StateP<Real> st, PidP<Real> pid,
-                                                                const typename TrajSpecT<Real>::spec* __restrict__ specs,
-                                                                const typename TrajSpecT<Real>::seg* __restrict__ segs,
-                                                                Real* __restrict__ action, const Real* __restrict__ fext, Real* __restrict__ obs_out,
-                                                                double* __restrict__ stats, double t, int E, int N_rt, int NP_rt) {
-  extern __shared__ __align__(32) unsigned char smem_raw[];
-  __shared__ typename Vec4T<Real>::type sm_pos[MDS_BLOCK];
-  const int N = ct_n<NT>(N_rt), NP = ct_np<NT>(NP_rt);
-  CbfSmem<Real> S = cbf_smem_carve<Real>(smem_raw, NP, N, Rc.n_obs);
-  GroupMap g = group_map(N, NP, E);
-  StepStats ss = {0.f, 1e30f, 0, 0, 0, 0};
-  if (g.env_valid) {
-    full_group_hint<NT>(g);
-    if (g.valid) {
-      prefetch_l1(specs + g.d);
-      prefetch_l1(reinterpret_cast<const char*>(specs + g.d) + 32);
-      if (CTRL == MDS_CTRL_LQR_OMEGA || CTRL == MDS_CTRL_LQR_YANK) { prefetch_l1(pid.a + g.d); prefetch_l1(pid.b + g.d); }
-    }
-    const Obs<Real> o = physics_body(P, st, action, fext, obs_out, sm_pos + (threadIdx.x - g.n), g, N, NP);
-    Real rpm[4] = {Real(0), Real(0), Real(0), Real(0)};
-    typename TrajSpecT<Real>::spec spec;
-    spec.kind = MDS_TRAJ_WAIT;
-    if (g.valid) spec = specs[g.d];
-    ctrl_body<Real, CTRL, USE_CBF>(P, Rc, G, L, C, Dg, dst, S, pid, spec, segs, o, g, N, NP, t, rpm, ss, g.d);
-    if (g.valid) store4(action, g.d, rpm);
-  }
-  if (stats) stats_block_reduce<USE_CBF>(stats, g.valid ? 1 : 0, ss, ss.err);
-}
-
 // Reference table of rollout_loop_kernel<..., REFTAB = true>: the references of MDS_REF_STEPS consecutive control steps for
 // the NT drones of an environment, slot (j, n) = 3 words at 3 (j NT + n).  A power of two (the step loop picks the row by a
 // mask); 32 steps x 8 drones = 12 KB in fp32.
@@ -925,183 +887,5 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
   if (FULLW && !live) { acc = {0.f, 1e30f, 0, 0, 0, 0}; max_err = 0.f; }  // a re-run environment counts nowhere
   acc.qp_cap = acc.qp_infeas >> 16;
   acc.qp_infeas &= 0xffff;
-  if (stats) stats_block_reduce<USE_CBF>(stats, steps_done, acc, max_err);
-}
-
-// ------------------------------------------------------------------ kernel: K-step rollout from a device-side work queue
-// L2-coherent (L1-bypassing) loads: a task's state may have been written by another SM a moment ago
-MDS_DEV float4 ld_cg(const float4* p) { return __ldcg(p); }
-MDS_DEV float2 ld_cg(const float2* p) { return __ldcg(p); }
-MDS_DEV float ld_cg(const float* p) { return __ldcg(p); }
-MDS_DEV double2 ld_cg(const double2* p) { return __ldcg(p); }
-MDS_DEV double ld_cg(const double* p) { return __ldcg(p); }
-MDS_DEV double4 ld_cg(const double4* p) {
-  const double2 a = __ldcg(reinterpret_cast<const double2*>(p)), b = __ldcg(reinterpret_cast<const double2*>(p) + 1);
-  double4 v; v.x = a.x; v.y = a.y; v.z = b.x; v.w = b.y;
-  return v;
-}
-template <typename Real> MDS_DEV Obs<Real> load_obs_cg(const Real* obs, int d) {
-  using R4 = typename Vec4T<Real>::type;
-  const R4* o4 = reinterpret_cast<const R4*>(obs + (size_t)d * MDS_OBS_DIM);
-  R4 a = ld_cg(o4), b = ld_cg(o4 + 1), c = ld_cg(o4 + 2), e = ld_cg(o4 + 3), f = ld_cg(o4 + 4);
-  Obs<Real> o;
-  o.p = {a.x, a.y, a.z}; o.qx = a.w; o.qy = b.x; o.qz = b.y; o.qw = b.z;
-  o.rpy = {b.w, c.x, c.y}; o.v = {c.z, c.w, e.x}; o.av = {e.y, e.z, e.w};
-  o.rpm[0] = f.x; o.rpm[1] = f.y; o.rpm[2] = f.z; o.rpm[3] = f.w;
-  return o;
-}
-
-// Work queue of the sliced rollout: `head` hands out task numbers, progress[w] = chunks of warp-tile w that are complete
-struct RolloutQueue {
-  int* head;
-  int* progress;
-  int tiles, chunks, chunk_steps;  // tasks = tiles * chunks, task = chunk * tiles + tile (chunk-major: a tile's chunks are far apart in the queue)
-};
-
-// The same K control steps as rollout_loop_kernel, scheduled at run time instead of by the block scheduler: a persistent grid
-// (one block per resident slot) whose WARPS pull tasks from a device-side queue.  A task = one warp-tile of environments
-// (32 / NP of them) x one chunk of consecutive control steps; the tile's state goes through HBM between chunks.  A swarm that
-// fills the GPU 1.65 times (15 625 environments on one of 8 GPUs: BASELINE.json configs[4] sharded 8 ways) then costs 1.65
-// rounds instead of the 2 waves of equal blocks the static grid needs, and large swarms lose their tail wave the same way.
-// A tile's chunk c waits (lane 0 spins on progress[tile]) until chunk c - 1 is complete; tasks are handed out in queue order
-// to warps that are running, so whoever holds the earlier chunk is making progress: no deadlock, whatever the grid size.
-template <typename Real, int CTRL, bool USE_CBF, int NT, int SPEC>
-__global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_queue_kernel(DroneP<Real> P, RolloutP<Real> Rc, GeoP<Real> G, LqrP<Real> L, CbfP<Real> C,
-                                                                   DslP<Real> Dg, DslStateP<Real> dst, StateP<Real> st, PidP<Real> pid,
-                                                                   const typename TrajSpecT<Real>::spec* __restrict__ specs,
-                                                                   const typename TrajSpecT<Real>::seg* __restrict__ segs,
-                                                                   Real* action, const Real* __restrict__ fext, Real* obs,
-                                                                   Real* __restrict__ obs_log, double* __restrict__ stats, double t0, double dt_ctrl, int K, int E,
-                                                                   int N_rt, int NP_rt, RolloutQueue Q) {
-  extern __shared__ __align__(32) unsigned char smem_raw[];
-  using R4 = typename Vec4T<Real>::type;
-  using R2 = typename Vec2T<Real>::type;
-  __shared__ R4 sm_pos[loop_block<Real>()];
-  constexpr bool STAGE = sizeof(Real) == 4;
-  __shared__ __align__(16) typename TrajSpecT<Real>::spec sm_spec[STAGE ? loop_block<Real>() : 1];
-  constexpr bool HAS_PID = (CTRL == MDS_CTRL_LQR_OMEGA || CTRL == MDS_CTRL_LQR_YANK);
-  __shared__ R4 sm_pid_a[(STAGE && HAS_PID) ? loop_block<Real>() : 1];
-  __shared__ R2 sm_pid_b[(STAGE && HAS_PID) ? loop_block<Real>() : 1];
-  __shared__ R4 sm_fx[STAGE ? loop_block<Real>() : 1];
-  // fp64 does not stage (shared-memory budget, see rollout_loop_kernel): its rate-PID state is held in two locals for the chunk
-  // instead -- never read through L1 from global memory, where another SM wrote it at the end of the tile's previous chunk
-  R4 pid_a_loc;
-  R2 pid_b_loc;
-  const PidP<Real> pid_s = STAGE ? PidP<Real>{sm_pid_a, sm_pid_b} : PidP<Real>{&pid_a_loc, &pid_b_loc};
-  const int N = ct_n<NT>(N_rt), NP = ct_np<NT>(NP_rt);
-  CbfSmem<Real> S = cbf_smem_carve<Real>(smem_raw, NP, N, Rc.n_obs);
-  const int lg = __ffs(NP) - 1, lane = threadIdx.x & 31;
-  const int envs_per_tile = 32 >> lg;
-  const bool has_fx = fext != nullptr;
-  const size_t obs_elems = (size_t)E * N * MDS_OBS_DIM;
-  StepStats acc = {0.f, 1e30f, 0, 0, 0, 0};  // qp_infeas holds infeasible | iteration-cap << 16 per task, unpacked below
-  int n_infeas = 0, n_cap = 0;
-  float max_err = 0.f;
-  int steps_done = 0;
-  const int n_tasks = Q.tiles * Q.chunks;
-  for (;;) {
-    int task = 0;
-    if (lane == 0) task = atomicAdd(Q.head, 1);
-    task = __shfl_sync(0xffffffffu, task, 0);
-    if (task >= n_tasks) break;
-    const int chunk = task / Q.tiles, tile = task - chunk * Q.tiles;
-    const int k0 = chunk * Q.chunk_steps, k1 = min(K, k0 + Q.chunk_steps);
-    if (chunk > 0) {  // the tile's previous chunk must have landed in HBM
-      if (lane == 0) {
-        while (*reinterpret_cast<volatile int*>(Q.progress + tile) < chunk) __nanosleep(64);
-        __threadfence();
-      }
-      __syncwarp();
-    }
-    GroupMap g;
-    g.el = threadIdx.x >> lg;
-    g.n = threadIdx.x & (NP - 1);
-    // A tile that sticks out beyond the last environment (only the last tile can) computes the last environment again in
-    // its surplus lane groups and keeps the copies to itself (no stores, no statistics): every group of every warp then runs
-    // the full step code, and for full lane groups `valid` is a compile-time true as in rollout_loop_kernel.
-    g.e = tile * envs_per_tile + (lane >> lg);
-    const bool dup = g.e >= E;
-    if (dup) g.e = E - 1;
-    g.env_valid = true;
-    g.valid = g.n < N;
-    full_group_hint<NT>(g);
-    g.d = g.e * N + g.n;
-    g.gmask = NP >= 32 ? 0xffffffffu : (((1u << NP) - 1u) << (lane & ~(NP - 1)));
-    g.cmask = g.gmask;
-    Obs<Real> o;
-    V3<Real> wb = {Real(0), Real(0), Real(0)};
-    typename TrajSpecT<Real>::spec spec_reg;
-    typename TrajSpecT<Real>::spec& spec = STAGE ? sm_spec[threadIdx.x] : spec_reg;
-    spec.kind = MDS_TRAJ_WAIT;
-    V3<Real> fx_reg = {Real(0), Real(0), Real(0)};
-    if (g.valid) {
-      o = load_obs_cg(obs, g.d);
-      spec = specs[g.d];
-      wb = {ld_cg(st.pos_wx + g.d).w, ld_cg(st.vel_wy + g.d).w, ld_cg(st.wz + g.d)};
-      if (has_fx) {
-        fx_reg = {fext[3 * g.d], fext[3 * g.d + 1], fext[3 * g.d + 2]};
-        if (STAGE) { R4 f4; f4.x = fx_reg.x; f4.y = fx_reg.y; f4.z = fx_reg.z; f4.w = Real(0); sm_fx[threadIdx.x] = f4; }
-      }
-      if (HAS_PID) {
-        const R4 pa = ld_cg(pid.a + g.d);
-        const R2 pb = ld_cg(pid.b + g.d);
-        if (STAGE) { sm_pid_a[threadIdx.x] = pa; sm_pid_b[threadIdx.x] = pb; }
-        else { pid_a_loc = pa; pid_b_loc = pb; }
-      }
-    }
-    Real rpm[4] = {Real(0), Real(0), Real(0), Real(0)};
-    const int every = Rc.write_obs_every;
-    int log_countdown = every > 0 ? every - (k0 % every) : 0;
-    Real* log_slot = every > 0 ? obs_log + (size_t)(k0 / every) * obs_elems : obs_log;
-    StepStats tk = {0.f, 1e30f, 0, 0, 0, 0};
-    for (int k = k0; k < k1; ++k) {
-      StepStats ss = {0.f, 1e30f, 0, 0, 0, 0};
-      M3<Real> R;
-      ctrl_body<Real, CTRL, USE_CBF, (NT < 0), SPEC, NT>(P, Rc, G, L, C, Dg, dst, S, pid_s, spec, segs, o, g, N, NP, t0 + (double)k * dt_ctrl, rpm, ss,
-                                                     STAGE ? (int)threadIdx.x : 0, HAS_PID ? &R : nullptr);
-      if (dup) { ss.err = 0.f; ss.min_h = 1e30f; ss.qp_solves = ss.qp_iters = ss.qp_infeas = ss.qp_cap = 0; }
-      tk.err += ss.err; max_err = fmaxf(max_err, ss.err); tk.min_h = fminf(tk.min_h, ss.min_h);
-      tk.qp_solves += ss.qp_solves; tk.qp_iters += ss.qp_iters; tk.qp_infeas += ss.qp_infeas; tk.qp_cap += ss.qp_cap;
-      Drone<Real> s;
-      s.p = o.p; s.qx = o.qx; s.qy = o.qy; s.qz = o.qz; s.qw = o.qw; s.v = o.v; s.w = wb;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) s.rpm[i] = o.rpm[i];
-      V3<Real> fx = fx_reg;
-      if (STAGE) {
-        fx = {Real(0), Real(0), Real(0)};
-        if (has_fx && g.valid) { const R4 f4 = sm_fx[threadIdx.x]; fx = {f4.x, f4.y, f4.z}; }
-      }
-      o = physics_core<SPEC>(P, s, rpm, fx, sm_pos + (threadIdx.x - g.n), g, N, NP, HAS_PID ? &R : nullptr);
-      wb = s.w;
-      if (every > 0 && --log_countdown == 0) {
-        if (g.valid && !dup) store_obs(log_slot, g.d, o, true);
-        log_slot += obs_elems;
-        log_countdown = every;
-      }
-    }
-    acc.err += tk.err; acc.min_h = fminf(acc.min_h, tk.min_h);
-    acc.qp_solves += tk.qp_solves; acc.qp_iters += tk.qp_iters; n_infeas += tk.qp_infeas; n_cap += tk.qp_cap;
-    if (g.valid && !dup) {
-      Drone<Real> s;
-      s.p = o.p; s.qx = o.qx; s.qy = o.qy; s.qz = o.qz; s.qw = o.qw; s.v = o.v; s.w = wb;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) s.rpm[i] = o.rpm[i];
-      store_drone(st, g.d, s);
-      store_obs(obs, g.d, o);
-      store4(action, g.d, rpm);
-      if (HAS_PID) {
-        pid.a[g.d] = STAGE ? sm_pid_a[threadIdx.x] : pid_a_loc;
-        pid.b[g.d] = STAGE ? sm_pid_b[threadIdx.x] : pid_b_loc;
-      }
-      steps_done += k1 - k0;
-    }
-    __syncwarp();  // every lane's stores are issued ...
-    if (lane == 0) {
-      __threadfence();  // ... and visible before the tile is published
-      atomicExch(Q.progress + tile, chunk + 1);
-    }
-    __syncwarp();  // the staged PID / descriptor slots are reused by the next task
-  }
-  acc.qp_infeas = n_infeas; acc.qp_cap = n_cap;
   if (stats) stats_block_reduce<USE_CBF>(stats, steps_done, acc, max_err);
 }

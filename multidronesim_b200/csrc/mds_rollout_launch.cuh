@@ -1,5 +1,5 @@
-// mds_rollout_launch.cuh -- host-side launchers of the three heavy rollout kernels.  Declared here, defined in
-// mds_rollout_tu.cu, which the Makefile compiles once per (precision, kernel kind): the ~120 instantiations build in
+// mds_rollout_launch.cuh -- host-side launchers of the two heavy rollout kernels.  Declared here, defined in
+// mds_rollout_tu.cu, which the Makefile compiles once per (precision, kernel kind): the ~110 instantiations build in
 // parallel instead of inside one translation unit.
 #pragma once
 #include <cuda_runtime.h>
@@ -33,8 +33,3 @@ template <typename Real> struct RolloutLaunch {
 // picked up by the caller's cudaGetLastError().
 template <typename Real> cudaError_t launch_loop_kernel(const RolloutLaunch<Real>& a, double t0, double dt_ctrl, int K);
 template <typename Real> cudaError_t launch_ctrl_kernel(const RolloutLaunch<Real>& a, double t, const Real* obs_in, bool set_attr);
-template <typename Real> cudaError_t launch_fused_kernel(const RolloutLaunch<Real>& a, double t, Real* obs_out, bool set_attr);
-// the work-queue form of the K-step rollout (rollout_queue_kernel); q: device queue already zeroed on a.cs, tiles / chunks set by the caller.
-// *grid_blocks (in: 0 = ask) receives / provides the persistent grid size
-template <typename Real> cudaError_t launch_queue_kernel(const RolloutLaunch<Real>& a, double t0, double dt_ctrl, int K, RolloutQueue q, int sm_count, bool query_only,
-                                                         int* blocks_per_sm);

@@ -1,17 +1,17 @@
 // mds_rollout_tu.cu -- one translation unit per (precision, kernel kind) of the rollout kernels:
-//   nvcc -DMDS_TU_REAL=float|double -DMDS_TU_KIND=0 (rollout_loop_kernel) | 1 (ctrl_step_kernel) | 2 (step_fused_kernel) | 3 (rollout_queue_kernel)
+//   nvcc -DMDS_TU_REAL=float|double -DMDS_TU_KIND=0 (rollout_loop_kernel) | 1 (ctrl_step_kernel)
 // Each defines the matching launcher of mds_rollout_launch.cuh; mds_kernels.cu (the C ABI) calls them.
 #include "mds_rollout_launch.cuh"
 
 #ifndef MDS_TU_REAL
 #error "compile with -DMDS_TU_REAL=float or double"
 #endif
-#ifndef MDS_TU_KIND
-#error "compile with -DMDS_TU_KIND=0, 1, 2 or 3"
+#if !defined(MDS_TU_KIND) || (MDS_TU_KIND != 0 && MDS_TU_KIND != 1)
+#error "compile with -DMDS_TU_KIND=0 or 1"
 #endif
 using Real = MDS_TU_REAL;
 
-// controller / filter dispatch shared by the three launchers: calls F.template run<CTRL, USE_CBF, PDKC>()
+// controller / filter dispatch shared by the two launchers: calls F.template run<CTRL, USE_CBF, PDKC>()
 template <typename F> static void dispatch_ctrl(int ctrl, int use_cbf, F&& f) {
   switch (ctrl) {
     case MDS_CTRL_GEOMETRIC: f.template run<MDS_CTRL_GEOMETRIC, false, false>(); break;
@@ -54,7 +54,7 @@ template <> cudaError_t launch_loop_kernel<Real>(const RolloutLaunch<Real>& a, d
   dispatch_ctrl(a.R.ctrl, a.R.use_cbf, l);
   return l.err;
 }
-#elif MDS_TU_KIND == 1
+#else
 struct CtrlLauncher {
   const RolloutLaunch<Real>& a;
   double t;
@@ -83,56 +83,6 @@ struct CtrlLauncher {
 };
 template <> cudaError_t launch_ctrl_kernel<Real>(const RolloutLaunch<Real>& a, double t, const Real* obs_in, bool set_attr) {
   CtrlLauncher l{a, t, obs_in, set_attr, cudaSuccess};
-  dispatch_ctrl(a.R.ctrl, a.R.use_cbf, l);
-  return l.err;
-}
-#elif MDS_TU_KIND == 2
-struct FusedLauncher {
-  const RolloutLaunch<Real>& a;
-  double t;
-  Real* obs_out;
-  bool set_attr;
-  cudaError_t err;
-  template <int CT, bool CB, bool PDKC> void run() {
-    auto kern = (a.N == 8) ? step_fused_kernel<Real, CT, CB, 8> : step_fused_kernel<Real, CT, CB, 0>;
-    if (set_attr) err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)a.smem);
-    kern<<<a.blocks, a.threads, a.smem, a.cs>>>(a.Pd, a.R, a.G, a.L, a.C, a.Dg, a.Ds, a.Sd, a.Pi, a.specs, a.segs, a.action, a.fext, obs_out, a.stats, t,
-                                                 a.E, a.N, a.NP);
-  }
-};
-template <> cudaError_t launch_fused_kernel<Real>(const RolloutLaunch<Real>& a, double t, Real* obs_out, bool set_attr) {
-  FusedLauncher l{a, t, obs_out, set_attr, cudaSuccess};
-  dispatch_ctrl(a.R.ctrl, a.R.use_cbf, l);
-  return l.err;
-}
-#else
-struct QueueLauncher {
-  const RolloutLaunch<Real>& a;
-  double t0, dt_ctrl;
-  int K;
-  RolloutQueue q;
-  int sm_count;
-  bool query_only;
-  int* blocks_per_sm;
-  cudaError_t err;
-  template <int CT, bool CB, bool PDKC> void run() {
-    const bool pdk = a.R.lqr_planes != nullptr;
-    auto kern = pdk ? rollout_queue_kernel<Real, CT, CB, (PDKC ? -1 : 0), 0>
-                    : (a.spec == 1 ? ((a.N == 8) ? rollout_queue_kernel<Real, CT, CB, 8, 1> : rollout_queue_kernel<Real, CT, CB, 0, 1>)
-                                   : ((a.N == 8) ? rollout_queue_kernel<Real, CT, CB, 8, 0> : rollout_queue_kernel<Real, CT, CB, 0, 0>));
-    err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)a.smem);
-    if (err != cudaSuccess) return;
-    if (query_only) {  // resident blocks per SM of this instantiation at this block size / shared-memory footprint
-      err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, kern, a.threads, a.smem);
-      return;
-    }
-    kern<<<a.blocks, a.threads, a.smem, a.cs>>>(a.Pd, a.R, a.G, a.L, a.C, a.Dg, a.Ds, a.Sd, a.Pi, a.specs, a.segs, a.action, a.fext, a.obs, a.obs_log,
-                                                 a.stats, t0, dt_ctrl, K, a.E, a.N, a.NP, q);
-  }
-};
-template <> cudaError_t launch_queue_kernel<Real>(const RolloutLaunch<Real>& a, double t0, double dt_ctrl, int K, RolloutQueue q, int sm_count, bool query_only,
-                                                  int* blocks_per_sm) {
-  QueueLauncher l{a, t0, dt_ctrl, K, q, sm_count, query_only, blocks_per_sm, cudaSuccess};
   dispatch_ctrl(a.R.ctrl, a.R.use_cbf, l);
   return l.err;
 }

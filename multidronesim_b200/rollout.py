@@ -1,6 +1,6 @@
 """K-step rollout (``mds_rollout``): by default ONE launch advances every environment K control steps (trajectory ->
 tracking controller -> CBF-QP -> inner loop -> physics sub-steps, observation and body rates in registers from step to
-step); other launch plans (one fused launch per step, two launches per step, single kernels) via ``stages``.
+step); other launch plans (two launches per step, single kernels) via ``stages``.
 
 It is the device equivalent of the reference's per-step Python loops
 (simulations/EnvGeometric.py:434-479, simulations/CBFTest.py:302-358,
@@ -76,18 +76,16 @@ class FusedRollout:
         """Advance every environment K control steps.  ``obs_log`` [K//log_every, E, N, 20] receives the
         observation after every ``log_every``-th step (the reference's ``observations.append(obs)``).
         ``stages`` (MdsRolloutCfg.stages): 0 = whole steps with the default plan (``plan()``: 6 = all K steps in ONE
-        launch, observation and body rates in registers from step to step);
-        3 = whole steps, one fused launch per step in the steady state;
+        launch, observation and body rates in registers from step to step; 6 selects it explicitly);
         4 = whole steps as two launches each; 1 = controller kernel only (fills the env's action buffer, time does
-        not advance); 2 = physics kernel only (consumes that action buffer); 5 = fused launches only (physics under
-        the current action buffer, then the controller at the new time).
+        not advance); 2 = physics kernel only (consumes that action buffer).  ``run(1, stages=1)`` then
+        ``run(1, stages=2)`` is one step of plan 4: K such pairs replay a rollout launch by launch.
         Returns the env's obs buffer (observation after the last step)."""
         env = self.env
         if t0 is None:
             t0 = self.t
-        if stages not in (0, 1, 2, 3, 4, 5, 6, 7):
-            raise ValueError("stages must be 0..7")
-        t_call = t0 + env.CTRL_TIMESTEP if stages == 5 else t0  # 5: the controller runs after the physics step
+        if stages not in (0, 1, 2, 4, 6):
+            raise ValueError("stages must be 0, 1, 2, 4 or 6")
         self.cfg.stages = int(stages)
         self.cfg.write_obs_every = int(log_every) if obs_log is not None else 0
         N = env.NUM_DRONES
@@ -115,7 +113,7 @@ class FusedRollout:
         cbf = self.qp.cbf.c_params() if self.qp is not None else None
         _lib.call("mds_rollout", env.dtype, env._prm, self.cfg, geo, lqr, cbf, env._state_struct(), pid, dsl, dsl_state,
                   _lib.ptr(self.trajs.specs), _lib.ptr(self.trajs.segs), _lib.ptr(env._obs), _lib.ptr(env._action), _lib.ptr(env._ext_force), _lib.ptr(obs_log),
-                  _lib.ptr(self.stats), float(t_call), int(K), env.NUM_ENVS, env.NUM_DRONES, _lib.stream_ptr(env.device))
+                  _lib.ptr(self.stats), float(t0), int(K), env.NUM_ENVS, env.NUM_DRONES, _lib.stream_ptr(env.device))
         if stages != 1:
             env.step_counter += K * env.PYB_STEPS_PER_CTRL
             self.t = t0 + K * env.CTRL_TIMESTEP

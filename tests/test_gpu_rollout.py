@@ -195,12 +195,13 @@ def test_c5_full_lap_vs_oracle(dtype, tol, lib_built):
 
 @pytest.mark.parametrize("ctrl,cbf_order,N,n_obs", [("yank10", 3, 8, 1), ("omega9", 2, 3, 1), ("geometric", None, 1, 0),
                                                     ("yank10", 3, 2, 4)])  # last: more obstacles than drones (SURVEY 8f-4)
-def test_launch_plans_agree(ctrl, cbf_order, N, n_obs, lib_built):
-    """MdsRolloutCfg.stages: the fused plan (one launch per step), the two-launch plan and a launch-by-launch
-    replay (1, then 5 x (K-1), then 2) are the same computation: bit-identical observations and statistics,
-    including the observation log."""
+def test_remaining_launch_plans_agree(ctrl, cbf_order, N, n_obs, lib_built):
+    """MdsRolloutCfg.stages: the two-launch plan (4) and a launch-by-launch replay (1, then 2, per step) are the same
+    computation: bit-identical observations, statistics, actions and rate-PID state.  The K-steps-in-one-launch plan (6)
+    agrees with them to fp32 rounding, including the observation log.  Plans 4 and 6 run the K steps as two calls, so the
+    second call starts from the state, rate-PID state and action the first one stored."""
     import multidronesim_b200.trajectories as T
-    E, K, dtype = 5, 9, torch.float32
+    E, K, K1, dtype = 5, 9, 3, torch.float32
     rng = np.random.default_rng(11)
     specs = [dict(a=1.0, center=np.array([0, 0, 0.5]), omega=0.5, yaw_rate=0.1, phase_shift=float(2 * np.pi / (N + 0.25) * k)) for k in range(N)]
     init = np.zeros((E, N, 3))
@@ -209,31 +210,38 @@ def test_launch_plans_agree(ctrl, cbf_order, N, n_obs, lib_built):
             init[e, j] = otj.Lemniscate(**sp)(0.0)[0] + rng.normal(0, 0.02, 3) + np.array([0, 0, 0.04 * j])
     obstacles = [[0.2, 0.0, 0.5, 0.1], [-0.3, 0.1, 0.6, 0.08], [0.9, 0.4, 0.45, 0.12], [-0.8, -0.3, 0.5, -0.1]][:n_obs] if cbf_order is not None else None
     outs = []
-    for plan in ("fused", "two", "replay", "loop"):
+    for plan in ("two", "replay", "loop"):
         mds, env, c, trk, ts, ro = build(E, N, dtype, "dyn_gnd_drag_dw", [T.Lemniscate(**sp) for sp in specs] * E, ctrl, cbf_order, obstacles, init)
         log = torch.zeros(K // 3, E, N, 20, device="cuda", dtype=dtype)
-        if plan == "fused":
-            assert ro.plan() == 6  # the default is the K-steps-in-one-launch plan
-            ro.run(K, obs_log=log, log_every=3, stages=3)
-        elif plan == "two":
-            ro.run(K, obs_log=log, log_every=3, stages=4)
-        elif plan == "loop":
-            ro.run(K, obs_log=log, log_every=3, stages=6)
+        if plan == "replay":
+            for k in range(K):
+                ro.run(1, stages=1)
+                ro.run(1, stages=2)
         else:
-            ro.run(1, stages=1)
-            for k in range(K - 1):
-                ro.run(1, stages=5)
-            ro.run(1, stages=2)
+            if plan == "loop":
+                assert ro.plan() == 6  # the default is the K-steps-in-one-launch plan
+            # K1 is a whole number of log periods: the two calls fill the log of one K-step call
+            ro.run(K1, obs_log=log[:K1 // 3], log_every=3, stages=4 if plan == "two" else 6)
+            ro.run(K - K1, obs_log=log[K1 // 3:], log_every=3, stages=4 if plan == "two" else 6)
         assert abs(ro.t - K * env.CTRL_TIMESTEP) < 1e-12
-        outs.append((env.obs.cpu().numpy().copy(), log.cpu().numpy().copy(), ro.stats.cpu().numpy().copy()))
-    assert np.array_equal(outs[0][0], outs[1][0]) and np.array_equal(outs[0][0], outs[2][0])
-    assert np.array_equal(outs[0][1], outs[1][1]) and np.abs(outs[0][1]).max() > 0
-    assert np.array_equal(outs[0][2], outs[1][2]) and np.array_equal(outs[0][2], outs[2][2])
+        pid = (c.low_level._a.cpu().numpy().copy(), c.low_level._b.cpu().numpy().copy()) if ctrl in ("yank10", "omega9") else ()
+        outs.append((env.obs.cpu().numpy().copy(), log.cpu().numpy().copy(), ro.stats.cpu().numpy().copy(), env._action.cpu().numpy().copy(), pid))
+    for s in (3, 5, 7):  # plans that no longer exist
+        with pytest.raises(ValueError):
+            ro.run(1, stages=s)
+    two, replay, loop = outs
+    assert np.array_equal(two[0], replay[0]) and np.array_equal(two[2], replay[2]) and np.array_equal(two[3], replay[3])
+    assert all(np.array_equal(x, y) for x, y in zip(two[4], replay[4]))
+    assert np.abs(two[1]).max() > 0
     # the K-steps-in-one-launch plan is the same arithmetic compiled as one loop body: nvcc may contract a*b+c into
     # an FMA differently there, so it agrees to fp32 rounding (amplified over K closed-loop steps), not bit for bit;
     # its per-thread float accumulation of the error sum rounds differently, the counters are exact
-    assert np.allclose(outs[0][0], outs[3][0], rtol=2e-4, atol=2e-4) and np.allclose(outs[0][1], outs[3][1], rtol=2e-4, atol=2e-4)
-    assert np.allclose(outs[0][2], outs[3][2], rtol=1e-3) and outs[0][2][0] == outs[3][2][0]
+    tol = dict(rtol=2e-4, atol=2e-4)
+    assert np.allclose(two[0], loop[0], **tol) and np.allclose(two[1], loop[1], **tol)
+    assert np.allclose(two[2], loop[2], rtol=1e-3) and two[2][0] == loop[2][0]
+    assert np.allclose(two[3], loop[3], rtol=tol["rtol"], atol=tol["atol"] * 2e4)  # rotor speeds, ~1e4 rpm
+    for x, y in zip(two[4], loop[4]):
+        assert np.allclose(x, y, rtol=tol["rtol"], atol=tol["atol"] * 10)
 
 
 def test_full_size_env_independence(lib_built):
@@ -257,7 +265,7 @@ def test_full_size_env_independence(lib_built):
         assert torch.equal(small["env"].obs[0], obs_big[e0]), e0
 
 
-def test_rollout_with_wind(lib_built):
+def test_rollout_with_wind_in_plans_6_and_4(lib_built):
     """A constant per-drone world-frame force (the reference's wind, EnvGeometric.py:463-467; set_external_force) acts in
     every launch plan of the rollout exactly as in the per-call loop, and changes the flight."""
     import multidronesim_b200.trajectories as T
@@ -266,13 +274,13 @@ def test_rollout_with_wind(lib_built):
     init = np.array([[otj.Lemniscate(**sp)(0.0)[0] for sp in specs]] * E)
     wind = np.zeros((E, N, 3)); wind[..., 0] = 0.00025 * (1 + np.arange(E))[:, None]
     outs = {}
-    for plan in ("percall", 6, 4, 3, "calm"):
+    for plan in ("percall", 6, 4, "calm"):
         mds, env, c, trk, ts, ro = build(E, N, dtype, "dyn_gnd_drag_dw", [T.Lemniscate(**sp) for sp in specs] * E, "geometric", init=init)
         if plan != "calm":
             env.set_external_force(wind)
         obs = percall_loop(mds, env, c, trk, ts, K, None) if plan == "percall" else ro.run(K, stages=6 if plan == "calm" else plan)
         outs[plan] = obs.cpu().numpy().copy()
-    for plan in (6, 4, 3):
+    for plan in (6, 4):
         assert np.max(np.abs(outs[plan] - outs["percall"])) < 1e-9 * (1 + np.max(np.abs(outs["percall"]))), plan
     assert np.max(np.abs(outs["calm"][..., 0:3] - outs[6][..., 0:3])) > 1e-5   # the wind moved the drones
 
@@ -357,49 +365,6 @@ def test_host_pipelines_equal_device_paths(lib_built):
         evs[j].synchronize()
         assert np.array_equal(out[j].numpy(), log[j * K:(j + 1) * K].cpu().numpy()), j
     hr.synchronize()
-
-
-@pytest.mark.parametrize("ctrl,cbf_order,N,E,K,every,dtype", [("yank10", 3, 8, 301, 24, 1, torch.float32), ("yank10", 3, 8, 45, 13, 3, torch.float64),
-                                                              ("omega9", 2, 3, 77, 10, 2, torch.float32), ("geometric", None, 1, 500, 16, 4, torch.float32),
-                                                              ("torque12", None, 5, 33, 7, 0, torch.float64)])
-def test_work_queue_plan_equals_loop_plan(ctrl, cbf_order, N, E, K, every, dtype, lib_built):
-    """Launch plan 7 (rollout_queue_kernel: a persistent grid whose warps pull (tile of environments, chunk of steps) tasks from a
-    device-side queue, the tile's state going through HBM between chunks) computes what plan 6 (one block-scheduled launch, state in
-    registers for all K steps) computes: same final observations / state / controller state, same observation log, same counters.
-    Sizes that leave the last warp-tile partly empty and chunkings that do not divide K."""
-    import multidronesim_b200.trajectories as T
-    rng = np.random.default_rng(21)
-    specs = [dict(a=1.0, center=np.array([0, 0, 0.5]), omega=0.5, yaw_rate=0.1, phase_shift=float(2 * np.pi / (N + 0.25) * k)) for k in range(N)]
-    init = np.zeros((E, N, 3))
-    for e in range(E):
-        for j, sp in enumerate(specs):
-            init[e, j] = otj.Lemniscate(**sp)(0.0)[0] + rng.normal(0, 0.02, 3) + np.array([0, 0, 0.04 * j])
-    obstacles = [[0.2, 0.0, 0.5, 0.1]] if cbf_order is not None else None
-    outs = []
-    for plan in (6, 7):
-        mds, env, c, trk, ts, ro = build(E, N, dtype, "dyn_gnd_drag_dw", [T.Lemniscate(**sp) for sp in specs] * E, ctrl, cbf_order, obstacles, init)
-        log = torch.zeros(max(1, K // max(1, every)), E, N, 20, device="cuda", dtype=dtype)
-        for _ in range(2):   # two calls: the second starts from the state the first one stored
-            ro.run(K, obs_log=log if every else None, log_every=every, stages=plan)
-        torch.cuda.synchronize()
-        pid = (c.low_level._a.cpu().numpy().copy(), c.low_level._b.cpu().numpy().copy()) if ctrl in ("yank10", "omega9") else ()
-        outs.append((env.obs.cpu().numpy().copy(), log.cpu().numpy().copy(), ro.stats.cpu().numpy().copy(), env.state_dict(), pid, env._action.cpu().numpy().copy()))
-    a, b = outs
-    # two compilations of the same step code (nvcc may contract a*b+c differently in each): equal to rounding, amplified
-    # over 2 K closed-loop steps -- not bit for bit
-    tol = dict(rtol=2e-4, atol=2e-4) if dtype == torch.float32 else dict(rtol=1e-9, atol=1e-9)
-    assert np.allclose(a[0], b[0], **tol) and np.allclose(a[1], b[1], **tol) and np.allclose(a[5], b[5], rtol=tol["rtol"], atol=tol["atol"] * 2e4)
-    assert np.abs(a[1]).max() > 0 or not every
-    for k in a[3]:
-        va, vb = a[3][k], b[3][k]
-        if isinstance(va, torch.Tensor):
-            assert np.allclose(va.double().cpu().numpy(), vb.double().cpu().numpy(), rtol=tol["rtol"], atol=tol["atol"] * (2e4 if "rpm" in k else 1)), k
-        else:
-            assert va == vb, k
-    for x, y in zip(a[4], b[4]):
-        assert np.allclose(x, y, rtol=tol["rtol"], atol=tol["atol"] * 10)
-    # counters exact; the error sum is accumulated per thread in a different grouping (float): close
-    assert np.array_equal(a[2][[0, 4, 6, 7]], b[2][[0, 4, 6, 7]]) and np.allclose(a[2], b[2], rtol=1e-4)
 
 
 def test_swarm_streams_equal_one_swarm(lib_built):

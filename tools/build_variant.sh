@@ -13,5 +13,5 @@ nvcc $FLAGS -DMDS_TU_REAL=float -DMDS_TU_KIND=0 -c -o build_$tag/rollout_float_0
 nvcc $FLAGS -DMDS_TU_REAL=double -DMDS_TU_KIND=0 -c -o build_$tag/rollout_double_0.o mds_rollout_tu.cu &
 wait
 nvcc -gencode arch=compute_100a,code=sm_100a -shared -o libmds_$tag.so build_$tag/mds_kernels.o build_$tag/rollout_float_0.o build_$tag/rollout_double_0.o \
-  build/rollout_float_1.o build/rollout_float_2.o build/rollout_float_3.o build/rollout_double_1.o build/rollout_double_2.o build/rollout_double_3.o
+  build/rollout_float_1.o build/rollout_double_1.o
 echo built libmds_$tag.so
