@@ -352,6 +352,24 @@ int mds_dlqr_ctrl_f32(const MdsDroneParams* prm, int variant, const float* K_dev
 int mds_dlqr_ctrl_f64(const MdsDroneParams* prm, int variant, const double* K_dev, int coupled, const double* obs_dev, const double* ref_dev,
                       double* u_dev, double* action_dev, MdsPidState pid, int E, int N, void* stream);
 
+/* The system-identification loop of the decentralised LQR (learning phases of simulations/CBFTest.py:150-265,
+ * CBFTestOrd3.py:150-270) for K control steps in ONE launch.  Step k of every drone: ref_k = trajectory at t0 + k*dt_ctrl,
+ * e_t = error state against ref_k, inner loop (variant MDS_CTRL_LQR_OMEGA: ThrustOmega, _YANK: YankOmega) on the caller's
+ * excitation inputs_dev[k] [D*4], physics step (ext_force_dev optional [D*3], as mds_physics_step), e_t+1 against the same
+ * ref_k, and -- if k >= learn_from -- one RLS step of `rls` with phi = [e_t, u_k], x1 = e_t+1 (rls->m = 9 with OMEGA, 10
+ * with YANK; project_theta at m = 10 only; drones_per_env = N).  The same results as that loop over mds_traj_eval,
+ * mds_error_state, mds_lowlevel, mds_physics_step and mds_rls_update.  theta_dev / P_dev planes as mds_rls_update, updated in place; resid_dev optional
+ * [D][m] (the residual of the last update, untouched when none ran); obs_dev [D*20] in/out; PID state in/out;
+ * obs_log_dev optional [K/write_obs_every][D*20].  K = 0 launches nothing (inputs_dev may then be NULL). */
+int mds_learning_rollout_f32(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,
+                             MdsPidState pid, const MdsTrajSpecF32* specs_dev, const MdsTrajSegF32* segs_dev, const float* inputs_dev,
+                             float* theta_dev, float* P_dev, float* resid_dev, float* obs_dev, const float* ext_force_dev, float* obs_log_dev,
+                             double t0, int K, int E, int N, void* stream);
+int mds_learning_rollout_f64(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,
+                             MdsPidState pid, const MdsTrajSpecF64* specs_dev, const MdsTrajSegF64* segs_dev, const double* inputs_dev,
+                             double* theta_dev, double* P_dev, double* resid_dev, double* obs_dev, const double* ext_force_dev, double* obs_log_dev,
+                             double t0, int K, int E, int N, void* stream);
+
 /* compute_controller (decentralized_lqr_omega.py:185-204): K_d = R^-1 B_d' X_d, X_d the stabilising solution of the
  * continuous-time algebraic Riccati equation of drone d's learned model theta_d = [A_d, B_d]^T, for diagonal Q (q_diag [m])
  * and R (r_diag [4], host arrays).  One warp per drone, double precision inside (matrix sign function; the reference calls

@@ -16,6 +16,8 @@ drone d at ``[k, d]`` -- so that one thread per drone reads and writes coalesced
 """
 from __future__ import annotations
 
+import inspect
+
 import numpy as np
 import scipy.linalg as la
 import torch
@@ -107,17 +109,37 @@ class _DecentralizedBase(BaseController):
         self.P_planes.copy_(_lib.require_cuda(P, "P", self.env.dtype).reshape(-1, self.mn * self.mn).t())
 
     # ------------------------------------------------------------------ model learning
-    def _rls(self, phis, xtp1s, target, predict_from_xtp1, normalize_gain, project):
+    # method -> (target, predict_from_xtp1, normalize_gain, project) of its RLS step; the variants fill it in
+    RLS_METHODS = {}
+
+    def rls_cfg(self, method, **options):
+        """MdsRlsCfg of the RLS step ``method`` defines (the per-call methods and LearningRollout both build it here).
+        ``options``: the keyword options the per-call method itself takes, nothing else -- ``project=False``
+        (approx_theta_update of the crazyflie variant) is the same step without project_theta."""
+        if method not in self.RLS_METHODS:
+            raise ValueError(f"{type(self).__name__} defines no RLS method {method!r}; it has {sorted(self.RLS_METHODS)}")
+        accepted = [n for n in inspect.signature(getattr(self, method)).parameters if n not in ("phis", "xtp1s")]
+        unknown = sorted(set(options) - set(accepted))
+        if unknown:
+            raise TypeError(f"{type(self).__name__}.{method} takes no option {', '.join(unknown)} (it takes {accepted or 'none'})")
+        target, predict_from_xtp1, normalize_gain, proj = self.RLS_METHODS[method]
+        if not options.get("project", True):
+            proj = RLS_PROJECT_NONE
+        env = self.env
+        cfg = _lib.RlsCfg()
+        cfg.m, cfg.target, cfg.predict_from_xtp1, cfg.normalize_gain = self.m, target, int(predict_from_xtp1), int(normalize_gain)
+        cfg.project, cfg.drones_per_env, cfg.dt = proj, env.NUM_DRONES, env.CTRL_TIMESTEP
+        codes = self._project_codes() if proj != RLS_PROJECT_NONE else np.ones((self.mn, self.m), dtype=np.uint8)
+        for k, v in enumerate(np.asarray(codes, dtype=np.uint8).reshape(-1)):
+            cfg.theta_code[k] = int(v)
+        return cfg
+
+    def _rls(self, phis, xtp1s, method, **options):
         env = self.env
         D = env.NUM_TOTAL
         phis = _lib.require_cuda(phis, "phis", env.dtype).reshape(D, self.mn)
         xtp1s = _lib.require_cuda(xtp1s, "xtp1s", env.dtype).reshape(D, self.m)
-        cfg = _lib.RlsCfg()
-        cfg.m, cfg.target, cfg.predict_from_xtp1, cfg.normalize_gain = self.m, target, int(predict_from_xtp1), int(normalize_gain)
-        cfg.project, cfg.drones_per_env, cfg.dt = project, env.NUM_DRONES, env.CTRL_TIMESTEP
-        codes = self._project_codes() if project != RLS_PROJECT_NONE else np.ones((self.mn, self.m), dtype=np.uint8)
-        for k, v in enumerate(np.asarray(codes, dtype=np.uint8).reshape(-1)):
-            cfg.theta_code[k] = int(v)
+        cfg = self.rls_cfg(method, **options)
         _lib.call("mds_rls_update", env.dtype, cfg, _lib.ptr(phis.contiguous()), _lib.ptr(xtp1s.contiguous()), _lib.ptr(self.theta_planes),
                   _lib.ptr(self.P_planes), _lib.ptr(self.resid), D, _lib.stream_ptr(env.device))
         return self.resid
@@ -265,6 +287,8 @@ class _DecentralizedBase(BaseController):
 class DecentralizedLQROmega(_DecentralizedBase):
     """9-dim thrust + body-rate model (control/dlqr/decentralized_lqr_omega.py)."""
     VARIANT, M = _lib.CTRL_LQR_OMEGA, 9
+    RLS_METHODS = {"theta_update": (RLS_TARGET_PREDICT, True, True, RLS_PROJECT_NONE),
+                   "theta_update2": (RLS_TARGET_PREDICT, True, False, RLS_PROJECT_NONE)}
 
     def _weights(self):
         mt = self.env.MAX_THRUST  # decentralized_lqr_omega.py:21-37
@@ -277,12 +301,12 @@ class DecentralizedLQROmega(_DecentralizedBase):
 
     def theta_update(self, phis, xtp1s):
         """:125-139 -- RLS on x_{t+1} - forward_predict(x_{t+1}, u) (the reference starts the prediction at x_{t+1})."""
-        return self._rls(phis, xtp1s, RLS_TARGET_PREDICT, True, True, RLS_PROJECT_NONE)
+        return self._rls(phis, xtp1s, "theta_update")
 
     def theta_update2(self, phis, xtp1s):
         """:110-123 -- information form: theta += V^-1 phi r, V += phi phi'.  ``P`` holds V^-1 here (V0 = I), kept current
         by the rank-one inverse update, so no 13 x 13 inverse per drone and step."""
-        return self._rls(phis, xtp1s, RLS_TARGET_PREDICT, True, False, RLS_PROJECT_NONE)
+        return self._rls(phis, xtp1s, "theta_update2")
 
 
 class DecentralizedLQRYankOmega(_DecentralizedBase):
@@ -290,6 +314,7 @@ class DecentralizedLQRYankOmega(_DecentralizedBase):
     index a 9-dim layout and raise in the reference (3 x 3 rotation applied to 4 entries); here they follow the
     LQRYankOmegaController error state (lqr_YO_controller.py:106-116), which is what the crazyflie variant's YOState does."""
     VARIANT, M = _lib.CTRL_LQR_YANK, 10
+    RLS_METHODS = {"theta_update": (RLS_TARGET_PREDICT, True, True, RLS_PROJECT_NONE)}
 
     def _weights(self):
         env = self.env  # decentralized_lqr_yank_omega.py:20-41
@@ -303,12 +328,13 @@ class DecentralizedLQRYankOmega(_DecentralizedBase):
 
     def theta_update(self, phis, xtp1s):
         """:112-126"""
-        return self._rls(phis, xtp1s, RLS_TARGET_PREDICT, True, True, RLS_PROJECT_NONE)
+        return self._rls(phis, xtp1s, "theta_update")
 
 
 class DecentralizedYOLQRCrazyflie(DecentralizedLQRYankOmega):
     """control/dlqr/decentralized_yolqr_crazyflie.py: caller-supplied Q / R, P0 = 5 I, x_dot regression with projection."""
     P0_SCALE = 5.0
+    RLS_METHODS = dict(DecentralizedLQRYankOmega.RLS_METHODS, approx_theta_update=(RLS_TARGET_XDOT, False, True, RLS_PROJECT_LOOP))
 
     def __init__(self, env, lin_models, indQ, indR, debug=False, P=None):
         self._qr = (np.asarray(indQ, float), np.asarray(indR, float))
@@ -335,7 +361,7 @@ class DecentralizedYOLQRCrazyflie(DecentralizedLQRYankOmega):
 
     def approx_theta_update(self, phis, xtp1s, project=True):
         """:259-290"""
-        return self._rls(phis, xtp1s, RLS_TARGET_XDOT, False, True, RLS_PROJECT_LOOP if project else RLS_PROJECT_NONE)
+        return self._rls(phis, xtp1s, "approx_theta_update", project=project)
 
 
 class DecentralizedLQR(_DecentralizedBase):
@@ -343,6 +369,8 @@ class DecentralizedLQR(_DecentralizedBase):
     VARIANT, M = _lib.CTRL_LQR_TORQUE, 12
     P0_SCALE = 20.0
     COUPLED = True
+    RLS_METHODS = {"theta_update": (RLS_TARGET_PREDICT, False, True, RLS_PROJECT_AFTER),
+                   "approx_theta_update": (RLS_TARGET_XDOT, False, True, RLS_PROJECT_LOOP)}
 
     def _weights(self):
         mt = self.env.MAX_THRUST  # decentralized_lqr.py:16-34
@@ -375,8 +403,8 @@ class DecentralizedLQR(_DecentralizedBase):
 
     def theta_update(self, phis, xtp1s):
         """:157-183 -- prediction from e_t, project_theta once after the robots' loop."""
-        return self._rls(phis, xtp1s, RLS_TARGET_PREDICT, False, True, RLS_PROJECT_AFTER)
+        return self._rls(phis, xtp1s, "theta_update")
 
     def approx_theta_update(self, phis, xtp1s):
         """:200-228"""
-        return self._rls(phis, xtp1s, RLS_TARGET_XDOT, False, True, RLS_PROJECT_LOOP)
+        return self._rls(phis, xtp1s, "approx_theta_update")

@@ -43,6 +43,7 @@ static int cuda_fail(const char* what, cudaError_t e) {
 
 #include "mds_rollout.cuh"
 #include "mds_rollout_launch.cuh"
+#include "mds_learn_launch.cuh"
 
 template <typename Real>
 __global__ void obs_from_state_kernel(DroneP<Real> P, StateP<Real> st, Real* __restrict__ obs, int D) {
@@ -796,6 +797,47 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   return check_launch("rollout");
 }
 
+template <typename Real>
+static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,
+                                 MdsPidState pid, const typename TrajSpecT<Real>::spec* specs, const typename TrajSpecT<Real>::seg* segs,
+                                 const Real* inputs, Real* theta, Real* Pm, Real* resid, Real* obs, const Real* fext, Real* obs_log, double t0, int K,
+                                 int E, int N, void* stream) {
+  // inputs [K][D*4] may be NULL when K = 0 (an empty excitation tensor has no storage)
+  MDS_REQUIRE(prm && rls && st.pos_wx && st.quat && st.vel_wy && st.rpm && st.wz && pid.a && pid.b && specs && (inputs || K == 0) && theta && Pm &&
+                  obs,
+              "learning_rollout: null pointer");
+  MDS_REQUIRE(variant == MDS_CTRL_LQR_OMEGA || variant == MDS_CTRL_LQR_YANK, "learning_rollout: variant must be LQR_OMEGA or LQR_YANK");
+  MDS_REQUIRE((variant == MDS_CTRL_LQR_OMEGA && rls->m == 9) || (variant == MDS_CTRL_LQR_YANK && rls->m == 10),
+              "learning_rollout: m must be 9 with LQR_OMEGA and 10 with LQR_YANK");
+  MDS_REQUIRE(rls->target == MDS_RLS_TARGET_PREDICT || rls->target == MDS_RLS_TARGET_XDOT, "learning_rollout: unknown target");
+  MDS_REQUIRE(!(rls->target == MDS_RLS_TARGET_XDOT && rls->m == 9), "learning_rollout: the reference defines est_x_dot for m = 10 and 12 only");
+  MDS_REQUIRE(rls->project >= MDS_RLS_PROJECT_NONE && rls->project <= MDS_RLS_PROJECT_LOOP, "learning_rollout: unknown projection mode");
+  // project_theta exists for the 10-dim crazyflie model only (decentralized_yolqr_crazyflie.py:245-257); the m = 9 kernel carries none
+  MDS_REQUIRE(!(rls->m == 9 && rls->project != MDS_RLS_PROJECT_NONE), "learning_rollout: project_theta is defined for m = 10 only");
+  MDS_REQUIRE(rls->dt > 0.0 && rls->drones_per_env == N, "learning_rollout: dt must be positive and drones_per_env equal to N");
+  MDS_REQUIRE(K >= 0 && E > 0 && N >= 1 && N <= MDS_MAX_DRONES_PER_ENV, "learning_rollout: bad K, E or N");
+  MDS_REQUIRE(prm->substeps >= 1, "learning_rollout: substeps must be >= 1");
+  MDS_REQUIRE(prm->physics == MDS_PHYSICS_DYN || prm->physics == MDS_PHYSICS_DYN_GND_DRAG_DW, "learning_rollout: unknown physics mode");
+  MDS_REQUIRE(!(write_obs_every > 0) || obs_log, "learning_rollout: obs_log buffer missing");
+  RlsP c;
+  c.target = rls->target; c.predict_from_xtp1 = rls->predict_from_xtp1; c.normalize_gain = rls->normalize_gain;
+  c.project = rls->project; c.drones_per_env = rls->drones_per_env; c.dt = rls->dt;
+  for (int i = 0; i < 16; ++i) c.row_code[i] = 0x55555555u;
+  for (int i = 0; i < rls->m + 4; ++i)
+    for (int j = 0; j < rls->m; ++j) {
+      const unsigned code = rls->theta_code[i * rls->m + j];
+      MDS_REQUIRE(code <= 2, "learning_rollout: theta_code entries must be 0, 1 or 2");
+      c.row_code[i] = (c.row_code[i] & ~(3u << (2 * j))) | (code << (2 * j));
+    }
+  if (K == 0) return MDS_OK;
+  LearnLaunch<Real> a{to_dev<Real>(*prm), c, rls->m, rls->project != MDS_RLS_PROJECT_NONE, learn_from, write_obs_every > 0 ? write_obs_every : 0,
+                      to_dev<Real>(st), to_dev<Real>(pid), specs, segs, inputs, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E, N,
+                      (cudaStream_t)stream};
+  const cudaError_t e = launch_learn_kernel<Real>(a);
+  if (e != cudaSuccess) return cuda_fail("learning_rollout: shared-memory opt-in", e);
+  return check_launch("learning_rollout");
+}
+
 extern "C" {
 
 int mds_abi_version(void) { return MDS_ABI_VERSION; }
@@ -932,6 +974,12 @@ int mds_cbf_num_rows(int order, int N, int n_obs) { return N * (N - 1) / 2 + 8 *
                         int K, int E, int N, void* stream) {                                                                                       \
     return rollout_impl<REAL>(prm, cfg, geo, lqr, cbf, st, pid, dsl, dsl_state, specs, segs, obs, action, fext, obs_log, stats, t0, K, E, N,      \
                               stream);                                                                                                             \
+  }                                                                                                                                                \
+  int mds_learning_rollout_##SUF(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,     \
+                                 MdsPidState pid, const SPEC* specs, const SEG* segs, const REAL* inputs, REAL* theta, REAL* Pm, REAL* resid,      \
+                                 REAL* obs, const REAL* fext, REAL* obs_log, double t0, int K, int E, int N, void* stream) {                       \
+    return learning_rollout_impl<REAL>(prm, rls, variant, learn_from, write_obs_every, st, pid, specs, segs, inputs, theta, Pm, resid, obs, fext,   \
+                                       obs_log, t0, K, E, N, stream);                                                                              \
   }
 
 MDS_DEFINE(f32, float, MdsTrajSpecF32, MdsTrajSegF32)

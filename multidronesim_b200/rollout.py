@@ -14,7 +14,7 @@ from . import _lib
 from .control.dslpid import DSLPIDControl
 from .control.geometric import GeometricControl
 from .control.lqr import LQRController, LQROmegaController, LQRYankOmegaController
-from .control.dlqr import _DecentralizedBase
+from .control.dlqr import DecentralizedLQR, _DecentralizedBase
 
 
 class FusedRollout:
@@ -122,6 +122,66 @@ class FusedRollout:
     def stats_dict(self):
         v = self.stats.tolist()
         return dict(zip(_lib.STAT_NAMES, v))
+
+
+class LearningRollout:
+    """The system-identification loop of the decentralised LQR (the warm-up / learning phases of the reference's
+    simulations/CBFTest.py:150-265 and CBFTestOrd3.py:150-270) for K control steps in ONE launch (``mds_learning_rollout``).
+    Every drone flies the caller's excitation inputs through its inner loop while its RLS model learns from the
+    transitions; theta and P stay in shared memory for the whole launch.  ``run`` equals this per-call loop::
+
+        for k in range(K):
+            dl.set_reference(trajs.eval(t0 + k * dt))
+            e_t = dl.error_state(obs); action = dl.compute_low_level(inputs[k], obs); obs = env.step(action)[0]
+            if k >= learn_from: getattr(dl, method)(torch.cat([e_t, inputs[k]], -1), dl.error_state(obs), **method_kwargs)
+
+    controller: DecentralizedLQROmega, DecentralizedLQRYankOmega or DecentralizedYOLQRCrazyflie (the variants with an inner
+    loop); trajs: TrajectorySet with one trajectory per drone (the references of the error states)."""
+
+    def __init__(self, env, trajs, controller):
+        if isinstance(controller, DecentralizedLQR):
+            raise _lib.MdsError("LearningRollout takes the decentralised LQR variants with an inner loop; the 12-dim torque model "
+                                "has none and a robot-coupled gain")
+        if not isinstance(controller, _DecentralizedBase):
+            raise TypeError("LearningRollout needs a decentralised LQR controller (control.dlqr)")
+        if trajs.num != env.NUM_TOTAL:
+            raise ValueError("need one trajectory per drone")
+        if controller.env is not env:
+            raise ValueError("the controller belongs to another env")
+        self.env, self.trajs, self.controller = env, trajs, controller
+        self.t = 0.0
+
+    def run(self, inputs, method="theta_update", learn_from=0, t0=None, obs_log=None, log_every=0, **method_kwargs):
+        """inputs [K, E, N, 4] (device, the env's dtype): the excitation of every step (``dl.sigma1()`` draws, say).
+        method: the controller's RLS method (``theta_update``, ``theta_update2``, ``approx_theta_update``), method_kwargs its
+        options (``project``).  The first RLS step is step ``learn_from`` (1 reproduces the reference's ``if i != 0``).
+        ``obs_log`` [K//log_every, E, N, 20] receives the observation after every ``log_every``-th step.  Leaves the env state
+        and obs, the inner loop's PID state, theta, P and ``resid`` (of the last update) as the loop does.  Returns the obs."""
+        env, dl = self.env, self.controller
+        if not isinstance(inputs, torch.Tensor):
+            raise TypeError("inputs must be a torch tensor [K, E, N, 4]")
+        if inputs.dim() != 4 or tuple(inputs.shape[1:]) != (env.NUM_ENVS, env.NUM_DRONES, 4):
+            raise ValueError(f"inputs must have shape [K, {env.NUM_ENVS}, {env.NUM_DRONES}, 4], got {tuple(inputs.shape)}")
+        _lib.require_cuda(inputs, "inputs", env.dtype)
+        cfg = dl.rls_cfg(method, **method_kwargs)
+        K = int(inputs.shape[0])
+        if t0 is None:
+            t0 = self.t
+        if K == 0:  # nothing to run (the C entry point takes K = 0 as well; an empty tensor has no storage to point at)
+            return env._obs
+        write_every = int(log_every) if obs_log is not None else 0
+        if obs_log is not None:
+            _lib.require_cuda(obs_log, "obs_log", env.dtype)
+            if write_every < 1 or obs_log.numel() < (K // write_every) * env.NUM_TOTAL * _lib.OBS_DIM:
+                raise ValueError("obs_log too small or log_every < 1")
+        _lib.call("mds_learning_rollout", env.dtype, env._prm, cfg, dl.VARIANT, int(learn_from), write_every, env._state_struct(),
+                  dl.low_level.pid_struct(), _lib.ptr(self.trajs.specs), _lib.ptr(self.trajs.segs), _lib.ptr(inputs), _lib.ptr(dl.theta_planes),
+                  _lib.ptr(dl.P_planes), _lib.ptr(dl.resid), _lib.ptr(env._obs), _lib.ptr(env._ext_force), _lib.ptr(obs_log), float(t0), K,
+                  env.NUM_ENVS, env.NUM_DRONES, _lib.stream_ptr(env.device))
+        env.step_counter += K * env.PYB_STEPS_PER_CTRL
+        dl.low_level.control_counter += K
+        self.t = t0 + K * env.CTRL_TIMESTEP
+        return env._obs
 
 
 class PerCallPipeline:
