@@ -476,14 +476,13 @@ static int lqr_impl(const MdsDroneParams* prm, const MdsLqrGains* g, int variant
                                                                              to_dev<Real>(pid), D);
   return check_launch("lqr_ctrl");
 }
-template <typename Real>
-static int rls_impl(const MdsRlsCfg* cfg, const Real* phi, const Real* xtp1, Real* theta, Real* Pm, Real* resid, int D, void* stream) {
-  MDS_REQUIRE(cfg && phi && xtp1 && theta && Pm && D > 0, "rls_update: bad argument");
-  MDS_REQUIRE(cfg->m == 9 || cfg->m == 10 || cfg->m == 12, "rls_update: m must be 9, 10 or 12");
-  MDS_REQUIRE(cfg->target == MDS_RLS_TARGET_PREDICT || cfg->target == MDS_RLS_TARGET_XDOT, "rls_update: unknown target");
-  MDS_REQUIRE(!(cfg->target == MDS_RLS_TARGET_XDOT && cfg->m == 9), "rls_update: the reference defines est_x_dot for m = 10 and 12 only");
-  MDS_REQUIRE(cfg->project >= MDS_RLS_PROJECT_NONE && cfg->project <= MDS_RLS_PROJECT_LOOP, "rls_update: unknown projection mode");
-  MDS_REQUIRE(cfg->dt > 0.0 && cfg->drones_per_env >= 1, "rls_update: dt and drones_per_env must be positive");
+// The MdsRlsCfg checks that mds_rls_update and mds_learning_rollout share, and its translation to the kernels' RlsP
+// (theta_code packed into 2-bit row codes).  cfg->m must already be checked: it sizes the theta_code walk.
+static int rls_params(const MdsRlsCfg* cfg, const char* who, RlsP* out) {
+  if (cfg->target != MDS_RLS_TARGET_PREDICT && cfg->target != MDS_RLS_TARGET_XDOT) return fail(MDS_ERR_ARG, "%s: unknown target", who);
+  if (cfg->target == MDS_RLS_TARGET_XDOT && cfg->m == 9)
+    return fail(MDS_ERR_ARG, "%s: the reference defines est_x_dot for m = 10 and 12 only", who);
+  if (cfg->project < MDS_RLS_PROJECT_NONE || cfg->project > MDS_RLS_PROJECT_LOOP) return fail(MDS_ERR_ARG, "%s: unknown projection mode", who);
   RlsP c;
   c.target = cfg->target; c.predict_from_xtp1 = cfg->predict_from_xtp1; c.normalize_gain = cfg->normalize_gain;
   c.project = cfg->project; c.drones_per_env = cfg->drones_per_env; c.dt = cfg->dt;
@@ -491,9 +490,19 @@ static int rls_impl(const MdsRlsCfg* cfg, const Real* phi, const Real* xtp1, Rea
   for (int i = 0; i < cfg->m + 4; ++i)
     for (int j = 0; j < cfg->m; ++j) {
       const unsigned code = cfg->theta_code[i * cfg->m + j];
-      MDS_REQUIRE(code <= 2, "rls_update: theta_code entries must be 0, 1 or 2");
+      if (code > 2) return fail(MDS_ERR_ARG, "%s: theta_code entries must be 0, 1 or 2", who);
       c.row_code[i] = (c.row_code[i] & ~(3u << (2 * j))) | (code << (2 * j));
     }
+  *out = c;
+  return MDS_OK;
+}
+template <typename Real>
+static int rls_impl(const MdsRlsCfg* cfg, const Real* phi, const Real* xtp1, Real* theta, Real* Pm, Real* resid, int D, void* stream) {
+  MDS_REQUIRE(cfg && phi && xtp1 && theta && Pm && D > 0, "rls_update: bad argument");
+  MDS_REQUIRE(cfg->m == 9 || cfg->m == 10 || cfg->m == 12, "rls_update: m must be 9, 10 or 12");
+  RlsP c;
+  if (const int rc = rls_params(cfg, "rls_update", &c)) return rc;
+  MDS_REQUIRE(cfg->dt > 0.0 && cfg->drones_per_env >= 1, "rls_update: dt and drones_per_env must be positive");
   cudaStream_t cs = (cudaStream_t)stream;
   cudaError_t ae = cudaSuccess;
   // One thread per drone, one warp (f32) / half a warp (f64) per block; P is read from its upper triangle (mds_sysid.cuh).  Round 1's
@@ -809,9 +818,8 @@ static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls
   MDS_REQUIRE(variant == MDS_CTRL_LQR_OMEGA || variant == MDS_CTRL_LQR_YANK, "learning_rollout: variant must be LQR_OMEGA or LQR_YANK");
   MDS_REQUIRE((variant == MDS_CTRL_LQR_OMEGA && rls->m == 9) || (variant == MDS_CTRL_LQR_YANK && rls->m == 10),
               "learning_rollout: m must be 9 with LQR_OMEGA and 10 with LQR_YANK");
-  MDS_REQUIRE(rls->target == MDS_RLS_TARGET_PREDICT || rls->target == MDS_RLS_TARGET_XDOT, "learning_rollout: unknown target");
-  MDS_REQUIRE(!(rls->target == MDS_RLS_TARGET_XDOT && rls->m == 9), "learning_rollout: the reference defines est_x_dot for m = 10 and 12 only");
-  MDS_REQUIRE(rls->project >= MDS_RLS_PROJECT_NONE && rls->project <= MDS_RLS_PROJECT_LOOP, "learning_rollout: unknown projection mode");
+  RlsP c;
+  if (const int rc = rls_params(rls, "learning_rollout", &c)) return rc;
   // project_theta exists for the 10-dim crazyflie model only (decentralized_yolqr_crazyflie.py:245-257); the m = 9 kernel carries none
   MDS_REQUIRE(!(rls->m == 9 && rls->project != MDS_RLS_PROJECT_NONE), "learning_rollout: project_theta is defined for m = 10 only");
   MDS_REQUIRE(rls->dt > 0.0 && rls->drones_per_env == N, "learning_rollout: dt must be positive and drones_per_env equal to N");
@@ -819,16 +827,6 @@ static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls
   MDS_REQUIRE(prm->substeps >= 1, "learning_rollout: substeps must be >= 1");
   MDS_REQUIRE(prm->physics == MDS_PHYSICS_DYN || prm->physics == MDS_PHYSICS_DYN_GND_DRAG_DW, "learning_rollout: unknown physics mode");
   MDS_REQUIRE(!(write_obs_every > 0) || obs_log, "learning_rollout: obs_log buffer missing");
-  RlsP c;
-  c.target = rls->target; c.predict_from_xtp1 = rls->predict_from_xtp1; c.normalize_gain = rls->normalize_gain;
-  c.project = rls->project; c.drones_per_env = rls->drones_per_env; c.dt = rls->dt;
-  for (int i = 0; i < 16; ++i) c.row_code[i] = 0x55555555u;
-  for (int i = 0; i < rls->m + 4; ++i)
-    for (int j = 0; j < rls->m; ++j) {
-      const unsigned code = rls->theta_code[i * rls->m + j];
-      MDS_REQUIRE(code <= 2, "learning_rollout: theta_code entries must be 0, 1 or 2");
-      c.row_code[i] = (c.row_code[i] & ~(3u << (2 * j))) | (code << (2 * j));
-    }
   if (K == 0) return MDS_OK;
   LearnLaunch<Real> a{to_dev<Real>(*prm), c, rls->m, rls->project != MDS_RLS_PROJECT_NONE, learn_from, write_obs_every > 0 ? write_obs_every : 0,
                       to_dev<Real>(st), to_dev<Real>(pid), specs, segs, inputs, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E, N,

@@ -13,128 +13,6 @@
 #include "mds_learn_launch.cuh"
 #include "mds_rollout.cuh"
 
-// ---- the sweeps of one RLS step over a thread's staged columns: the arithmetic of rls_update_kernel (mds_sysid.cuh) in the
-// same order, with a run-time thread stride T.  Shared memory is [entry][thread]; sP is the packed upper triangle of P, sT
-// theta, s_phi / s_w / s_term scratch columns (MN, MN, M entries), all already offset to the calling thread.
-// (rls_update_kernel keeps its own copy: calling these from it changed its fp64 SASS by 16-24 instructions per variant.)
-
-// project_theta before the update (MDS_RLS_PROJECT_LOOP, robots after the first of an env): s_code holds the codes per theta row
-template <typename Real, int M> MDS_DEV void rls_pre_project(Real* sT, const unsigned* s_code, int T) {
-  constexpr int MN = M + 4;
-#pragma unroll 1
-  for (int i = 0; i < MN; ++i) {
-    const unsigned word = s_code[i];
-#pragma unroll
-    for (int j = 0; j < M; ++j) {
-      const unsigned code = (word >> (2 * j)) & 3u;
-      if (code != 1u) sT[(i * M + j) * T] = code == 0u ? Real(0) : Real(1);
-    }
-  }
-}
-
-// gain: w = P phi (= v'), s = 1 + phi' P phi; returns s.  v[] must be zero on entry and holds w on return (also in s_w).
-// Row i of the triangle holds P(i, j >= i): it contributes P(i,j) phi_j to w_i and, for j > i, P(i,j) phi_i to w_j.  The
-// run-time row loop of the fp64 RLS kernel in both precisions (the fully unrolled fp32 form takes 255 registers on its own):
-// the row's own part of w_i goes to shared memory, the transposed contributions to v[j] with static j.
-template <typename Real, int MN>
-MDS_DEV Real rls_gain(const Real* sP, const Real* s_phi, Real* s_w, const Real (&phi)[MN], Real (&v)[MN], int T) {
-  Real s = Real(1);
-#pragma unroll 2
-  for (int i = 0; i < MN; ++i) {
-    const Real phi_i = s_phi[i * T];
-    Real wi = Real(0);
-    const int row0 = i * MN - i * (i - 1) / 2 - i;  // rls_tri(i, j) = row0 + j
-#pragma unroll
-    for (int j = 0; j < MN; ++j) {
-      if (j >= i) {
-        const Real p = sP[(row0 + j) * T];
-        wi += p * phi[j];
-        if (j > i) v[j] += p * phi_i;
-      }
-    }
-    s_w[i * T] = wi;
-  }
-#pragma unroll
-  for (int i = 0; i < MN; ++i) v[i] += s_w[i * T];
-#pragma unroll
-  for (int i = 0; i < MN; ++i) { s_w[i * T] = v[i]; s += phi[i] * v[i]; }
-  return s;
-}
-
-// regression residual r (m) of the staged theta: est_x_dot - theta' phi (XDOT) or x1 - forward_predict (PREDICT)
-template <typename Real, int M>
-MDS_DEV void rls_residual(const RlsP& c, const Real (&phi)[M + 4], const Real (&x1)[M], const Real* s_phi, const Real* sT, Real* s_term,
-                          Real (&r)[M], int T) {
-  constexpr int MN = M + 4;
-  if (c.target == MDS_RLS_TARGET_XDOT) {
-    // est_x_dot, then x_dot - theta' phi
-    const Real inv_dt = Real(1.0 / c.dt);
-    if (M == 12) {  // decentralized_lqr.py:185-198
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        r[k] = x1[3 + k];
-        r[3 + k] = (x1[3 + k] - phi[3 + k]) * inv_dt;
-        r[6 + k] = (x1[6 + k] - phi[6 + k]) * inv_dt;
-        r[9 + k] = x1[6 + k];
-      }
-    } else {  // decentralized_yolqr_crazyflie.py:228-243 (m = 10; m = 9 is rejected on the host)
-#pragma unroll
-      for (int k = 0; k < 3; ++k) {
-        r[k] = phi[M + 1 + k];
-        r[4 + k] = (x1[4 + k] - phi[4 + k]) * inv_dt;
-        r[7 + k] = x1[4 + k];
-      }
-      r[3] = phi[M];
-    }
-#pragma unroll kRlsRowUnroll
-    for (int i = 0; i < MN; ++i) {
-      const Real phi_i = s_phi[i * T];
-#pragma unroll
-      for (int j = 0; j < M; ++j) r[j] -= sT[(i * M + j) * T] * phi_i;
-    }
-  } else {
-    // forward_predict: e' = Ahat e + Bhat u over dt from e0, Ahat = theta[:m]^T, Bhat = theta[m:]^T.  The reference runs
-    // scipy RK45 (its error over one 1/240 s step is far below its 1e-3 tolerance); here the exact solution
-    // e(dt) = e0 + sum_{k>=1} dt^k / k! A^(k-1) (A e0 + B u), summed until the terms vanish in Real.
-    Real acc[M], nt[M];
-#pragma unroll
-    for (int j = 0; j < M; ++j) {
-      acc[j] = c.predict_from_xtp1 ? x1[j] : phi[j];
-      s_term[j * T] = acc[j];
-      nt[j] = Real(0);
-    }
-#pragma unroll kRlsRowUnroll
-    for (int i = 0; i < MN; ++i) {  // A e0 + B u = theta' [e0; u]
-      const Real zi = i < M ? s_term[i * T] : s_phi[i * T];
-#pragma unroll
-      for (int j = 0; j < M; ++j) nt[j] += sT[(i * M + j) * T] * zi;
-    }
-    Real coef = Real(c.dt);
-    const Real eps = sizeof(Real) == 4 ? Real(1e-9) : Real(1e-18);
-#pragma unroll 1
-    for (int k = 1; k <= 16; ++k) {
-      Real big = Real(0), mag = Real(0);
-#pragma unroll
-      for (int j = 0; j < M; ++j) {
-        const Real inc = coef * nt[j];
-        acc[j] += inc;
-        big = max_(big, abs_(inc)); mag = max_(mag, abs_(acc[j]));
-        s_term[j * T] = nt[j]; nt[j] = Real(0);
-      }
-      if (big <= eps * mag) break;  // the series has converged in Real (|A| dt ~ 0.05: 5-7 terms)
-      coef *= Real(c.dt) / Real(k + 1);
-#pragma unroll kRlsRowUnroll
-      for (int i = 0; i < M; ++i) {
-        const Real ti = s_term[i * T];
-#pragma unroll
-        for (int j = 0; j < M; ++j) nt[j] += sT[(i * M + j) * T] * ti;
-      }
-    }
-#pragma unroll
-    for (int j = 0; j < M; ++j) r[j] = x1[j] - acc[j];
-  }
-}
-
 // Threads per block: the RLS kernel's (one warp in fp32, half a warp in fp64; the staged columns set the occupancy),
 // raised to the lane-group size NP where that is larger.  Both are at most 32.
 template <typename Real, int M> static int learn_threads(int NP) { return rls_threads<Real, M>() > NP ? rls_threads<Real, M>() : NP; }
@@ -209,7 +87,8 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
       log_countdown = write_obs_every;
     }
     if (!g.valid || k < learn_from) continue;
-    // ---- one RLS step in the staged columns: phi = [e_t, u], x1 = e_t+1 against the same reference sample
+    // ---- one RLS step in the staged columns (the sweeps of mds_sysid.cuh): phi = [e_t, u], x1 = e_t+1 against the same
+    // reference sample
     Real e1[12], phi[MN], x1[M], v[MN];
     lqr_error_state(P, CTRL, o, ref, e1);
 #pragma unroll

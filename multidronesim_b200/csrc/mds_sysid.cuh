@@ -39,110 +39,63 @@ template <int MN> MDS_DEV constexpr int rls_tri(int i, int j) { return i * MN - 
 // load / compute / store phases overlap; measured at 1 M drones, m = 9 f32: 0.61 ms at 32 threads, 0.80 ms at 64 or 128.
 // Row loops over the staged columns: unrolled by 4 so that several rows' shared-memory loads are in flight (registers are
 // free here: occupancy is set by the staging footprint, not by registers).
-#ifndef MDS_RLS_ROW_UNROLL
-#define MDS_RLS_ROW_UNROLL 4
-#endif
-constexpr int kRlsRowUnroll = MDS_RLS_ROW_UNROLL;  // (#pragma unroll takes a constant expression, not a macro)
-#ifndef MDS_RLS_T32
-#define MDS_RLS_T32 32
-#endif
-template <typename Real, int M> constexpr int rls_threads() { return sizeof(Real) == 4 ? MDS_RLS_T32 : MDS_RLS_T32 / 2; }
+constexpr int kRlsRowUnroll = 4;  // (#pragma unroll takes a constant expression, not a macro)
+template <typename Real, int M> constexpr int rls_threads() { return sizeof(Real) == 4 ? 32 : 16; }
 
-// One RLS step for drone d.  phi = [e_t (m), u_t (4)], x1 = e_{t+1} (m).
-// Both matrices are needed twice (gain / prediction over the WHOLE matrix first, rank-one update second), and a swarm's
-// in-flight footprint (1.1 KB per drone) exceeds L2, so a second sweep over HBM planes would double the traffic.  Each
-// thread therefore stages its own columns of P and theta in shared memory ([entry][thread]: conflict-free) with cp.async,
-// works there (run-time row loops, register-resident column vectors) and writes the updated entries straight back:
-// HBM sees every entry once in and once out.  A thread only ever touches its own shared column.
-// PROJECT: whether project_theta is applied at all (compile-time: the unprojected variants carry none of its code)
-template <typename Real, int M, bool PROJECT>
-__global__ void __launch_bounds__(rls_threads<Real, M>()) rls_update_kernel(RlsP c, const Real* __restrict__ phi_in, const Real* __restrict__ x1_in,
-                                                                         Real* __restrict__ theta, Real* __restrict__ Pm, Real* __restrict__ resid_out,
-                                                                         int D_) {
-  constexpr int MN = M + 4, T = rls_threads<Real, M>();
-  extern __shared__ __align__(16) unsigned char rls_smem[];
-  const int tid = threadIdx.x;
-  constexpr int TRI = MN * (MN + 1) / 2;
-  Real* sP = reinterpret_cast<Real*>(rls_smem) + tid;  // packed upper triangle of P: entry (i, j >= i) at sP[rls_tri<MN>(i, j) * T]
-  Real* sT = sP + TRI * T;
-  Real* s_phi = sT + MN * M * T;
-  Real* s_w = s_phi + MN * T;
-  Real* s_term = s_w + MN * T;
-  // project_theta codes per theta row, block-shared (a parameter array indexed by the run-time row would be copied to
-  // local memory); the only block barrier of the kernel, before any thread leaves
-  __shared__ unsigned s_code[16];
-  if (PROJECT && tid == 0) {
-#pragma unroll
-    for (int i = 0; i < MN; ++i) s_code[i] = c.row_code[i];
-  }
-  if (PROJECT) __syncthreads();
-  const size_t d = (size_t)blockIdx.x * T + tid, D = (size_t)D_;
-  if (d >= D) return;
+// ---- the sweeps of one RLS step over a thread's staged columns, shared by rls_update_kernel and learn_rollout_kernel
+// (mds_learn.cuh).  Shared memory is [entry][thread] with thread stride T (a constant in rls_update_kernel, the block size
+// in learn_rollout_kernel); sP is the packed upper triangle of P, sT theta, s_phi / s_w / s_term scratch columns (MN, MN,
+// M entries), all already offset to the calling thread.
+
+// project_theta before the update (MDS_RLS_PROJECT_LOOP, robots after the first of an env): s_code holds the codes per theta row
+template <typename Real, int M> MDS_DEV void rls_pre_project(Real* sT, const unsigned* s_code, int T) {
+  constexpr int MN = M + 4;
 #pragma unroll 1
-  for (int i = 0; i < MN; ++i)
-#pragma unroll 1
-    for (int j = i; j < MN; ++j) cp_async_real(sP + rls_tri<MN>(i, j) * T, Pm + (size_t)(i * MN + j) * D + d);
-#pragma unroll 1
-  for (int k = 0; k < MN * M; ++k) cp_async_real(sT + k * T, theta + (size_t)k * D + d);
-  Real x1[M], phi[MN], v[MN];  // v = phi' P = (P phi)' = w' by symmetry: accumulated from both halves of the triangle
+  for (int i = 0; i < MN; ++i) {
+    const unsigned word = s_code[i];
 #pragma unroll
-  for (int i = 0; i < MN; ++i) { phi[i] = phi_in[d * MN + i]; s_phi[i * T] = phi[i]; v[i] = Real(0); }
-#pragma unroll
-  for (int i = 0; i < M; ++i) x1[i] = x1_in[d * M + i];
-  cp_async_wait_all();
-  // robots after the first of an env see the projection of the earlier robots' loop iterations before their own update
-  const bool pre_project = PROJECT && c.project == MDS_RLS_PROJECT_LOOP && (d % (size_t)c.drones_per_env) != 0;
-  if (pre_project) {
-#pragma unroll 1
-    for (int i = 0; i < MN; ++i) {
-      const unsigned word = s_code[i];
-#pragma unroll
-      for (int j = 0; j < M; ++j) {
-        const unsigned code = (word >> (2 * j)) & 3u;
-        if (code != 1u) sT[(i * M + j) * T] = code == 0u ? Real(0) : Real(1);
-      }
+    for (int j = 0; j < M; ++j) {
+      const unsigned code = (word >> (2 * j)) & 3u;
+      if (code != 1u) sT[(i * M + j) * T] = code == 0u ? Real(0) : Real(1);
     }
   }
-  // ---- gain: w = P phi (= v'), s = 1 + phi' P phi.  Row i of the triangle holds P(i, j >= i): it contributes P(i,j) phi_j to w_i and,
-  // for j > i, P(i,j) phi_i to w_j
+}
+
+// gain: w = P phi (= v'), s = 1 + phi' P phi; returns s.  v[] must be zero on entry and holds w on return (also in s_w).
+// Row i of the triangle holds P(i, j >= i): it contributes P(i,j) phi_j to w_i and, for j > i, P(i,j) phi_i to w_j.  The
+// fp64 RLS kernel's run-time row loop, used by learn_rollout_kernel in both precisions (the fully unrolled fp32 form takes
+// 255 registers on its own): the row's own part of w_i goes to shared memory, the transposed contributions to v[j] with
+// static j; the two halves are joined afterwards.
+template <typename Real, int MN>
+MDS_DEV Real rls_gain(const Real* sP, const Real* s_phi, Real* s_w, const Real (&phi)[MN], Real (&v)[MN], int T) {
   Real s = Real(1);
-  if (sizeof(Real) == 4) {  // fully unrolled: every index is static, w lives in v[] (255 registers in fp32, no spills)
-#pragma unroll
-    for (int i = 0; i < MN; ++i) {
-      Real wi = v[i];
-#pragma unroll
-      for (int j = i; j < MN; ++j) {
-        const Real p = sP[rls_tri<MN>(i, j) * T];
-        wi += p * phi[j];
-        if (j > i) v[j] += p * phi[i];
-      }
-      v[i] = wi;
-    }
-  } else {  // fp64: a run-time row loop (the full unroll spills 850 B): the row's own part of w_i goes to shared memory, the
-            // transposed contributions to v[j] with static j; the two halves are joined afterwards
 #pragma unroll 2
-    for (int i = 0; i < MN; ++i) {
-      const Real phi_i = s_phi[i * T];
-      Real wi = Real(0);
-      const int row0 = i * MN - i * (i - 1) / 2 - i;  // rls_tri(i, j) = row0 + j
+  for (int i = 0; i < MN; ++i) {
+    const Real phi_i = s_phi[i * T];
+    Real wi = Real(0);
+    const int row0 = i * MN - i * (i - 1) / 2 - i;  // rls_tri(i, j) = row0 + j
 #pragma unroll
-      for (int j = 0; j < MN; ++j) {
-        if (j >= i) {
-          const Real p = sP[(row0 + j) * T];
-          wi += p * phi[j];
-          if (j > i) v[j] += p * phi_i;
-        }
+    for (int j = 0; j < MN; ++j) {
+      if (j >= i) {
+        const Real p = sP[(row0 + j) * T];
+        wi += p * phi[j];
+        if (j > i) v[j] += p * phi_i;
       }
-      s_w[i * T] = wi;
     }
-#pragma unroll
-    for (int i = 0; i < MN; ++i) v[i] += s_w[i * T];
+    s_w[i * T] = wi;
   }
+#pragma unroll
+  for (int i = 0; i < MN; ++i) v[i] += s_w[i * T];
 #pragma unroll
   for (int i = 0; i < MN; ++i) { s_w[i * T] = v[i]; s += phi[i] * v[i]; }
-  const Real inv_s = Real(1) / s;
-  // ---- regression residual r (m)
-  Real r[M];
+  return s;
+}
+
+// regression residual r (m) of the staged theta: est_x_dot - theta' phi (XDOT) or x1 - forward_predict (PREDICT)
+template <typename Real, int M>
+MDS_DEV void rls_residual(const RlsP& c, const Real (&phi)[M + 4], const Real (&x1)[M], const Real* s_phi, const Real* sT, Real* s_term,
+                          Real (&r)[M], int T) {
+  constexpr int MN = M + 4;
   if (c.target == MDS_RLS_TARGET_XDOT) {
     // est_x_dot, then x_dot - theta' phi
     const Real inv_dt = Real(1.0 / c.dt);
@@ -210,6 +163,92 @@ __global__ void __launch_bounds__(rls_threads<Real, M>()) rls_update_kernel(RlsP
 #pragma unroll
     for (int j = 0; j < M; ++j) r[j] = x1[j] - acc[j];
   }
+}
+
+// One RLS step for drone d.  phi = [e_t (m), u_t (4)], x1 = e_{t+1} (m).
+// Both matrices are needed twice (gain / prediction over the WHOLE matrix first, rank-one update second), and a swarm's
+// in-flight footprint (1.1 KB per drone) exceeds L2, so a second sweep over HBM planes would double the traffic.  Each
+// thread therefore stages its own columns of P and theta in shared memory ([entry][thread]: conflict-free) with cp.async,
+// works there (run-time row loops, register-resident column vectors) and writes the updated entries straight back:
+// HBM sees every entry once in and once out.  A thread only ever touches its own shared column.
+// PROJECT: whether project_theta is applied at all (compile-time: the unprojected variants carry none of its code)
+template <typename Real, int M, bool PROJECT>
+__global__ void __launch_bounds__(rls_threads<Real, M>()) rls_update_kernel(RlsP c, const Real* __restrict__ phi_in, const Real* __restrict__ x1_in,
+                                                                         Real* __restrict__ theta, Real* __restrict__ Pm, Real* __restrict__ resid_out,
+                                                                         int D_) {
+  constexpr int MN = M + 4, T = rls_threads<Real, M>();
+  extern __shared__ __align__(16) unsigned char rls_smem[];
+  const int tid = threadIdx.x;
+  constexpr int TRI = MN * (MN + 1) / 2;
+  Real* sP = reinterpret_cast<Real*>(rls_smem) + tid;  // packed upper triangle of P: entry (i, j >= i) at sP[rls_tri<MN>(i, j) * T]
+  Real* sT = sP + TRI * T;
+  Real* s_phi = sT + MN * M * T;
+  Real* s_w = s_phi + MN * T;
+  Real* s_term = s_w + MN * T;
+  // project_theta codes per theta row, block-shared (a parameter array indexed by the run-time row would be copied to
+  // local memory); the only block barrier of the kernel, before any thread leaves
+  __shared__ unsigned s_code[16];
+  if (PROJECT && tid == 0) {
+#pragma unroll
+    for (int i = 0; i < MN; ++i) s_code[i] = c.row_code[i];
+  }
+  if (PROJECT) __syncthreads();
+  const size_t d = (size_t)blockIdx.x * T + tid, D = (size_t)D_;
+  if (d >= D) return;
+#pragma unroll 1
+  for (int i = 0; i < MN; ++i)
+#pragma unroll 1
+    for (int j = i; j < MN; ++j) cp_async_real(sP + rls_tri<MN>(i, j) * T, Pm + (size_t)(i * MN + j) * D + d);
+#pragma unroll 1
+  for (int k = 0; k < MN * M; ++k) cp_async_real(sT + k * T, theta + (size_t)k * D + d);
+  Real x1[M], phi[MN], v[MN];  // v = phi' P = (P phi)' = w' by symmetry: accumulated from both halves of the triangle
+#pragma unroll
+  for (int i = 0; i < MN; ++i) { phi[i] = phi_in[d * MN + i]; s_phi[i * T] = phi[i]; v[i] = Real(0); }
+#pragma unroll
+  for (int i = 0; i < M; ++i) x1[i] = x1_in[d * M + i];
+  cp_async_wait_all();
+  // robots after the first of an env see the projection of the earlier robots' loop iterations before their own update
+  const bool pre_project = PROJECT && c.project == MDS_RLS_PROJECT_LOOP && (d % (size_t)c.drones_per_env) != 0;
+  if (pre_project) rls_pre_project<Real, M>(sT, s_code, T);
+  // ---- gain: w = P phi (= v'), s = 1 + phi' P phi
+  Real s = Real(1);
+  if (sizeof(Real) == 4) {  // fully unrolled: every index is static, w lives in v[] (255 registers in fp32, no spills)
+#pragma unroll
+    for (int i = 0; i < MN; ++i) {
+      Real wi = v[i];
+#pragma unroll
+      for (int j = i; j < MN; ++j) {
+        const Real p = sP[rls_tri<MN>(i, j) * T];
+        wi += p * phi[j];
+        if (j > i) v[j] += p * phi[i];
+      }
+      v[i] = wi;
+    }
+  } else {  // fp64: rls_gain's row loop, inline (rls_gain itself costs this kernel 16-24 more instructions per variant, all
+            // address arithmetic: the loads lose their shared base register with immediate offsets)
+#pragma unroll 2
+    for (int i = 0; i < MN; ++i) {
+      const Real phi_i = s_phi[i * T];
+      Real wi = Real(0);
+      const int row0 = i * MN - i * (i - 1) / 2 - i;  // rls_tri(i, j) = row0 + j
+#pragma unroll
+      for (int j = 0; j < MN; ++j) {
+        if (j >= i) {
+          const Real p = sP[(row0 + j) * T];
+          wi += p * phi[j];
+          if (j > i) v[j] += p * phi_i;
+        }
+      }
+      s_w[i * T] = wi;
+    }
+#pragma unroll
+    for (int i = 0; i < MN; ++i) v[i] += s_w[i * T];
+  }
+#pragma unroll
+  for (int i = 0; i < MN; ++i) { s_w[i * T] = v[i]; s += phi[i] * v[i]; }
+  const Real inv_s = Real(1) / s;
+  Real r[M];
+  rls_residual<Real, M>(c, phi, x1, s_phi, sT, s_term, r, T);
   if (resid_out) {
 #pragma unroll
     for (int j = 0; j < M; ++j) resid_out[d * M + j] = r[j];

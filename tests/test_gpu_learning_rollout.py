@@ -297,19 +297,21 @@ def test_obs_log_matches_percall_steps(dtype, lib_built):
     assert np.abs(last.double().cpu().numpy()[..., :16] - want[-1][..., :16]).max() <= tol * max(1.0, np.abs(want[-1][..., :16]).max())
 
 
+def cfg(m=9, target=0, project=0, dpe=2, code=1, dt=1 / 48):
+    """an MdsRlsCfg with every theta_code entry set to `code`"""
+    c = _lib.RlsCfg()
+    c.m, c.target, c.predict_from_xtp1, c.normalize_gain, c.project, c.drones_per_env, c.dt = m, target, 1, 1, project, dpe, dt
+    for k in range(16 * 12):
+        c.theta_code[k] = code
+    return c
+
+
 def test_c_argument_errors_do_not_need_a_gpu(lib_built):
     """mds_learning_rollout validates every argument before it launches anything (non-null dummy pointers are never touched)."""
     from multidronesim_b200.constants import DroneConstants
     prm = DroneConstants().c_params()
     p = ctypes.c_void_p(64)
     st, pid = _lib.State(64, 64, 64, 64, 64), _lib.PidState(64, 64)
-
-    def cfg(m=9, target=0, project=0, dpe=2, code=1):
-        c = _lib.RlsCfg()
-        c.m, c.target, c.predict_from_xtp1, c.normalize_gain, c.project, c.drones_per_env, c.dt = m, target, 1, 1, project, dpe, 1 / 48
-        for k in range(16 * 12):
-            c.theta_code[k] = code
-        return c
 
     def call(c, variant=_lib.CTRL_LQR_OMEGA, K=4, E=3, N=2, null=False, fn=lib_built.mds_learning_rollout_f32):
         q = None if null else p
@@ -342,3 +344,30 @@ def test_c_argument_errors_do_not_need_a_gpu(lib_built):
     assert lib_built.mds_learning_rollout_f32(prm, c, _lib.CTRL_LQR_OMEGA, 0, 0, st, pid, p, p, None, p, p, None, p, None, None, 0.0, 0, 3, 2, None) == 0
     rc = lib_built.mds_learning_rollout_f32(prm, c, _lib.CTRL_LQR_OMEGA, 0, 0, st, pid, p, p, None, p, p, None, p, None, None, 0.0, 1, 3, 2, None)
     assert rc == -1 and b"null pointer" in lib_built.mds_last_error()
+
+
+def test_rls_update_c_argument_errors_do_not_need_a_gpu(lib_built):
+    """mds_rls_update refuses a bad configuration or argument before it launches anything (the dummy pointers are never touched)."""
+    p = ctypes.c_void_p(64)
+
+    def call(c, D=6, null=False, fn=lib_built.mds_rls_update_f32):
+        return fn(c, None if null else p, p, p, p, None, D, None)
+
+    cases = [
+        (dict(c=cfg(), null=True), b"bad argument"),
+        (dict(c=cfg(), D=0), b"bad argument"),
+        (dict(c=cfg(m=11)), b"m must be 9, 10 or 12"),
+        (dict(c=cfg(target=2), fn=lib_built.mds_rls_update_f64), b"unknown target"),
+        (dict(c=cfg(m=9, target=1)), b"est_x_dot"),
+        (dict(c=cfg(m=10, project=3)), b"unknown projection mode"),
+        (dict(c=cfg(m=12, project=-1), fn=lib_built.mds_rls_update_f64), b"unknown projection mode"),
+        (dict(c=cfg(dt=0.0)), b"dt and drones_per_env must be positive"),
+        (dict(c=cfg(dt=-1 / 48), fn=lib_built.mds_rls_update_f64), b"dt and drones_per_env must be positive"),
+        (dict(c=cfg(dpe=0)), b"dt and drones_per_env must be positive"),
+        (dict(c=cfg(m=10, target=1, project=2, code=3)), b"theta_code"),
+        (dict(c=cfg(m=12, code=3), fn=lib_built.mds_rls_update_f64), b"theta_code"),
+    ]
+    for kw, msg in cases:
+        rc = call(**kw)
+        err = lib_built.mds_last_error()
+        assert rc == -1 and err.startswith(b"rls_update: ") and msg in err, (kw, err)
