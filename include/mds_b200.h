@@ -369,6 +369,21 @@ int mds_learning_rollout_f64(const MdsDroneParams* prm, const MdsRlsCfg* rls, in
                              MdsPidState pid, const MdsTrajSpecF64* specs_dev, const MdsTrajSegF64* segs_dev, const double* inputs_dev,
                              double* theta_dev, double* P_dev, double* resid_dev, double* obs_dev, const double* ext_force_dev, double* obs_log_dev,
                              double t0, int K, int E, int N, void* stream);
+/* mds_learning_rollout under each drone's own gain (closed-loop exploration): the inner loop flies
+ * u_k = -K_d e_t (+ m g unless MDS_CTRL_LQR_YANK; MDS_CTRL_LQR_OMEGA caps the thrust as mds_dlqr_ctrl does) + inputs_dev[k],
+ * and the RLS step takes phi = [e_t, u_k] with that applied u_k.  inputs_dev[k] [D*4] are perturbations of the law (with
+ * LQR_YANK, entry 0 perturbs the yank).  gain_dev [4*m][D]: the uncoupled planes of mds_dlqr_ctrl, non-NULL, read once
+ * per launch (constant for its K steps).  The same results as the mds_learning_rollout loop with mds_dlqr_ctrl (no
+ * action) and an add before mds_lowlevel; every other argument and check is mds_learning_rollout's. */
+int mds_learning_rollout_feedback_f32(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every,
+                                      MdsState st, MdsPidState pid, const MdsTrajSpecF32* specs_dev, const MdsTrajSegF32* segs_dev,
+                                      const float* inputs_dev, const float* gain_dev, float* theta_dev, float* P_dev, float* resid_dev,
+                                      float* obs_dev, const float* ext_force_dev, float* obs_log_dev, double t0, int K, int E, int N, void* stream);
+int mds_learning_rollout_feedback_f64(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every,
+                                      MdsState st, MdsPidState pid, const MdsTrajSpecF64* specs_dev, const MdsTrajSegF64* segs_dev,
+                                      const double* inputs_dev, const double* gain_dev, double* theta_dev, double* P_dev, double* resid_dev,
+                                      double* obs_dev, const double* ext_force_dev, double* obs_log_dev, double t0, int K, int E, int N,
+                                      void* stream);
 
 /* compute_controller (decentralized_lqr_omega.py:185-204): K_d = R^-1 B_d' X_d, X_d the stabilising solution of the
  * continuous-time algebraic Riccati equation of drone d's learned model theta_d = [A_d, B_d]^T, for diagonal Q (q_diag [m])

@@ -124,6 +124,8 @@ _SIGS = {
     "mds_rollout": [_PRM, C.POINTER(RolloutCfg), C.POINTER(GeoGains), C.POINTER(LqrGains), C.POINTER(CbfParams),
                     State, PidState, C.POINTER(DslPidGains), DslPidState, _P, _P, _P, _P, _P, _P, _P, _D, _I, _I, _I, _P],
     "mds_learning_rollout": [_PRM, C.POINTER(RlsCfg), _I, _I, _I, State, PidState, _P, _P, _P, _P, _P, _P, _P, _P, _P, _D, _I, _I, _I, _P],
+    "mds_learning_rollout_feedback": [_PRM, C.POINTER(RlsCfg), _I, _I, _I, State, PidState, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _D, _I, _I,
+                                      _I, _P],
 }
 _PLAIN = {
     "mds_abi_version": ([], _I),

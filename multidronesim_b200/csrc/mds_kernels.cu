@@ -809,9 +809,9 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
 template <typename Real>
 static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,
                                  MdsPidState pid, const typename TrajSpecT<Real>::spec* specs, const typename TrajSpecT<Real>::seg* segs,
-                                 const Real* inputs, Real* theta, Real* Pm, Real* resid, Real* obs, const Real* fext, Real* obs_log, double t0, int K,
-                                 int E, int N, void* stream) {
-  // inputs [K][D*4] may be NULL when K = 0 (an empty excitation tensor has no storage)
+                                 const Real* inputs, const Real* gain, Real* theta, Real* Pm, Real* resid, Real* obs, const Real* fext, Real* obs_log,
+                                 double t0, int K, int E, int N, void* stream) {
+  // inputs [K][D*4] may be NULL when K = 0 (an empty excitation tensor has no storage); gain: NULL flies the inputs open loop
   MDS_REQUIRE(prm && rls && st.pos_wx && st.quat && st.vel_wy && st.rpm && st.wz && pid.a && pid.b && specs && (inputs || K == 0) && theta && Pm &&
                   obs,
               "learning_rollout: null pointer");
@@ -829,7 +829,7 @@ static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls
   MDS_REQUIRE(!(write_obs_every > 0) || obs_log, "learning_rollout: obs_log buffer missing");
   if (K == 0) return MDS_OK;
   LearnLaunch<Real> a{to_dev<Real>(*prm), c, rls->m, rls->project != MDS_RLS_PROJECT_NONE, learn_from, write_obs_every > 0 ? write_obs_every : 0,
-                      to_dev<Real>(st), to_dev<Real>(pid), specs, segs, inputs, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E, N,
+                      to_dev<Real>(st), to_dev<Real>(pid), specs, segs, inputs, gain, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E, N,
                       (cudaStream_t)stream};
   const cudaError_t e = launch_learn_kernel<Real>(a);
   if (e != cudaSuccess) return cuda_fail("learning_rollout: shared-memory opt-in", e);
@@ -976,8 +976,16 @@ int mds_cbf_num_rows(int order, int N, int n_obs) { return N * (N - 1) / 2 + 8 *
   int mds_learning_rollout_##SUF(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,     \
                                  MdsPidState pid, const SPEC* specs, const SEG* segs, const REAL* inputs, REAL* theta, REAL* Pm, REAL* resid,      \
                                  REAL* obs, const REAL* fext, REAL* obs_log, double t0, int K, int E, int N, void* stream) {                       \
-    return learning_rollout_impl<REAL>(prm, rls, variant, learn_from, write_obs_every, st, pid, specs, segs, inputs, theta, Pm, resid, obs, fext,   \
-                                       obs_log, t0, K, E, N, stream);                                                                              \
+    return learning_rollout_impl<REAL>(prm, rls, variant, learn_from, write_obs_every, st, pid, specs, segs, inputs, (const REAL*)nullptr, theta,  \
+                                       Pm, resid, obs, fext, obs_log, t0, K, E, N, stream);                                                        \
+  }                                                                                                                                                \
+  int mds_learning_rollout_feedback_##SUF(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every,       \
+                                          MdsState st, MdsPidState pid, const SPEC* specs, const SEG* segs, const REAL* inputs,                    \
+                                          const REAL* gain, REAL* theta, REAL* Pm, REAL* resid, REAL* obs, const REAL* fext, REAL* obs_log,        \
+                                          double t0, int K, int E, int N, void* stream) {                                                          \
+    MDS_REQUIRE(gain, "learning_rollout: null gain pointer");                                                                                      \
+    return learning_rollout_impl<REAL>(prm, rls, variant, learn_from, write_obs_every, st, pid, specs, segs, inputs, gain, theta, Pm, resid, obs,  \
+                                       fext, obs_log, t0, K, E, N, stream);                                                                        \
   }
 
 MDS_DEFINE(f32, float, MdsTrajSpecF32, MdsTrajSegF32)

@@ -8,6 +8,10 @@
 // rls_update_kernel does), keeps them there for all K steps and writes theta and both triangles of P back at the end;
 // state, observation, PID state and trajectory descriptor stay in registers.  Per step HBM sees u[k] (16 or 32 B per
 // drone) and the observation-log slot when one is due.
+// FEEDBACK: closed-loop exploration -- every drone flies its own learned gain plus the caller's perturbation,
+//   u = -K_d e_t (+ m g unless yank-omega; LQR_OMEGA: cap_thrust) + u[k],  phi = [e_t, u]
+// which is the per-call loop with mds_dlqr_ctrl(skip_low_level) and an add before mds_lowlevel.  The gain [4*m][D] planes
+// (mds_dlqr_ctrl's uncoupled layout) are read once per launch and staged next to theta and P: constant within the launch.
 #pragma once
 #include <cuda_runtime.h>
 #include "mds_learn_launch.cuh"
@@ -16,17 +20,21 @@
 // Threads per block: the RLS kernel's (one warp in fp32, half a warp in fp64; the staged columns set the occupancy),
 // raised to the lane-group size NP where that is larger.  Both are at most 32.
 template <typename Real, int M> static int learn_threads(int NP) { return rls_threads<Real, M>() > NP ? rls_threads<Real, M>() : NP; }
+// Staged words per thread: the RLS kernel's columns, plus the 4*M gain entries when FEEDBACK
+template <typename Real, int M, bool FEEDBACK> constexpr int learn_words_per_thread() { return rls_words_per_thread<Real, M>() + (FEEDBACK ? 4 * M : 0); }
 
 // M = 9: DecentralizedLQROmega (LQR_OMEGA error state, ThrustOmega inner loop); M = 10: the yank-omega variants (LQR_YANK,
 // YankOmega inner loop).  PROJECT: project_theta is applied (approx_theta_update(project=True)), compile-time like the RLS kernel.
-template <typename Real, int M, bool PROJECT>
+// FEEDBACK: inputs are perturbations of the law u = -K_d e_t (gain: [4*M][D] planes; the last parameter, so that the open-loop
+// kernels keep their parameter layout); otherwise inputs are the inner loop's inputs and gain is unused.
+template <typename Real, int M, bool PROJECT, bool FEEDBACK>
 __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP c, StateP<Real> st, PidP<Real> pid,
                                                            const typename TrajSpecT<Real>::spec* __restrict__ specs,
                                                            const typename TrajSpecT<Real>::seg* __restrict__ segs,
                                                            const Real* __restrict__ inputs, Real* __restrict__ theta, Real* __restrict__ Pm,
                                                            Real* __restrict__ resid_out, Real* __restrict__ obs, const Real* __restrict__ fext,
                                                            Real* __restrict__ obs_log, double t0, double dt_ctrl, int learn_from, int write_obs_every,
-                                                           int K, int E, int N, int NP) {
+                                                           int K, int E, int N, int NP, const Real* __restrict__ gain) {
   constexpr int MN = M + 4, TRI = MN * (MN + 1) / 2;
   constexpr int CTRL = M == 9 ? MDS_CTRL_LQR_OMEGA : MDS_CTRL_LQR_YANK;
   using R4 = typename Vec4T<Real>::type;
@@ -46,6 +54,7 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
   Real* s_phi = sT + MN * M * T;
   Real* s_w = s_phi + MN * T;
   Real* s_term = s_w + MN * T;
+  Real* sK = s_term + M * T;  // FEEDBACK: gain entry (i, k) of u_i = -sum_k K_ik e_k at sK[(i * M + k) * T]
   const size_t D = (size_t)E * N, d = (size_t)g.d;
   Drone<Real> s;
   Pid<Real> ps;
@@ -59,6 +68,10 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
       for (int j = i; j < MN; ++j) cp_async_real(sP + rls_tri<MN>(i, j) * T, Pm + (size_t)(i * MN + j) * D + d);
 #pragma unroll 1
     for (int k = 0; k < MN * M; ++k) cp_async_real(sT + k * T, theta + (size_t)k * D + d);
+    if (FEEDBACK) {
+#pragma unroll 1
+      for (int k = 0; k < 4 * M; ++k) cp_async_real(sK + k * T, gain + (size_t)k * D + d);
+    }
     s = load_drone(st, g.d);
     ps = load_pid(pid, g.d);
     o = load_obs(obs, g.d);
@@ -78,6 +91,17 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
       ref = eval_traj<Real>(spec, segs, t0 + (double)k * dt_ctrl);  // the time expression of the rollout kernel and its host plans
       lqr_error_state(P, CTRL, o, ref, e0);
       load4(inputs + (size_t)k * D * 4, g.d, u);
+      if (FEEDBACK) {  // dlqr_ctrl_kernel's law and order of operations (skip_low_level: capped, no max(u, 0)), then + u[k]
+        Real uf[4] = {Real(0), Real(0), Real(0), Real(0)};
+#pragma unroll
+        for (int i = 0; i < 4; ++i)
+#pragma unroll
+          for (int j = 0; j < M; ++j) uf[i] -= sK[(i * M + j) * T] * e0[j];
+        if (CTRL != MDS_CTRL_LQR_YANK) uf[0] += P.m * P.g;
+        if (CTRL == MDS_CTRL_LQR_OMEGA) uf[0] = cap_thrust(P, uf[0]);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) u[i] = uf[i] + u[i];
+      }
       low_level(P, CTRL, ps, u, o, rpm);
     }
     o = physics_core<0>(P, s, rpm, fx, sm_pos + (tid - g.n), g, N, NP);

@@ -19,6 +19,7 @@ template <typename Real> struct LearnLaunch {
   const typename TrajSpecT<Real>::spec* specs;
   const typename TrajSpecT<Real>::seg* segs;
   const Real* inputs;  // [K][D*4]
+  const Real* gain;    // [4*m][D] gain planes of the closed-loop law; NULL: inputs are the inner loop's inputs (open loop)
   Real *theta, *Pm, *resid, *obs;
   const Real* fext;
   Real* obs_log;

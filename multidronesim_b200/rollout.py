@@ -135,6 +135,21 @@ class LearningRollout:
             e_t = dl.error_state(obs); action = dl.compute_low_level(inputs[k], obs); obs = env.step(action)[0]
             if k >= learn_from: getattr(dl, method)(torch.cat([e_t, inputs[k]], -1), dl.error_state(obs), **method_kwargs)
 
+    ``run(..., feedback=True)`` is closed-loop exploration (``mds_learning_rollout_feedback``): every drone flies its own
+    learned gain ``dl.K_planes`` plus the perturbation ``inputs[k]`` while its model learns -- the certainty-equivalence loop
+    ``compute_controller() -> run(feedback=True) -> compute_controller() -> ...``.  It equals this per-call loop::
+
+        for k in range(K):
+            dl.set_reference(trajs.eval(t0 + k * dt))
+            e_t = dl.error_state(obs).clone()
+            _, u = dl.compute(obs, skip_low_level=True)   # u = -K_d e_t (+ m g unless yank-omega); LQR_OMEGA: cap_u
+            u = u + inputs[k]                              # exploration perturbation
+            obs = env.step(dl.compute_low_level(u, obs))[0]
+            if k >= learn_from: getattr(dl, method)(torch.cat([e_t, u], -1), dl.error_state(obs), **method_kwargs)
+
+    The gain is read once per launch and stays constant within it (the loop above does not recompute it either), and the
+    feedback acts from step 0 whatever ``learn_from`` is.
+
     controller: DecentralizedLQROmega, DecentralizedLQRYankOmega or DecentralizedYOLQRCrazyflie (the variants with an inner
     loop); trajs: TrajectorySet with one trajectory per drone (the references of the error states)."""
 
@@ -151,8 +166,9 @@ class LearningRollout:
         self.env, self.trajs, self.controller = env, trajs, controller
         self.t = 0.0
 
-    def run(self, inputs, method="theta_update", learn_from=0, t0=None, obs_log=None, log_every=0, **method_kwargs):
-        """inputs [K, E, N, 4] (device, the env's dtype): the excitation of every step (``dl.sigma1()`` draws, say).
+    def run(self, inputs, method="theta_update", learn_from=0, t0=None, obs_log=None, log_every=0, feedback=False, **method_kwargs):
+        """inputs [K, E, N, 4] (device, the env's dtype): the excitation of every step (``dl.sigma1()`` draws, say); with
+        ``feedback=True`` the perturbations added to the law's output (entry 0 perturbs the yank of the yank-omega variants).
         method: the controller's RLS method (``theta_update``, ``theta_update2``, ``approx_theta_update``), method_kwargs its
         options (``project``).  The first RLS step is step ``learn_from`` (1 reproduces the reference's ``if i != 0``).
         ``obs_log`` [K//log_every, E, N, 20] receives the observation after every ``log_every``-th step.  Leaves the env state
@@ -164,6 +180,8 @@ class LearningRollout:
             raise ValueError(f"inputs must have shape [K, {env.NUM_ENVS}, {env.NUM_DRONES}, 4], got {tuple(inputs.shape)}")
         _lib.require_cuda(inputs, "inputs", env.dtype)
         cfg = dl.rls_cfg(method, **method_kwargs)
+        if feedback and dl.K is None:
+            raise _lib.MdsError("feedback=True flies the learned gain: call compute_controller() first")
         K = int(inputs.shape[0])
         if t0 is None:
             t0 = self.t
@@ -174,10 +192,11 @@ class LearningRollout:
             _lib.require_cuda(obs_log, "obs_log", env.dtype)
             if write_every < 1 or obs_log.numel() < (K // write_every) * env.NUM_TOTAL * _lib.OBS_DIM:
                 raise ValueError("obs_log too small or log_every < 1")
-        _lib.call("mds_learning_rollout", env.dtype, env._prm, cfg, dl.VARIANT, int(learn_from), write_every, env._state_struct(),
-                  dl.low_level.pid_struct(), _lib.ptr(self.trajs.specs), _lib.ptr(self.trajs.segs), _lib.ptr(inputs), _lib.ptr(dl.theta_planes),
-                  _lib.ptr(dl.P_planes), _lib.ptr(dl.resid), _lib.ptr(env._obs), _lib.ptr(env._ext_force), _lib.ptr(obs_log), float(t0), K,
-                  env.NUM_ENVS, env.NUM_DRONES, _lib.stream_ptr(env.device))
+        name, gain = ("mds_learning_rollout_feedback", [_lib.ptr(dl.K_planes)]) if feedback else ("mds_learning_rollout", [])
+        _lib.call(name, env.dtype, env._prm, cfg, dl.VARIANT, int(learn_from), write_every, env._state_struct(), dl.low_level.pid_struct(),
+                  _lib.ptr(self.trajs.specs), _lib.ptr(self.trajs.segs), _lib.ptr(inputs), *gain, _lib.ptr(dl.theta_planes), _lib.ptr(dl.P_planes),
+                  _lib.ptr(dl.resid), _lib.ptr(env._obs), _lib.ptr(env._ext_force), _lib.ptr(obs_log), float(t0), K, env.NUM_ENVS,
+                  env.NUM_DRONES, _lib.stream_ptr(env.device))
         env.step_counter += K * env.PYB_STEPS_PER_CTRL
         dl.low_level.control_counter += K
         self.t = t0 + K * env.CTRL_TIMESTEP

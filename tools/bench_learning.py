@@ -2,7 +2,11 @@
 For every (precision, m, K, E x N): warm-up, then the two paths timed with CUDA events, alternating, from the same saved
 state; in the same run one pair of runs from identical states is compared (fp64: 1e-9 of each quantity's scale; fp32: 2e-4,
 the per-call RLS tests' fp32 tolerance).  Prints the card name and power limit first, then one JSON line per case.
-usage: python tools/bench_learning.py [reps=3]"""
+--feedback: the same for closed-loop exploration (run(feedback=True) against the per-call loop with dl.compute and an add;
+gains from compute_controller() on the prior models, perturbations: the open-loop draws centred and scaled by 1/4, i.e.
++-0.1 m g and +-0.05 rad/s); at 1 M drones the fused
+open-loop call on the open-loop excitation is timed alongside (fused_open_ms), which shows what flying the gain costs.
+usage: python tools/bench_learning.py [reps=3] [--feedback]"""
 import json
 import os
 import subprocess
@@ -18,7 +22,9 @@ import multidronesim_b200 as mds  # noqa: E402
 from multidronesim_b200 import _lib  # noqa: E402
 from multidronesim_b200.control import dlqr  # noqa: E402
 
-REPS = int(sys.argv[1]) if len(sys.argv) > 1 else 3
+ARGS = [a for a in sys.argv[1:] if a != "--feedback"]
+FEEDBACK = "--feedback" in sys.argv[1:]
+REPS = int(ARGS[0]) if ARGS else 3
 
 
 def card():
@@ -58,8 +64,12 @@ def percall(env, dl, ts, us):
     for k in range(us.shape[0]):
         dl.set_reference(ts.eval(k * env.CTRL_TIMESTEP))
         e_t = dl.error_state(obs).clone()
-        phis = torch.cat([e_t, us[k]], dim=-1)
-        obs = env.step(dl.compute_low_level(us[k], obs))[0]
+        if FEEDBACK:
+            u = dl.compute(obs, skip_low_level=True)[1] + us[k]
+        else:
+            u = us[k]
+        phis = torch.cat([e_t, u], dim=-1)
+        obs = env.step(dl.compute_low_level(u, obs))[0]
         dl.theta_update(phis, dl.error_state(obs))
 
 
@@ -69,45 +79,55 @@ def outputs(env, dl):
 
 
 def main():
-    print(json.dumps({"card": card(), "torch": torch.__version__}), flush=True)
+    print(json.dumps({"card": card(), "torch": torch.__version__, "feedback": FEEDBACK}), flush=True)
     for dtype in (torch.float32, torch.float64):
         for m in (9, 10):
             for E, N in ((125000, 8), (1, 2), (1, 7)):
                 env, dl, ts = setup(E, N, dtype, m)
+                if FEEDBACK:
+                    dl.compute_controller()
                 ro = mds.LearningRollout(env, ts, dl)
                 s0 = snapshot(env, dl)
                 for K in (24, 40):
                     mg = env.M * env.G
                     g = torch.Generator(device="cuda").manual_seed(K)
                     thrust = torch.empty(K, E, N, 1, device="cuda", dtype=dtype).uniform_(0.7 * mg, 1.5 * mg, generator=g)
-                    us = torch.cat([thrust, torch.empty(K, E, N, 3, device="cuda", dtype=dtype).uniform_(-0.2, 0.2, generator=g)], -1).contiguous()
+                    us_open = torch.cat([thrust, torch.empty(K, E, N, 3, device="cuda", dtype=dtype).uniform_(-0.2, 0.2, generator=g)], -1).contiguous()
+                    us = (us_open - torch.tensor([1.1 * mg, 0, 0, 0], device="cuda", dtype=dtype)) / 4 if FEEDBACK else us_open  # +-0.1 m g
                     # agreement from identical states
                     restore(env, dl, s0); percall(env, dl, ts, us); torch.cuda.synchronize(); want = outputs(env, dl)
-                    restore(env, dl, s0); ro.run(us, t0=0.0); torch.cuda.synchronize(); got = outputs(env, dl)
+                    restore(env, dl, s0); ro.run(us, t0=0.0, feedback=FEEDBACK); torch.cuda.synchronize(); got = outputs(env, dl)
                     tol = 1e-9 if dtype == torch.float64 else 2e-4
                     errs = [float(np.abs(a - b).max()) / max(1.0, float(np.abs(b).max())) for a, b in zip(got, want)]
                     # timing: warm-up, then alternate the two paths, each from the saved state (the restore is outside the events)
                     a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    t_call, t_fused = [], []
+                    D = E * N
+                    times = {"percall": [], "fused": []}
+                    if FEEDBACK and D >= 1_000_000:
+                        times["fused_open"] = []
                     for rep in range(REPS + 1):
-                        for name in ("percall", "fused"):
+                        for name in times:
                             restore(env, dl, s0)
                             torch.cuda.synchronize()
                             a.record()
                             if name == "percall":
                                 percall(env, dl, ts, us)
+                            elif name == "fused":
+                                ro.run(us, t0=0.0, feedback=FEEDBACK)
                             else:
-                                ro.run(us, t0=0.0)
+                                ro.run(us_open, t0=0.0)
                             b.record()
                             torch.cuda.synchronize()
                             if rep > 0:
-                                (t_call if name == "percall" else t_fused).append(a.elapsed_time(b))
-                    D = E * N
-                    tc, tf = float(np.median(t_call)), float(np.median(t_fused))
-                    print(json.dumps({"dtype": str(dtype).split(".")[1], "m": m, "K": K, "E": E, "N": N, "percall_ms": round(tc, 4), "fused_ms": round(tf, 4),
-                                      "speedup": round(tc / tf, 2), "fused_drone_steps_per_s": D * K / (tf * 1e-3),
-                                      "percall_drone_steps_per_s": D * K / (tc * 1e-3), "max_rel_err": max(errs), "tol": tol,
-                                      "agree": bool(max(errs) <= tol), "t": time.strftime("%H:%M:%S")}), flush=True)
+                                times[name].append(a.elapsed_time(b))
+                    tc, tf = float(np.median(times["percall"])), float(np.median(times["fused"]))
+                    line = {"dtype": str(dtype).split(".")[1], "m": m, "K": K, "E": E, "N": N, "feedback": FEEDBACK, "percall_ms": round(tc, 4),
+                            "fused_ms": round(tf, 4), "speedup": round(tc / tf, 2), "fused_drone_steps_per_s": D * K / (tf * 1e-3),
+                            "percall_drone_steps_per_s": D * K / (tc * 1e-3), "max_rel_err": max(errs), "tol": tol,
+                            "agree": bool(max(errs) <= tol), "t": time.strftime("%H:%M:%S")}
+                    if "fused_open" in times:
+                        line["fused_open_ms"] = round(float(np.median(times["fused_open"])), 4)
+                    print(json.dumps(line), flush=True)
                 del env, dl, ts, ro, s0
                 torch.cuda.empty_cache()
 
