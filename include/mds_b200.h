@@ -384,6 +384,22 @@ int mds_learning_rollout_feedback_f64(const MdsDroneParams* prm, const MdsRlsCfg
                                       const double* inputs_dev, const double* gain_dev, double* theta_dev, double* P_dev, double* resid_dev,
                                       double* obs_dev, const double* ext_force_dev, double* obs_log_dev, double t0, int K, int E, int N,
                                       void* stream);
+/* The same loop for the 12-dim torque-level model (MDS_CTRL_LQR_TORQUE error state, decentralized_lqr.py), which has no inner
+ * loop and no PID state: step k flies input_to_action(u_k), which clamps u_k[0] >= 0 in place, and the RLS step takes
+ * phi = [e_t, u_k] with the clamped u_k.  gain_dev NULL: open loop, u_k = inputs_dev[k] [D*4] = [f, tx, ty, tz].  Otherwise
+ * u_k = max(-sum_j K_dj e_j + m g, 0 on the thrust) + inputs_dev[k] (mds_dlqr_ctrl's law and clamp, then the perturbation),
+ * the gain read once per launch: coupled = 0: K_dj = 0 for j != d, gain_dev [48][D] planes (staged with theta and P);
+ * coupled = 1: the robot-coupled gain_dev [N][48][D] planes of mds_dlqr_ctrl (read from device memory every step).
+ * rls->m = 12, rls->project AFTER (theta_update) or LOOP (approx_theta_update): both methods project theta.  Every other
+ * argument and check is mds_learning_rollout's; error messages start with "learning_rollout_torque: ". */
+int mds_learning_rollout_torque_f32(const MdsDroneParams* prm, const MdsRlsCfg* rls, int learn_from, int write_obs_every, MdsState st,
+                                    const MdsTrajSpecF32* specs_dev, const MdsTrajSegF32* segs_dev, const float* inputs_dev, const float* gain_dev,
+                                    int coupled, float* theta_dev, float* P_dev, float* resid_dev, float* obs_dev, const float* ext_force_dev,
+                                    float* obs_log_dev, double t0, int K, int E, int N, void* stream);
+int mds_learning_rollout_torque_f64(const MdsDroneParams* prm, const MdsRlsCfg* rls, int learn_from, int write_obs_every, MdsState st,
+                                    const MdsTrajSpecF64* specs_dev, const MdsTrajSegF64* segs_dev, const double* inputs_dev, const double* gain_dev,
+                                    int coupled, double* theta_dev, double* P_dev, double* resid_dev, double* obs_dev, const double* ext_force_dev,
+                                    double* obs_log_dev, double t0, int K, int E, int N, void* stream);
 
 /* compute_controller (decentralized_lqr_omega.py:185-204): K_d = R^-1 B_d' X_d, X_d the stabilising solution of the
  * continuous-time algebraic Riccati equation of drone d's learned model theta_d = [A_d, B_d]^T, for diagonal Q (q_diag [m])

@@ -6,8 +6,8 @@ from . import _lib
 from .enums import DroneModel, Physics
 from .constants import DroneConstants
 from .envs import BatchedCtrlAviary, CtrlAviary
-from .rollout import FusedRollout, HostPipeline, HostRollout, LearningRollout, PerCallPipeline, SwarmStreams
+from .rollout import FusedRollout, HostPipeline, HostRollout, LearningRollout, PerCallPipeline, SwarmStreams, TorqueLearningRollout
 from . import control, model, cbf, trajectories, obstacles, utils, dist, scenarios, fedce
 
-__all__ = ["DroneModel", "Physics", "DroneConstants", "BatchedCtrlAviary", "CtrlAviary", "FusedRollout", "HostPipeline", "HostRollout", "LearningRollout", "PerCallPipeline", "SwarmStreams",
+__all__ = ["DroneModel", "Physics", "DroneConstants", "BatchedCtrlAviary", "CtrlAviary", "FusedRollout", "HostPipeline", "HostRollout", "LearningRollout", "PerCallPipeline", "SwarmStreams", "TorqueLearningRollout",
            "control", "model", "cbf", "trajectories", "obstacles", "utils", "dist", "scenarios", "_lib"]

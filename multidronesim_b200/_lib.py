@@ -126,6 +126,7 @@ _SIGS = {
     "mds_learning_rollout": [_PRM, C.POINTER(RlsCfg), _I, _I, _I, State, PidState, _P, _P, _P, _P, _P, _P, _P, _P, _P, _D, _I, _I, _I, _P],
     "mds_learning_rollout_feedback": [_PRM, C.POINTER(RlsCfg), _I, _I, _I, State, PidState, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _D, _I, _I,
                                       _I, _P],
+    "mds_learning_rollout_torque": [_PRM, C.POINTER(RlsCfg), _I, _I, State, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P, _P, _D, _I, _I, _I, _P],
 }
 _PLAIN = {
     "mds_abi_version": ([], _I),

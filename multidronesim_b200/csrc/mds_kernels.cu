@@ -806,6 +806,16 @@ static int rollout_impl(const MdsDroneParams* prm, const MdsRolloutCfg* cfg, con
   return check_launch("rollout");
 }
 
+// The checks of the fused learning rollouts after their model checks: sizes, physics and the observation log
+static int learn_shape_checks(const MdsDroneParams* prm, const MdsRlsCfg* rls, int write_obs_every, const void* obs_log, int K, int E, int N,
+                              const char* who) {
+  if (!(rls->dt > 0.0 && rls->drones_per_env == N)) return fail(MDS_ERR_ARG, "%s: dt must be positive and drones_per_env equal to N", who);
+  if (!(K >= 0 && E > 0 && N >= 1 && N <= MDS_MAX_DRONES_PER_ENV)) return fail(MDS_ERR_ARG, "%s: bad K, E or N", who);
+  if (prm->substeps < 1) return fail(MDS_ERR_ARG, "%s: substeps must be >= 1", who);
+  if (prm->physics != MDS_PHYSICS_DYN && prm->physics != MDS_PHYSICS_DYN_GND_DRAG_DW) return fail(MDS_ERR_ARG, "%s: unknown physics mode", who);
+  if (write_obs_every > 0 && !obs_log) return fail(MDS_ERR_ARG, "%s: obs_log buffer missing", who);
+  return MDS_OK;
+}
 template <typename Real>
 static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls, int variant, int learn_from, int write_obs_every, MdsState st,
                                  MdsPidState pid, const typename TrajSpecT<Real>::spec* specs, const typename TrajSpecT<Real>::seg* segs,
@@ -822,18 +832,39 @@ static int learning_rollout_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls
   if (const int rc = rls_params(rls, "learning_rollout", &c)) return rc;
   // project_theta exists for the 10-dim crazyflie model only (decentralized_yolqr_crazyflie.py:245-257); the m = 9 kernel carries none
   MDS_REQUIRE(!(rls->m == 9 && rls->project != MDS_RLS_PROJECT_NONE), "learning_rollout: project_theta is defined for m = 10 only");
-  MDS_REQUIRE(rls->dt > 0.0 && rls->drones_per_env == N, "learning_rollout: dt must be positive and drones_per_env equal to N");
-  MDS_REQUIRE(K >= 0 && E > 0 && N >= 1 && N <= MDS_MAX_DRONES_PER_ENV, "learning_rollout: bad K, E or N");
-  MDS_REQUIRE(prm->substeps >= 1, "learning_rollout: substeps must be >= 1");
-  MDS_REQUIRE(prm->physics == MDS_PHYSICS_DYN || prm->physics == MDS_PHYSICS_DYN_GND_DRAG_DW, "learning_rollout: unknown physics mode");
-  MDS_REQUIRE(!(write_obs_every > 0) || obs_log, "learning_rollout: obs_log buffer missing");
+  if (const int rc = learn_shape_checks(prm, rls, write_obs_every, obs_log, K, E, N, "learning_rollout")) return rc;
   if (K == 0) return MDS_OK;
   LearnLaunch<Real> a{to_dev<Real>(*prm), c, rls->m, rls->project != MDS_RLS_PROJECT_NONE, learn_from, write_obs_every > 0 ? write_obs_every : 0,
-                      to_dev<Real>(st), to_dev<Real>(pid), specs, segs, inputs, gain, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E, N,
-                      (cudaStream_t)stream};
+                      to_dev<Real>(st), to_dev<Real>(pid), specs, segs, inputs, gain, 0, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E,
+                      N, (cudaStream_t)stream};
   const cudaError_t e = launch_learn_kernel<Real>(a);
   if (e != cudaSuccess) return cuda_fail("learning_rollout: shared-memory opt-in", e);
   return check_launch("learning_rollout");
+}
+
+// The 12-dim torque-level model: no inner loop and no PID state; both of its reference methods project theta.  gain NULL: open
+// loop; coupled: gain holds the robot-coupled [N][48][D] planes, otherwise the per-drone [48][D] planes.
+template <typename Real>
+static int learning_rollout_torque_impl(const MdsDroneParams* prm, const MdsRlsCfg* rls, int learn_from, int write_obs_every, MdsState st,
+                                        const typename TrajSpecT<Real>::spec* specs, const typename TrajSpecT<Real>::seg* segs, const Real* inputs,
+                                        const Real* gain, int coupled, Real* theta, Real* Pm, Real* resid, Real* obs, const Real* fext, Real* obs_log,
+                                        double t0, int K, int E, int N, void* stream) {
+  MDS_REQUIRE(prm && rls && st.pos_wx && st.quat && st.vel_wy && st.rpm && st.wz && specs && (inputs || K == 0) && theta && Pm && obs,
+              "learning_rollout_torque: null pointer");
+  MDS_REQUIRE(rls->m == 12, "learning_rollout_torque: m must be 12");
+  RlsP c;
+  if (const int rc = rls_params(rls, "learning_rollout_torque", &c)) return rc;
+  MDS_REQUIRE(rls->project != MDS_RLS_PROJECT_NONE,
+              "learning_rollout_torque: project must be AFTER (theta_update) or LOOP (approx_theta_update): both methods project theta");
+  MDS_REQUIRE(!coupled || gain, "learning_rollout_torque: a coupled law needs a gain");
+  if (const int rc = learn_shape_checks(prm, rls, write_obs_every, obs_log, K, E, N, "learning_rollout_torque")) return rc;
+  if (K == 0) return MDS_OK;
+  LearnLaunch<Real> a{to_dev<Real>(*prm), c, 12, 1, learn_from, write_obs_every > 0 ? write_obs_every : 0, to_dev<Real>(st), PidP<Real>{nullptr, nullptr},
+                      specs, segs, inputs, gain, coupled ? 1 : 0, theta, Pm, resid, obs, fext, obs_log, t0, prm->dt_ctrl, K, E, N,
+                      (cudaStream_t)stream};
+  const cudaError_t e = launch_learn_torque_kernel<Real>(a);
+  if (e != cudaSuccess) return cuda_fail("learning_rollout_torque: shared-memory opt-in", e);
+  return check_launch("learning_rollout_torque");
 }
 
 extern "C" {
@@ -986,6 +1017,12 @@ int mds_cbf_num_rows(int order, int N, int n_obs) { return N * (N - 1) / 2 + 8 *
     MDS_REQUIRE(gain, "learning_rollout: null gain pointer");                                                                                      \
     return learning_rollout_impl<REAL>(prm, rls, variant, learn_from, write_obs_every, st, pid, specs, segs, inputs, gain, theta, Pm, resid, obs,  \
                                        fext, obs_log, t0, K, E, N, stream);                                                                        \
+  }                                                                                                                                                \
+  int mds_learning_rollout_torque_##SUF(const MdsDroneParams* prm, const MdsRlsCfg* rls, int learn_from, int write_obs_every, MdsState st,         \
+                                        const SPEC* specs, const SEG* segs, const REAL* inputs, const REAL* gain, int coupled, REAL* theta, REAL* Pm, \
+                                        REAL* resid, REAL* obs, const REAL* fext, REAL* obs_log, double t0, int K, int E, int N, void* stream) {     \
+    return learning_rollout_torque_impl<REAL>(prm, rls, learn_from, write_obs_every, st, specs, segs, inputs, gain, coupled, theta, Pm, resid, obs, \
+                                              fext, obs_log, t0, K, E, N, stream);                                                                 \
   }
 
 MDS_DEFINE(f32, float, MdsTrajSpecF32, MdsTrajSegF32)

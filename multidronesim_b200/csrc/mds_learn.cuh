@@ -12,6 +12,14 @@
 //   u = -K_d e_t (+ m g unless yank-omega; LQR_OMEGA: cap_thrust) + u[k],  phi = [e_t, u]
 // which is the per-call loop with mds_dlqr_ctrl(skip_low_level) and an add before mds_lowlevel.  The gain [4*m][D] planes
 // (mds_dlqr_ctrl's uncoupled layout) are read once per launch and staged next to theta and P: constant within the launch.
+// M = 12: the torque-level model (decentralized_lqr.py), no inner loop and no PID state: the action is input_to_action(u),
+// which clamps u[0] >= 0 in place, so phi carries the clamped u.  Its law is
+//   u = max(-sum_j K_dj e_j + m g, 0 on the thrust) + u[k]
+// with K_dj the drone's own gain (FEEDBACK) or, COUPLED, the robot-coupled gain [N][48][D] planes of mds_dlqr_ctrl.  The
+// coupled gain is not staged (N * 48 words per thread would not fit beside theta and P at N = 32 in fp64): it is read from
+// HBM every step, as dlqr_ctrl_kernel does.  The partners' error states come through shared memory: each lane publishes
+// e_t in its s_phi column (where the RLS step puts phi[:12] = e_t anyway), the lane group syncs, sums over its N sources and
+// syncs again before any lane writes s_phi -- in every physics mode, DYN included, whose physics step has no group sync.
 #pragma once
 #include <cuda_runtime.h>
 #include "mds_learn_launch.cuh"
@@ -22,12 +30,16 @@
 template <typename Real, int M> static int learn_threads(int NP) { return rls_threads<Real, M>() > NP ? rls_threads<Real, M>() : NP; }
 // Staged words per thread: the RLS kernel's columns, plus the 4*M gain entries when FEEDBACK
 template <typename Real, int M, bool FEEDBACK> constexpr int learn_words_per_thread() { return rls_words_per_thread<Real, M>() + (FEEDBACK ? 4 * M : 0); }
+// COUPLED stages no gain
+template <typename Real, int M, bool FEEDBACK, bool COUPLED> constexpr int learn_words_per_thread() { return learn_words_per_thread<Real, M, FEEDBACK && !COUPLED>(); }
 
 // M = 9: DecentralizedLQROmega (LQR_OMEGA error state, ThrustOmega inner loop); M = 10: the yank-omega variants (LQR_YANK,
-// YankOmega inner loop).  PROJECT: project_theta is applied (approx_theta_update(project=True)), compile-time like the RLS kernel.
+// YankOmega inner loop); M = 12: DecentralizedLQR (LQR_TORQUE error state, input_to_action, pid unused; PROJECT only).
+// PROJECT: project_theta is applied (approx_theta_update(project=True)), compile-time like the RLS kernel.
 // FEEDBACK: inputs are perturbations of the law u = -K_d e_t (gain: [4*M][D] planes; the last parameter, so that the open-loop
 // kernels keep their parameter layout); otherwise inputs are the inner loop's inputs and gain is unused.
-template <typename Real, int M, bool PROJECT, bool FEEDBACK>
+// COUPLED (M = 12, with FEEDBACK): gain holds the robot-coupled [N][4*M][D] planes, read from HBM every step.
+template <typename Real, int M, bool PROJECT, bool FEEDBACK, bool COUPLED>
 __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP c, StateP<Real> st, PidP<Real> pid,
                                                            const typename TrajSpecT<Real>::spec* __restrict__ specs,
                                                            const typename TrajSpecT<Real>::seg* __restrict__ segs,
@@ -36,7 +48,9 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
                                                            Real* __restrict__ obs_log, double t0, double dt_ctrl, int learn_from, int write_obs_every,
                                                            int K, int E, int N, int NP, const Real* __restrict__ gain) {
   constexpr int MN = M + 4, TRI = MN * (MN + 1) / 2;
-  constexpr int CTRL = M == 9 ? MDS_CTRL_LQR_OMEGA : MDS_CTRL_LQR_YANK;
+  constexpr int CTRL = M == 9 ? MDS_CTRL_LQR_OMEGA : (M == 10 ? MDS_CTRL_LQR_YANK : MDS_CTRL_LQR_TORQUE);
+  static_assert(M != 12 || PROJECT, "both 12-dim reference methods project theta");
+  static_assert(!COUPLED || (M == 12 && FEEDBACK), "the robot-coupled law is the 12-dim model's");
   using R4 = typename Vec4T<Real>::type;
   extern __shared__ __align__(16) unsigned char learn_smem[];
   __shared__ R4 sm_pos[32];  // downwash positions of the block's lane groups
@@ -54,7 +68,7 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
   Real* s_phi = sT + MN * M * T;
   Real* s_w = s_phi + MN * T;
   Real* s_term = s_w + MN * T;
-  Real* sK = s_term + M * T;  // FEEDBACK: gain entry (i, k) of u_i = -sum_k K_ik e_k at sK[(i * M + k) * T]
+  Real* sK = s_term + M * T;  // FEEDBACK, not COUPLED: gain entry (i, k) of u_i = -sum_k K_ik e_k at sK[(i * M + k) * T]
   const size_t D = (size_t)E * N, d = (size_t)g.d;
   Drone<Real> s;
   Pid<Real> ps;
@@ -68,12 +82,12 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
       for (int j = i; j < MN; ++j) cp_async_real(sP + rls_tri<MN>(i, j) * T, Pm + (size_t)(i * MN + j) * D + d);
 #pragma unroll 1
     for (int k = 0; k < MN * M; ++k) cp_async_real(sT + k * T, theta + (size_t)k * D + d);
-    if (FEEDBACK) {
+    if (FEEDBACK && !COUPLED) {
 #pragma unroll 1
       for (int k = 0; k < 4 * M; ++k) cp_async_real(sK + k * T, gain + (size_t)k * D + d);
     }
     s = load_drone(st, g.d);
-    ps = load_pid(pid, g.d);
+    if constexpr (M != 12) ps = load_pid(pid, g.d);
     o = load_obs(obs, g.d);
     spec = specs[g.d];
     if (fext) fx = {fext[3 * d], fext[3 * d + 1], fext[3 * d + 2]};
@@ -91,7 +105,7 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
       ref = eval_traj<Real>(spec, segs, t0 + (double)k * dt_ctrl);  // the time expression of the rollout kernel and its host plans
       lqr_error_state(P, CTRL, o, ref, e0);
       load4(inputs + (size_t)k * D * 4, g.d, u);
-      if (FEEDBACK) {  // dlqr_ctrl_kernel's law and order of operations (skip_low_level: capped, no max(u, 0)), then + u[k]
+      if (FEEDBACK && !COUPLED) {  // dlqr_ctrl_kernel's law and order of operations (skip_low_level: capped, no max(u, 0)), then + u[k]
         Real uf[4] = {Real(0), Real(0), Real(0), Real(0)};
 #pragma unroll
         for (int i = 0; i < 4; ++i)
@@ -99,10 +113,38 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
           for (int j = 0; j < M; ++j) uf[i] -= sK[(i * M + j) * T] * e0[j];
         if (CTRL != MDS_CTRL_LQR_YANK) uf[0] += P.m * P.g;
         if (CTRL == MDS_CTRL_LQR_OMEGA) uf[0] = cap_thrust(P, uf[0]);
+        if (CTRL == MDS_CTRL_LQR_TORQUE) uf[0] = max_(uf[0], Real(0));  // dlqr_ctrl_kernel's input_to_action clamp
 #pragma unroll
         for (int i = 0; i < 4; ++i) u[i] = uf[i] + u[i];
       }
-      low_level(P, CTRL, ps, u, o, rpm);
+      if constexpr (M == 12) {
+        if (!COUPLED) input_to_action(P, u, rpm);  // clamps u[0] >= 0 in place: phi carries the clamped u
+      } else {
+        low_level(P, CTRL, ps, u, o, rpm);
+      }
+    }
+    if constexpr (COUPLED) {  // u = -sum_j K_dj e_j over the env's N drones: publish e_t, sync, sum, sync (s_phi is reused below)
+      if (g.valid) {
+#pragma unroll
+        for (int i = 0; i < M; ++i) s_phi[i * T] = e0[i];
+      }
+      __syncwarp(g.gmask);
+      if (g.valid) {
+        Real uf[4] = {Real(0), Real(0), Real(0), Real(0)};
+        for (int j = 0; j < N; ++j) {  // dlqr_ctrl_kernel's order: source j, then row i, then column k
+          const Real* ej = s_phi + (j - g.n);
+          const Real* Kj = gain + (size_t)j * 4 * M * D + d;
+#pragma unroll
+          for (int i = 0; i < 4; ++i)
+#pragma unroll
+            for (int k = 0; k < M; ++k) uf[i] -= Kj[(size_t)(i * M + k) * D] * ej[k * T];
+        }
+        uf[0] = max_(uf[0] + P.m * P.g, Real(0));
+#pragma unroll
+        for (int i = 0; i < 4; ++i) u[i] = uf[i] + u[i];
+        input_to_action(P, u, rpm);
+      }
+      __syncwarp(g.gmask);  // every lane of the group has read its partners' e_t
     }
     o = physics_core<0>(P, s, rpm, fx, sm_pos + (tid - g.n), g, N, NP);
     if (write_obs_every > 0 && --log_countdown == 0) {
@@ -157,7 +199,7 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
   // ---- write back: state, observation, PID state; theta and both triangles of P (the planes keep the full square)
   store_drone(st, g.d, s);
   store_obs(obs, g.d, o);
-  store_pid(pid, g.d, ps);
+  if constexpr (M != 12) store_pid(pid, g.d, ps);
 #pragma unroll 1
   for (int k = 0; k < MN * M; ++k) theta[(size_t)k * D + d] = sT[k * T];
 #pragma unroll 1
@@ -168,4 +210,21 @@ __global__ void __launch_bounds__(32) learn_rollout_kernel(DroneP<Real> P, RlsP 
       Pm[(size_t)(i * MN + j) * D + d] = pij;
       if (j > i) Pm[(size_t)(j * MN + i) * D + d] = pij;
     }
+}
+
+// Shared-memory opt-in and launch of one instantiation (mds_learn_tu.cu, mds_learn_torque_tu.cu)
+template <typename Real, int M, bool PROJECT, bool FEEDBACK, bool COUPLED> static cudaError_t launch_learn(const LearnLaunch<Real>& a) {
+  const int NP = next_pow2(a.N), threads = learn_threads<Real, M>(NP);
+  const size_t smem = (size_t)learn_words_per_thread<Real, M, FEEDBACK, COUPLED>() * threads * sizeof(Real);
+  auto kern = learn_rollout_kernel<Real, M, PROJECT, FEEDBACK, COUPLED>;
+  // N = 32 in fp64 stages 61-105 KB per block: past the default 48 KB of dynamic shared memory (so does m = 12 feedback in fp32)
+  const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return e;
+  const int epb = threads / NP, blocks = (a.E + epb - 1) / epb;
+  kern<<<blocks, threads, smem, a.cs>>>(a.Pd, a.c, a.Sd, a.Pi, a.specs, a.segs, a.inputs, a.theta, a.Pm, a.resid, a.obs, a.fext, a.obs_log, a.t0,
+                                        a.dt_ctrl, a.learn_from, a.write_obs_every, a.K, a.E, a.N, NP, a.gain);
+  return cudaSuccess;
+}
+template <typename Real, int M, bool PROJECT> static cudaError_t launch_learn(const LearnLaunch<Real>& a) {
+  return a.gain ? launch_learn<Real, M, PROJECT, true, false>(a) : launch_learn<Real, M, PROJECT, false, false>(a);
 }

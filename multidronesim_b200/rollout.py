@@ -156,7 +156,7 @@ class LearningRollout:
     def __init__(self, env, trajs, controller):
         if isinstance(controller, DecentralizedLQR):
             raise _lib.MdsError("LearningRollout takes the decentralised LQR variants with an inner loop; the 12-dim torque model "
-                                "has none and a robot-coupled gain")
+                                "runs through TorqueLearningRollout")
         if not isinstance(controller, _DecentralizedBase):
             raise TypeError("LearningRollout needs a decentralised LQR controller (control.dlqr)")
         if trajs.num != env.NUM_TOTAL:
@@ -174,24 +174,9 @@ class LearningRollout:
         ``obs_log`` [K//log_every, E, N, 20] receives the observation after every ``log_every``-th step.  Leaves the env state
         and obs, the inner loop's PID state, theta, P and ``resid`` (of the last update) as the loop does.  Returns the obs."""
         env, dl = self.env, self.controller
-        if not isinstance(inputs, torch.Tensor):
-            raise TypeError("inputs must be a torch tensor [K, E, N, 4]")
-        if inputs.dim() != 4 or tuple(inputs.shape[1:]) != (env.NUM_ENVS, env.NUM_DRONES, 4):
-            raise ValueError(f"inputs must have shape [K, {env.NUM_ENVS}, {env.NUM_DRONES}, 4], got {tuple(inputs.shape)}")
-        _lib.require_cuda(inputs, "inputs", env.dtype)
-        cfg = dl.rls_cfg(method, **method_kwargs)
-        if feedback and dl.K is None:
-            raise _lib.MdsError("feedback=True flies the learned gain: call compute_controller() first")
-        K = int(inputs.shape[0])
-        if t0 is None:
-            t0 = self.t
+        cfg, K, t0, write_every = _learning_args(self, inputs, method, t0, obs_log, log_every, feedback, method_kwargs)
         if K == 0:  # nothing to run (the C entry point takes K = 0 as well; an empty tensor has no storage to point at)
             return env._obs
-        write_every = int(log_every) if obs_log is not None else 0
-        if obs_log is not None:
-            _lib.require_cuda(obs_log, "obs_log", env.dtype)
-            if write_every < 1 or obs_log.numel() < (K // write_every) * env.NUM_TOTAL * _lib.OBS_DIM:
-                raise ValueError("obs_log too small or log_every < 1")
         name, gain = ("mds_learning_rollout_feedback", [_lib.ptr(dl.K_planes)]) if feedback else ("mds_learning_rollout", [])
         _lib.call(name, env.dtype, env._prm, cfg, dl.VARIANT, int(learn_from), write_every, env._state_struct(), dl.low_level.pid_struct(),
                   _lib.ptr(self.trajs.specs), _lib.ptr(self.trajs.segs), _lib.ptr(inputs), *gain, _lib.ptr(dl.theta_planes), _lib.ptr(dl.P_planes),
@@ -199,6 +184,80 @@ class LearningRollout:
                   env.NUM_DRONES, _lib.stream_ptr(env.device))
         env.step_counter += K * env.PYB_STEPS_PER_CTRL
         dl.low_level.control_counter += K
+        self.t = t0 + K * env.CTRL_TIMESTEP
+        return env._obs
+
+
+def _learning_args(ro, inputs, method, t0, obs_log, log_every, feedback, method_kwargs):
+    """the checks LearningRollout.run and TorqueLearningRollout.run share, all before any launch -> (MdsRlsCfg, K, t0,
+    write_obs_every); obs_log is checked only when there is something to run (K > 0)"""
+    env, dl = ro.env, ro.controller
+    if not isinstance(inputs, torch.Tensor):
+        raise TypeError("inputs must be a torch tensor [K, E, N, 4]")
+    if inputs.dim() != 4 or tuple(inputs.shape[1:]) != (env.NUM_ENVS, env.NUM_DRONES, 4):
+        raise ValueError(f"inputs must have shape [K, {env.NUM_ENVS}, {env.NUM_DRONES}, 4], got {tuple(inputs.shape)}")
+    _lib.require_cuda(inputs, "inputs", env.dtype)
+    cfg = dl.rls_cfg(method, **method_kwargs)
+    if feedback and dl.K is None:
+        raise _lib.MdsError("feedback=True flies the learned gain: call compute_controller() first")
+    K = int(inputs.shape[0])
+    if t0 is None:
+        t0 = ro.t
+    write_every = int(log_every) if obs_log is not None else 0
+    if obs_log is not None and K > 0:
+        _lib.require_cuda(obs_log, "obs_log", env.dtype)
+        if write_every < 1 or obs_log.numel() < (K // write_every) * env.NUM_TOTAL * _lib.OBS_DIM:
+            raise ValueError("obs_log too small or log_every < 1")
+    return cfg, K, t0, write_every
+
+
+class TorqueLearningRollout:
+    """The learning loop of the 12-dim torque-level decentralised LQR (``DecentralizedLQR``; the FedCE learning phases of the
+    reference's simulations/EnvGeometric.py:200-320) for K control steps in ONE launch (``mds_learning_rollout_torque``).  The
+    model has no inner loop: every drone flies ``input_to_action`` of its input while its RLS model learns; theta and P stay
+    in shared memory for the whole launch.  With ``U = multidronesim_b200.utils``, ``run`` equals this per-call loop::
+
+        for k in range(K):
+            dl.set_reference(trajs.eval(t0 + k * dt))
+            e_t = dl.error_state(obs).clone()
+            u = inputs[k].clone()
+            obs = env.step(U.input_to_action(env, u))[0]     # clamps u[..., 0] >= 0 in place: phi carries the clamped u
+            if k >= learn_from: getattr(dl, method)(torch.cat([e_t, u], -1), dl.error_state(obs), **method_kwargs)
+
+    ``run(..., feedback=True)`` flies the learned gain plus the perturbation ``inputs[k]``: ``u = dl.compute(obs,
+    skip_low_level=True)[1] + inputs[k]`` in the loop above, ``u_d = max(-sum_j K_dj e_j + m g, 0 on the thrust)``.  With
+    ``dl._coupled`` (``compute_controller()`` with N >= 2) K_dj is the robot-coupled gain of the environment, read from device
+    memory every step; otherwise each drone's own gain (``force_diagonal=True`` or N = 1).  The gain is read once per launch.
+
+    controller: DecentralizedLQR; trajs: TrajectorySet with one trajectory per drone (the references of the error states)."""
+
+    def __init__(self, env, trajs, controller):
+        if not isinstance(controller, DecentralizedLQR):
+            raise TypeError("TorqueLearningRollout needs the 12-dim torque-level DecentralizedLQR (the other variants run through "
+                            "LearningRollout)")
+        if trajs.num != env.NUM_TOTAL:
+            raise ValueError("need one trajectory per drone")
+        if controller.env is not env:
+            raise ValueError("the controller belongs to another env")
+        self.env, self.trajs, self.controller = env, trajs, controller
+        self.t = 0.0
+
+    def run(self, inputs, method="theta_update", learn_from=0, t0=None, obs_log=None, log_every=0, feedback=False, **method_kwargs):
+        """inputs [K, E, N, 4] (device, the env's dtype): the torque-level inputs [f, tx, ty, tz] of every step; with
+        ``feedback=True`` the perturbations added to the law's output.  method: ``theta_update`` or ``approx_theta_update``.
+        The first RLS step is step ``learn_from``.  ``obs_log`` [K//log_every, E, N, 20] receives the observation after every
+        ``log_every``-th step.  Leaves the env state and obs, theta, P and ``resid`` (of the last update) as the loop does.
+        Returns the obs."""
+        env, dl = self.env, self.controller
+        cfg, K, t0, write_every = _learning_args(self, inputs, method, t0, obs_log, log_every, feedback, method_kwargs)
+        if K == 0:
+            return env._obs
+        gain, coupled = (_lib.ptr(dl.K_planes), int(dl._coupled)) if feedback else (None, 0)
+        _lib.call("mds_learning_rollout_torque", env.dtype, env._prm, cfg, int(learn_from), write_every, env._state_struct(),
+                  _lib.ptr(self.trajs.specs), _lib.ptr(self.trajs.segs), _lib.ptr(inputs), gain, coupled, _lib.ptr(dl.theta_planes),
+                  _lib.ptr(dl.P_planes), _lib.ptr(dl.resid), _lib.ptr(env._obs), _lib.ptr(env._ext_force), _lib.ptr(obs_log), float(t0), K,
+                  env.NUM_ENVS, env.NUM_DRONES, _lib.stream_ptr(env.device))
+        env.step_counter += K * env.PYB_STEPS_PER_CTRL
         self.t = t0 + K * env.CTRL_TIMESTEP
         return env._obs
 
