@@ -83,18 +83,14 @@ template <int NT> MDS_DEV void full_group_hint(GroupMap& g) {
   if (NT > 0 && (NT & (NT - 1)) == 0) g.valid = true;
 }
 
-// Downwash sum for this lane's drone over its env mates; positions staged in shared memory (env_pos: the environment's NP
-// slots -- a slice of a per-block array, or the head of the environment's CBF block, which is idle during the physics).  Called by every lane of the
-// group (two group syncs, shuffles).  Only the LOWER drone of a pair feels the other's downwash, so each unordered pair is
-// evaluated once, by the lane that owns it under the CBF stage's ownership (mds_cbf.cuh: lane n owns (n, n+s+1 mod N) for
-// s < (N-1)/2, and the "diameter" (n, n+N/2) for n < N/2 when N is even); the owner keeps the term if it is the lower one
-// and otherwise hands it to its partner with one shuffle per slot.
-template <typename Real>
-MDS_DEV Real downwash_group(const DroneP<Real>& P, typename Vec4T<Real>::type* env_pos, V3<Real> p, const GroupMap& g, int N, int NP) {
-  typename Vec4T<Real>::type me;
-  me.x = p.x; me.y = p.y; me.z = p.z; me.w = Real(0);
-  env_pos[g.n] = me;
-  __syncwarp(g.cmask);
+// Downwash sum for this lane's drone over its env mates, whose positions the group has already published in shared memory:
+// drone m's position is the (x, y, z) of pos[STRIDE m].  Called by every lane of the group (shuffles, no sync).  Only the
+// LOWER drone of a pair feels the other's downwash, so each unordered pair is evaluated once, by the lane that owns it under
+// the CBF stage's ownership (mds_cbf.cuh: lane n owns (n, n+s+1 mod N) for s < (N-1)/2, and the "diameter" (n, n+N/2) for
+// n < N/2 when N is even); the owner keeps the term if it is the lower one and otherwise hands it to its partner with one
+// shuffle per slot.
+template <int STRIDE, typename Real>
+MDS_DEV Real downwash_exchange(const DroneP<Real>& P, const typename Vec4T<Real>::type* pos, V3<Real> p, const GroupMap& g, int N, int NP) {
   Real dw = Real(0);
   const int n = g.n, lane0 = (threadIdx.x & 31) - n;
   const int K1 = (N - 1) >> 1, half = (N & 1) ? 0 : (N >> 1), S0 = K1 + (half ? 1 : 0);
@@ -112,7 +108,7 @@ MDS_DEV Real downwash_group(const DroneP<Real>& P, typename Vec4T<Real>::type* e
     }
     Real give = Real(0);
     if (own) {
-      const auto q = env_pos[m];
+      const auto q = pos[STRIDE * m];
       const Real dz = q.z - p.z, dx = q.x - p.x, dy = q.y - p.y;  // dz > 0: the partner is above, this drone is pushed down
       const Real dxy2 = dx * dx + dy * dy;
       Real v = Real(0);
@@ -123,7 +119,6 @@ MDS_DEV Real downwash_group(const DroneP<Real>& P, typename Vec4T<Real>::type* e
     const Real got = __shfl_sync(g.cmask, give, lane0 + src);
     if (recv) dw += got;
   }
-  __syncwarp(g.cmask);
   return dw;
 }
 
@@ -131,9 +126,8 @@ MDS_DEV Real downwash_group(const DroneP<Real>& P, typename Vec4T<Real>::type* e
 // high halves; a slot this lane does not own is evaluated against the lane's own position (dz = 0: no force).  Per pair of
 // slots ~30 instructions instead of 2 x 25, and the half-populated "diameter" slot rides along for free.
 #ifndef MDS_NO_DW_PACK
-MDS_DEV float downwash_group(const DroneP<float>& P, float4* env_pos, V3<float> p, const GroupMap& g, int N, int NP) {
-  env_pos[g.n] = make_float4(p.x, p.y, p.z, 0.f);
-  __syncwarp(g.cmask);
+template <int STRIDE>
+MDS_DEV float downwash_exchange(const DroneP<float>& P, const float4* pos, V3<float> p, const GroupMap& g, int N, int NP) {
   float dw = 0.f;
   const int n = g.n;
   const int K1 = (N - 1) >> 1, half = (N & 1) ? 0 : (N >> 1), S0 = K1 + (half ? 1 : 0);
@@ -153,7 +147,7 @@ MDS_DEV float downwash_group(const DroneP<float>& P, float4* env_pos, V3<float> 
         else { src[h] = n - half; recv[h] = true; }
       }
     }
-    const float4 q0 = env_pos[m[0]], q1 = env_pos[m[1]];
+    const float4 q0 = pos[STRIDE * m[0]], q1 = pos[STRIDE * m[1]];
     const F2 dz(q0.z - p.z, q1.z - p.z), dx(q0.x - p.x, q1.x - p.x), dy(q0.y - p.y, q1.y - p.y);  // dz > 0: the partner is above
     const F2 dxy2 = fma_(dy, dy, dx * dx);
     const F2 v = downwash_pair2(P, F2(abs_(dz.v.x), abs_(dz.v.y)), dxy2);
@@ -167,10 +161,22 @@ MDS_DEV float downwash_group(const DroneP<float>& P, float4* env_pos, V3<float> 
       if (recv[1]) dw += got1;
     }
   }
-  __syncwarp(g.cmask);
   return dw;
 }
 #endif
+
+// The same with the positions staged here: env_pos is the environment's NP slots -- a slice of a per-block array, or the
+// head of the environment's CBF block, which is idle during the physics.  Two group syncs.
+template <typename Real>
+MDS_DEV Real downwash_group(const DroneP<Real>& P, typename Vec4T<Real>::type* env_pos, V3<Real> p, const GroupMap& g, int N, int NP) {
+  typename Vec4T<Real>::type me;
+  me.x = p.x; me.y = p.y; me.z = p.z; me.w = Real(0);
+  env_pos[g.n] = me;
+  __syncwarp(g.cmask);
+  const Real dw = downwash_exchange<1>(P, env_pos, p, g, N, NP);
+  __syncwarp(g.cmask);
+  return dw;
+}
 
 // per-env shared-memory block of the CBF stage (in Reals; every part is a multiple of 4 so that the Vec4
 // accesses stay aligned):
@@ -225,11 +231,17 @@ template <typename Real> MDS_DEV CbfSmem<Real> cbf_smem_carve(unsigned char* raw
 // that one runs out of workspace / iterations or its factor breaks down, the scratch solver (qp_solve_group_big).
 // NT > 0 (compile-time drone count) in fp32: the pair rows are evaluated two at a time with packed fp32 instructions
 // (cbf_row2) and stay in registers -- they are written to shared memory only if the cooperative solver is needed.
+// dw_out (optional): receives this lane's downwash sum (downwash_group's value) when dw_on -- the agents the stage exchanges
+// carry the positions the physics starts from, and the pair rows have the downwash's pair ownership, so the physics' own
+// publication of the positions and its two group syncs are not needed.  The packed path takes each slot's downwash from the
+// partner it has just loaded for the row; the scalar path runs downwash_exchange over the published agents.
 template <int ORD, typename Real, int NT = 0>
 MDS_DEV int cbf_filter_group(const DroneP<Real>& P, const CbfP<Real>& C, const CbfSmem<Real>& S, const Real* obstacles, int n_obs,
                              const GroupMap& g, int N, int NP, const CbfAgent<Real>& ag, Real F, const Real unom[4], Real usafe[4],
-                             Real* min_h, int* iters_out) {
+                             Real* min_h, int* iters_out, Real* dw_out = nullptr, bool dw_on = false) {
   using R4 = typename Vec4T<Real>::type;
+  const bool fuse_dw = dw_out != nullptr && dw_on;  // uniform over the group
+  Real dw = Real(0);
   const int n = g.n;
   const RowMap M = row_map(N, n_obs);
   Real* env = S.env0 + (size_t)g.el * S.stride;
@@ -324,6 +336,8 @@ MDS_DEV int cbf_filter_group(const DroneP<Real>& P, const CbfP<Real>& C, const C
   constexpr int S0C = PACK ? (NT - 1) / 2 + ((NT & 1) ? 0 : 1) : 1, NPAIR = (S0C + 1) / 2;
   F2 pa[NPAIR][3], prhs[NPAIR];  // packed path: the pair rows, slot 2q in the low halves and 2q + 1 in the high halves
   if constexpr (PACK) {
+    // the downwash shuffles below need every lane of the group: `valid` must be the compile-time true of full_group_hint
+    static_assert((NT & (NT - 1)) == 0, "the packed pair loop needs a drone count that fills its lane group");
     if (g.valid) {
 #pragma unroll
       for (int q = 0; q < NPAIR; ++q) {
@@ -343,6 +357,28 @@ MDS_DEV int cbf_filter_group(const DroneP<Real>& P, const CbfP<Real>& C, const C
         if (ok1) *min_h = min_(*min_h, h0.v.y);
         else { pa[q][0].v.y = 0.f; pa[q][1].v.y = 0.f; pa[q][2].v.y = 0.f; rhs.v.y = 1e30f; }
         prhs[q] = rhs;
+        if (fuse_dw) {
+          // The two slots' downwash: packed downwash_exchange, the same operations in the same order, from the partners just
+          // loaded.  It reads the row's differences e = own - partner where downwash_exchange forms d = partner - own: IEEE
+          // subtraction is sign-symmetric (flushed denormals included), so |dz| = |ez|, dz > 0 <=> ez < 0, and
+          // dxy2 = fma(dy, dy, dx dx) is bit for bit the row's rho = fma(ey, ey, ex ex) -- the same instructions as the row's.
+          const F2 ex(ag.p.x - o0.p.x, ag.p.x - o1.p.x), ey(ag.p.y - o0.p.y, ag.p.y - o1.p.y), ez(ag.p.z - o0.p.z, ag.p.z - o1.p.z);
+          const F2 dxy2 = fma_(ey, ey, ex * ex);
+          const F2 v = downwash_pair2(P, F2(abs_(ez.v.x), abs_(ez.v.y)), dxy2);
+          const float v0 = (ez.v.x != 0.f && dxy2.v.x < 100.f) ? v.v.x : 0.f, v1 = (ez.v.y != 0.f && dxy2.v.y < 100.f) ? v.v.y : 0.f;
+          dw += ez.v.x < 0.f ? v0 : 0.f;  // the partner is above: this drone is pushed down
+          dw += ez.v.y < 0.f ? v1 : 0.f;
+          // the lane that owns the slot's pair with this lane as its partner (none: the lower half's diameter slot)
+          const bool recv0 = s0 < M.K1 || n >= M.half, recv1 = s1 < M.K1 || n >= M.half;
+          const int src0 = s0 < M.K1 ? wrap_n(n - s0 - 1, N) : (recv0 ? n - M.half : n);
+          const int src1 = s1 < M.K1 ? wrap_n(n - s1 - 1, N) : (recv1 ? n - M.half : n);
+          const float got0 = __shfl_sync(g.cmask, ez.v.x < 0.f ? 0.f : v0, src0, NP);
+          if (recv0) dw += got0;
+          if (s1 < S0C) {
+            const float got1 = __shfl_sync(g.cmask, ez.v.y < 0.f ? 0.f : v1, src1, NP);
+            if (recv1) dw += got1;
+          }
+        }
         // G u = -a . u_n + a . u_m <= rhs  <=>  slack = rhs + a . (u_n - u_m) >= 0
         const F2 sl = fma_(pa[q][2], F2(xn[2] - xm0.z, xn[2] - xm1.z),
                            fma_(pa[q][1], F2(xn[1] - xm0.y, xn[1] - xm1.y), fma_(pa[q][0], F2(xn[0] - xm0.x, xn[0] - xm1.x), rhs)));
@@ -384,6 +420,10 @@ MDS_DEV int cbf_filter_group(const DroneP<Real>& P, const CbfP<Real>& C, const C
       rows[n * M.RPL + s] = row;
     }
   }
+  if constexpr (!PACK) {
+    if (fuse_dw) dw = downwash_exchange<3>(P, agents, ag.p, g, N, NP);  // before the QP workspace overlays the agents
+  }
+  if (dw_out != nullptr) *dw_out = dw;
   // one group-wide OR of (escalate, infeasible 4th-input interval, projected) -- the step's only collective in the common case
   const unsigned any = group_or(g.cmask, NP, (unsigned)(escalate | (fl << 1) | (touched << 2)));
   int status = MDS_QP_OPTIMAL, iters = (any & 4u) ? 1 : 0;
@@ -461,9 +501,11 @@ template <typename Real> MDS_DEV void load4(const Real* p, int d, Real v[4]) {
 // One control period of the env for this lane's drone with the state in registers (every lane of a valid group
 // calls it): clips the action, runs the sub-steps, returns the new observation.  R0 (optional): the rotation matrix of the
 // attitude the period starts from, when the caller already has it (the inner loop of the controller stack builds it).
+// dw0 (optional): the downwash of the first sub-step, when the caller has summed it from the positions the period starts
+// from (cbf_filter_group's dw_out); later sub-steps exchange their moved positions.
 template <int SPEC, typename Real>
 MDS_DEV Obs<Real> physics_core(const DroneP<Real>& P, Drone<Real>& s, const Real action[4], V3<Real> fx, typename Vec4T<Real>::type* env_pos,
-                               const GroupMap& g, int N, int NP, const M3<Real>* R0 = nullptr) {
+                               const GroupMap& g, int N, int NP, const M3<Real>* R0 = nullptr, const Real* dw0 = nullptr) {
   using S = PhysSpec<SPEC>;
   Real rpm[4];
 #pragma unroll
@@ -473,7 +515,7 @@ MDS_DEV Obs<Real> physics_core(const DroneP<Real>& P, Drone<Real>& s, const Real
   const int substeps = S::substeps(P);
   for (int k = 0; k < substeps; ++k) {
     Real dw = Real(0);
-    if (dwash) dw = downwash_group(P, env_pos, s.p, g, N, NP);
+    if (dwash) dw = (dw0 != nullptr && k == 0) ? *dw0 : downwash_group(P, env_pos, s.p, g, N, NP);
     if (g.valid) {
       const M3<Real> R = (R0 != nullptr && k == 0) ? *R0 : quat_to_mat(s.qx, s.qy, s.qz, s.qw);
       av = physics_substep<SPEC>(P, s, rpm, dw, fx, R);
@@ -560,14 +602,15 @@ struct StepStats {
 // PDK: a gain per drone (Rc.lqr_planes) instead of LqrP's; SPEC: compile-time parameter switches (PhysSpec); R_out (optional)
 // receives the rotation matrix of the observation's attitude when the inner loop built it (HAS_PID controllers).
 // REFTAB: the reference is read from ref_slot (a slot of rollout_loop_kernel's reference table) instead of evaluated from
-// (spec, segs, t), which are then unused.
+// (spec, segs, t), which are then unused.  dw_out (optional, with USE_CBF): receives the downwash of the physics sub-step that
+// follows from the observation's positions, summed by the CBF stage (physics_core's dw0).
 template <typename Real, int CTRL, bool USE_CBF, bool PDK = false, int SPEC = 0, int NT = 0, bool REFTAB = false>
 MDS_DEV void ctrl_body(const DroneP<Real>& P, const RolloutP<Real>& Rc, const GeoP<Real>& G, const LqrP<Real>& L, const CbfP<Real>& C,
                        const DslP<Real>& Dg, const DslStateP<Real>& dst, const CbfSmem<Real>& S, const PidP<Real>& pid,
                        const typename TrajSpecT<Real>::spec& spec,
                        const typename TrajSpecT<Real>::seg* __restrict__ segs, const Obs<Real>& o, const GroupMap& g, int N, int NP,
                        double t, Real rpm[4], StepStats& ss, int pid_idx, M3<Real>* R_out = nullptr,
-                       const typename Vec4T<Real>::type* ref_slot = nullptr) {
+                       const typename Vec4T<Real>::type* ref_slot = nullptr, Real* dw_out = nullptr) {
   constexpr bool HAS_PID = (CTRL == MDS_CTRL_LQR_OMEGA || CTRL == MDS_CTRL_LQR_YANK);
   constexpr int ORD = CTRL == MDS_CTRL_LQR_OMEGA ? 2 : 3;  // rollout_impl pairs the order-2 filter with LQR_OMEGA, order 3 with LQR_YANK
   Real u[4] = {Real(0), Real(0), Real(0), Real(0)};
@@ -606,7 +649,8 @@ MDS_DEV void ctrl_body(const DroneP<Real>& P, const RolloutP<Real>& Rc, const Ge
       }
       Real mh = Real(1e30);
       int it = 0;
-      int stt = cbf_filter_group<ORD, Real, NT>(P, C, S, Rc.obstacles, Rc.n_obs, g, N, NP, ag, F, unom, usafe, &mh, &it);
+      const bool dwash = (PhysSpec<SPEC>::physics(P) == MDS_PHYSICS_DYN_GND_DRAG_DW) && (N > 1);  // physics_core's condition
+      int stt = cbf_filter_group<ORD, Real, NT>(P, C, S, Rc.obstacles, Rc.n_obs, g, N, NP, ag, F, unom, usafe, &mh, &it, dw_out, dwash);
       if (g.valid) {
         ss.min_h = (float)mh;
         if (g.n == 0) {
@@ -773,9 +817,10 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
                                                                   int N_rt, int NP_rt) {
   extern __shared__ __align__(32) unsigned char smem_raw[];
   using R4 = typename Vec4T<Real>::type;
-  // downwash positions: with the CBF stage they live in the head of the environment's CBF block (idle during the physics; the
-  // stage's closing group sync orders the reuse), otherwise in a per-block array.  Every KB of shared memory the kernel does
-  // not take is L1 for its spill slots (L1 = 228 KB - shared memory in use).
+  // downwash positions (with the CBF stage only those of the sub-steps after the first: FUSE_DW below): with the CBF stage
+  // they live in the head of the environment's CBF block (idle during the physics; the stage's closing group sync orders the
+  // reuse), otherwise in a per-block array.  Every KB of shared memory the kernel does not take is L1 for its spill slots
+  // (L1 = 228 KB - shared memory in use).
   __shared__ R4 sm_pos[USE_CBF ? 1 : loop_block<Real>()];
   // fp32 stages the per-step read-mostly data (trajectory descriptor, rate-PID state) in shared memory for the launch;
   // fp64 does not: with the CBF stage's 91 KB that would leave one resident block per SM instead of two (0.41 vs 0.31 ms)
@@ -783,6 +828,7 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
   __shared__ __align__(16) typename TrajSpecT<Real>::spec sm_spec[(STAGE && !REFTAB) ? loop_block<Real>() : 1];
   __shared__ R4 sm_ref[REFTAB ? 3 * MDS_REF_STEPS * NT : 1];
   constexpr bool HAS_PID = (CTRL == MDS_CTRL_LQR_OMEGA || CTRL == MDS_CTRL_LQR_YANK);
+  constexpr bool FUSE_DW = USE_CBF && HAS_PID;  // the CBF stage runs (ctrl_body) and sums the downwash of the physics
   __shared__ R4 sm_pid_a[(STAGE && HAS_PID) ? loop_block<Real>() : 1];
   __shared__ typename Vec2T<Real>::type sm_pid_b[(STAGE && HAS_PID) ? loop_block<Real>() : 1];
   const PidP<Real> pid_s = STAGE ? PidP<Real>{sm_pid_a, sm_pid_b} : pid;
@@ -850,9 +896,10 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
       }
       StepStats ss = {0.f, 1e30f, 0, 0, 0, 0};
       M3<Real> R;
+      Real dw = Real(0);  // with the CBF stage: the downwash of the step's first physics sub-step, summed by the stage
       ctrl_body<Real, CTRL, USE_CBF, (NT < 0), SPEC, NT, REFTAB>(P, Rc, G, L, C, Dg, dst, S, pid_s, spec, segs, o, g, N, NP, t0 + (double)k * dt_ctrl,
                                                              rpm, ss, STAGE ? (int)threadIdx.x : g.d, HAS_PID ? &R : nullptr,  // the host plans form t exactly like this
-                                                             REFTAB ? sm_ref + 3 * (row * NT + g.n) : nullptr);
+                                                             REFTAB ? sm_ref + 3 * (row * NT + g.n) : nullptr, FUSE_DW ? &dw : nullptr);
       acc.err += ss.err; max_err = fmaxf(max_err, ss.err); acc.min_h = fminf(acc.min_h, ss.min_h);
       acc.qp_solves += ss.qp_solves; acc.qp_iters += ss.qp_iters; acc.qp_infeas += ss.qp_infeas + (ss.qp_cap << 16);
       Drone<Real> s;
@@ -864,7 +911,7 @@ __global__ void __launch_bounds__(loop_block<Real>(), MDS_LOOP_MINB) rollout_loo
         fx = {Real(0), Real(0), Real(0)};
         if (has_fx && g.valid) fx = {__ldg(fext + 3 * g.d), __ldg(fext + 3 * g.d + 1), __ldg(fext + 3 * g.d + 2)};
       }
-      o = physics_core<SPEC>(P, s, rpm, fx, env_pos, g, N, NP, HAS_PID ? &R : nullptr);
+      o = physics_core<SPEC>(P, s, rpm, fx, env_pos, g, N, NP, HAS_PID ? &R : nullptr, FUSE_DW ? &dw : nullptr);
       wb = s.w;
       if (Rc.write_obs_every > 0 && --log_countdown == 0) {
         if (g.valid && live) store_obs(log_slot, g.d, o, true);  // streaming stores: the log is write-once
