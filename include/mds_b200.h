@@ -409,6 +409,21 @@ int mds_learning_rollout_torque_f64(const MdsDroneParams* prm, const MdsRlsCfg* 
 int mds_care_gains_f32(int m, const double* q_diag, const double* r_diag, const float* theta_dev, float* K_dev, int* status_dev, int D, void* stream);
 int mds_care_gains_f64(int m, const double* q_diag, const double* r_diag, const double* theta_dev, double* K_dev, int* status_dev, int D, void* stream);
 
+/* compute_controller of the 12-dim model when Q couples robots 0 and 1 of every environment (decentralized_lqr.py:44-53,
+ * 300-317): the environment's Q is kron(I_N, diag(q_diag)) plus the cross block q_cross [m*m] (row-major, host array;
+ * Q[k][m + l] = Q[m + l][k] = q_cross[k*m + l], robot 0's state k against robot 1's state l), R = kron(I_N, diag(r_diag)).
+ * The environment's stabilising solution is block diagonal over the drones {0, 1}, {2}, ..., {N-1}: one warp solves each
+ * 24-state pair problem and each 12-state single problem in double.  theta_dev [(m+4)*m][D] planes -> K_dev the robot-coupled
+ * [N][4*m][D] planes that mds_dlqr_ctrl (coupled = 1) and mds_learning_rollout_torque read (entry (j, i*m + k, d = e*N + r) =
+ * K_e[4r + i][m j + k]); a solved drone's entries for source drones outside its problem are written as zeros.
+ * status_dev optional [D]: 0 ok, 1 the drone's problem has no stabilising solution found (its entries left untouched; both
+ * drones of a failed pair).  Refuses (MDS_ERR_ARG) m != 12, N outside [2, MDS_MAX_DRONES_PER_ENV], E < 1, null pointers,
+ * non-positive q or r, and a cross block for which the pair's Q is not positive semidefinite. */
+int mds_care_gains_coupled_f32(int m, const double* q_diag, const double* r_diag, const double* q_cross, const float* theta_dev, float* K_dev,
+                               int* status_dev, int E, int N, void* stream);
+int mds_care_gains_coupled_f64(int m, const double* q_diag, const double* r_diag, const double* q_cross, const double* theta_dev, double* K_dev,
+                               int* status_dev, int E, int N, void* stream);
+
 /* launch plan (a MdsRolloutCfg.stages value) that stages == 0 selects for E envs of N drones */
 int mds_rollout_plan(int E, int N);
 

@@ -112,6 +112,7 @@ _SIGS = {
     "mds_lowlevel": [_PRM, _I, _P, _P, PidState, _P, _I, _P],
     "mds_rls_update": [C.POINTER(RlsCfg), _P, _P, _P, _P, _P, _I, _P],
     "mds_care_gains": [_I, C.POINTER(_D), C.POINTER(_D), _P, _P, _P, _I, _P],
+    "mds_care_gains_coupled": [_I, C.POINTER(_D), C.POINTER(_D), C.POINTER(_D), _P, _P, _P, _I, _I, _P],
     "mds_error_state": [_PRM, _I, _P, _P, _P, _I, _P],
     "mds_state_feedback": [_I, _P, _P, _P, _P, _P, _I, _P],
     "mds_dlqr_ctrl": [_PRM, _I, _P, _I, _P, _P, _P, _P, PidState, _I, _I, _P],

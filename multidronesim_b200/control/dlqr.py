@@ -11,8 +11,11 @@ drone d at ``[k, d]`` -- so that one thread per drone reads and writes coalesced
   theta_update / theta_update2 / approx_theta_update : one launch of ``mds_rls_update`` for all E*N drones
   compute                                            : one launch of ``mds_dlqr_ctrl``
   compute_controller                                 : one launch of ``mds_care_gains`` (one warp per drone solves its Riccati
-                                                       equation) for diagonal per-drone weights; scipy on the host, like the
-                                                       reference, for the robot-coupled 12-dim case and non-diagonal weights
+                                                       equation) for diagonal per-drone weights; with ``solver="device"`` the
+                                                       robot-coupled 12-dim case through ``mds_care_gains_coupled`` (one warp
+                                                       per pair problem of robots 0 and 1, one per other drone); scipy on the
+                                                       host, like the reference, for non-diagonal weights and by default for
+                                                       the robot-coupled case
 """
 from __future__ import annotations
 
@@ -171,19 +174,64 @@ class _DecentralizedBase(BaseController):
         Block-diagonal Q, R (or ``force_diagonal``): one m x m problem per drone, K_d [4, m] -- solved ON DEVICE by
         ``mds_care_gains`` (one warp per drone, matrix sign function in double; <= 2e-12 of scipy's answer) when Q and R are
         diagonal, as all of the reference's Bryson weights are.  ``solver="host"`` forces the reference's own route
-        (scipy.linalg.solve_continuous_are per DISTINCT model, ~1 ms each); it is also what non-diagonal weights and the
-        robot-coupled Q of the 12-dim variant with N >= 2 (one mN x mN problem per environment, full K [4N, mN]) use.
-        ``self.care_status`` [D] (device, int32) after a device solve: 0 ok, 1 no stabilising solution (gain left as it was)."""
+        (scipy.linalg.solve_continuous_are per DISTINCT model, ~1 ms each); it is also what non-diagonal weights use.
+
+        The robot-coupled Q of the 12-dim variant with N >= 2 (one mN x mN problem per environment, full K [4N, mN]): by
+        default (``"auto"``) and with ``"host"`` scipy solves it per environment and ``self.K`` is the numpy [E, 4N, mN] gain.
+        ``solver="device"`` solves it ON DEVICE through ``mds_care_gains_coupled`` when the per-drone Q and R are diagonal and
+        the environment's Q is kron(I, Q_d) apart from a cross block between robots 0 and 1 (the reference's weights): the
+        stabilising solution is block diagonal over the drones {0, 1}, {2}, ..., {N-1}, so one 24-state problem per
+        environment and one 12-state problem per other drone give the whole gain.  ``self.K`` is then ``self.K_planes``, the
+        robot-coupled [N][4*m][D] planes (no host copy).  Any other coupling raises MdsError before anything runs.
+        ``self.care_status`` [D] (device, int32) after a device solve: 0 ok, 1 no stabilising solution (gain left as it was;
+        both drones of a failed pair)."""
         N = self.num_robots
         coupled = bool(self.COUPLED and N >= 2 and not force_diagonal)
         diag_w = np.count_nonzero(self.ind_Q - np.diag(np.diag(self.ind_Q))) == 0 and np.count_nonzero(self.ind_R - np.diag(np.diag(self.ind_R))) == 0
         if solver not in ("auto", "device", "host"):
             raise ValueError("solver must be 'auto', 'device' or 'host'")
-        if solver == "device" and (coupled or not diag_w):
+        if solver == "device" and coupled:
+            cross = self._pair_cross_block() if diag_w else None
+            if cross is None:
+                raise _lib.MdsError("the device Riccati solver takes diagonal per-drone Q and R, coupled at most through a cross block "
+                                    "between robots 0 and 1; use solver='host'")
+            return self._compute_controller_device_coupled(cross)
+        if solver == "device" and not diag_w:
             raise _lib.MdsError("the device Riccati solver takes diagonal, per-drone Q and R; use solver='host'")
         if solver != "host" and not coupled and diag_w:
             return self._compute_controller_device()
         return self._compute_controller_host(force_diagonal)
+
+    def _pair_cross_block(self):
+        """C [m, m] when ``_env_weights()`` is (kron(I, ind_Q), kron(I, ind_R)) apart from Q[:m, m:2m] = C and Q[m:2m, :m] = C';
+        None for any other coupling."""
+        Q, R = self._env_weights()
+        N, m = self.num_robots, self.m
+        Q0, R0 = np.kron(np.eye(N), self.ind_Q), np.kron(np.eye(N), self.ind_R)
+        if Q.shape != Q0.shape or R.shape != R0.shape or not np.array_equal(R, R0):
+            return None
+        C = np.array(Q[:m, m:2 * m], dtype=np.float64)
+        rest = np.array(Q, dtype=np.float64) - Q0
+        rest[:m, m:2 * m] -= C
+        rest[m:2 * m, :m] -= C.T
+        return C if not np.any(rest) else None
+
+    def _compute_controller_device_coupled(self, cross):
+        env = self.env
+        E, N, D, m = env.NUM_ENVS, self.num_robots, env.NUM_TOTAL, self.m
+        rows = N * self.n * m
+        K_planes = self.K_planes if self.K_planes.shape[0] == rows else torch.zeros(rows, D, device=env.device, dtype=env.dtype)
+        status = getattr(self, "care_status", None)
+        if status is None:
+            status = torch.zeros(D, device=env.device, dtype=torch.int32)
+        q = (_lib.C.c_double * m)(*np.diag(self.ind_Q).tolist())
+        r = (_lib.C.c_double * 4)(*np.diag(self.ind_R).tolist())
+        qx = (_lib.C.c_double * (m * m))(*cross.reshape(-1).tolist())
+        _lib.call("mds_care_gains_coupled", env.dtype, m, q, r, qx, _lib.ptr(self.theta_planes), _lib.ptr(K_planes), _lib.ptr(status), E, N,
+                  _lib.stream_ptr(env.device))
+        self.K_planes, self.care_status, self._coupled = K_planes, status, True
+        self.K = self.K_planes  # planes [N][4*m][D]: entry (j, i*m + k, e*N + r) = K_e[4r + i, m j + k]
+        return self.K
 
     def _compute_controller_device(self):
         env = self.env
@@ -203,7 +251,7 @@ class _DecentralizedBase(BaseController):
     def K_matrix(self, i=0, env_idx=0):
         """[4, m] gain of robot i in environment env_idx (uncoupled variants)."""
         if self._coupled:
-            raise _lib.MdsError("coupled gain: read self.K [E, 4N, mN]")
+            raise _lib.MdsError("coupled gain: read self.K_planes [N*4*m, D] (or self.K [E, 4N, mN] after the host solver)")
         return self.K_planes[:, self._drone(i, env_idx)].reshape(self.n, self.m).clone()
 
     def _compute_controller_host(self, force_diagonal=False):

@@ -44,6 +44,7 @@ static int cuda_fail(const char* what, cudaError_t e) {
 #include "mds_rollout.cuh"
 #include "mds_rollout_launch.cuh"
 #include "mds_learn_launch.cuh"
+#include "mds_care_launch.cuh"
 
 template <typename Real>
 __global__ void obs_from_state_kernel(DroneP<Real> P, StateP<Real> st, Real* __restrict__ obs, int D) {
@@ -547,6 +548,44 @@ static int care_impl(int m, const double* q, const double* r, const Real* theta,
   if (ae != cudaSuccess) return cuda_fail("care_gains: shared-memory opt-in", ae);
   return check_launch("care_gains");
 }
+// The robot-coupled solve (mds_care_tu.cu): Q = kron(I_N, diag(q)) plus the cross block q_cross [m][m] between robots 0 and 1
+template <typename Real>
+static int care_coupled_impl(int m, const double* q, const double* r, const double* q_cross, const Real* theta, Real* K, int* status, int E, int N,
+                             void* stream) {
+  MDS_REQUIRE(q && r && q_cross && theta && K, "care_gains_coupled: null pointer");
+  MDS_REQUIRE(m == 12, "care_gains_coupled: m must be 12 (the robot-coupled weights are the torque-level model's)");
+  MDS_REQUIRE(E >= 1 && N >= 2 && N <= MDS_MAX_DRONES_PER_ENV && (long long)E * N <= 0x7fffffffLL, "care_gains_coupled: bad E or N (N in [2, 32])");
+  CareCoupledP c;
+  for (int i = 0; i < 12; ++i) { MDS_REQUIRE(q[i] > 0.0, "care_gains_coupled: Q must be diagonal and positive"); c.sq[i] = sqrt(q[i]); }
+  for (int i = 0; i < 4; ++i) { MDS_REQUIRE(r[i] > 0.0, "care_gains_coupled: R must be diagonal and positive"); c.rinv[i] = 1.0 / r[i]; }
+  for (int k = 0; k < 12; ++k)
+    for (int l = 0; l < 12; ++l) {
+      MDS_REQUIRE(isfinite(q_cross[k * 12 + l]), "care_gains_coupled: q_cross must be finite");
+      c.cross[k * 12 + l] = q_cross[k * 12 + l] / (c.sq[k] * c.sq[l]);
+    }
+  // the pair's scaled Q~ = [[I, C], [C', I]] is positive semidefinite iff I - C'C is: Cholesky with a tolerance for the
+  // semidefinite case (a diagonal C needs |q_cross_kk| <= q_kk)
+  double S[12][12];
+  for (int k = 0; k < 12; ++k)
+    for (int l = 0; l < 12; ++l) {
+      double v = k == l ? 1.0 : 0.0;
+      for (int i = 0; i < 12; ++i) v -= c.cross[i * 12 + k] * c.cross[i * 12 + l];
+      S[k][l] = v;
+    }
+  const double tol = 1e-12;
+  for (int k = 0; k < 12; ++k) {
+    MDS_REQUIRE(S[k][k] >= -tol, "care_gains_coupled: the pair's Q is not positive semidefinite");
+    if (S[k][k] <= tol) {
+      for (int i = k + 1; i < 12; ++i) MDS_REQUIRE(fabs(S[i][k]) <= 1e-6, "care_gains_coupled: the pair's Q is not positive semidefinite");
+      continue;
+    }
+    for (int i = k + 1; i < 12; ++i)
+      for (int j = k + 1; j < 12; ++j) S[i][j] -= S[i][k] * S[k][j] / S[k][k];
+  }
+  const cudaError_t ae = launch_care_coupled<Real>(c, theta, K, status, E, N, (cudaStream_t)stream);
+  if (ae != cudaSuccess) return cuda_fail("care_gains_coupled: shared-memory opt-in", ae);
+  return check_launch("care_gains_coupled");
+}
 static bool lqr_variant_ok(int v) { return v == MDS_CTRL_LQR_TORQUE || v == MDS_CTRL_LQR_OMEGA || v == MDS_CTRL_LQR_YANK; }
 template <typename Real>
 static int error_state_impl(const MdsDroneParams* prm, int variant, const Real* obs, const Real* ref, Real* e, int D, void* stream) {
@@ -962,6 +1001,10 @@ int mds_cbf_num_rows(int order, int N, int n_obs) { return N * (N - 1) / 2 + 8 *
   }                                                                                                                                                \
   int mds_care_gains_##SUF(int m, const double* q, const double* r, const REAL* theta, REAL* K, int* status, int D, void* stream) {                 \
     return care_impl<REAL>(m, q, r, theta, K, status, D, stream);                                                                                  \
+  }                                                                                                                                                \
+  int mds_care_gains_coupled_##SUF(int m, const double* q, const double* r, const double* q_cross, const REAL* theta, REAL* K, int* status, int E, \
+                                   int N, void* stream) {                                                                                         \
+    return care_coupled_impl<REAL>(m, q, r, q_cross, theta, K, status, E, N, stream);                                                            \
   }                                                                                                                                                \
   int mds_state_feedback_##SUF(int variant, const REAL* K, const REAL* x, const REAL* xdes, REAL* e, REAL* u, int D, void* stream) {                \
     return state_feedback_impl<REAL>(variant, K, x, xdes, e, u, D, stream);                                                                        \
