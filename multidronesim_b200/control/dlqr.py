@@ -195,7 +195,7 @@ class _DecentralizedBase(BaseController):
             if cross is None:
                 raise _lib.MdsError("the device Riccati solver takes diagonal per-drone Q and R, coupled at most through a cross block "
                                     "between robots 0 and 1; use solver='host'")
-            return self._compute_controller_device_coupled(cross)
+            return self._compute_controller_device(cross)
         if solver == "device" and not diag_w:
             raise _lib.MdsError("the device Riccati solver takes diagonal, per-drone Q and R; use solver='host'")
         if solver != "host" and not coupled and diag_w:
@@ -216,36 +216,28 @@ class _DecentralizedBase(BaseController):
         rest[m:2 * m, :m] -= C.T
         return C if not np.any(rest) else None
 
-    def _compute_controller_device_coupled(self, cross):
+    def _compute_controller_device(self, cross=None):
+        """One device Riccati solve: per drone (``mds_care_gains``) or, given the pair's cross block ``cross`` [m, m],
+        robot-coupled (``mds_care_gains_coupled``).  K_planes and care_status are replaced only after the call succeeds."""
         env = self.env
         E, N, D, m = env.NUM_ENVS, self.num_robots, env.NUM_TOTAL, self.m
-        rows = N * self.n * m
+        coupled = cross is not None
+        rows = (N if coupled else 1) * self.n * m
         K_planes = self.K_planes if self.K_planes.shape[0] == rows else torch.zeros(rows, D, device=env.device, dtype=env.dtype)
         status = getattr(self, "care_status", None)
         if status is None:
             status = torch.zeros(D, device=env.device, dtype=torch.int32)
         q = (_lib.C.c_double * m)(*np.diag(self.ind_Q).tolist())
         r = (_lib.C.c_double * 4)(*np.diag(self.ind_R).tolist())
-        qx = (_lib.C.c_double * (m * m))(*cross.reshape(-1).tolist())
-        _lib.call("mds_care_gains_coupled", env.dtype, m, q, r, qx, _lib.ptr(self.theta_planes), _lib.ptr(K_planes), _lib.ptr(status), E, N,
-                  _lib.stream_ptr(env.device))
-        self.K_planes, self.care_status, self._coupled = K_planes, status, True
-        self.K = self.K_planes  # planes [N][4*m][D]: entry (j, i*m + k, e*N + r) = K_e[4r + i, m j + k]
-        return self.K
-
-    def _compute_controller_device(self):
-        env = self.env
-        D = env.NUM_TOTAL
-        self._coupled = False
-        if self.K_planes.shape[0] != self.n * self.m:
-            self.K_planes = torch.zeros(self.n * self.m, D, device=env.device, dtype=env.dtype)
-        if getattr(self, "care_status", None) is None:
-            self.care_status = torch.zeros(D, device=env.device, dtype=torch.int32)
-        q = (_lib.C.c_double * self.m)(*np.diag(self.ind_Q).tolist())
-        r = (_lib.C.c_double * 4)(*np.diag(self.ind_R).tolist())
-        _lib.call("mds_care_gains", env.dtype, self.m, q, r, _lib.ptr(self.theta_planes), _lib.ptr(self.K_planes), _lib.ptr(self.care_status), D,
-                  _lib.stream_ptr(env.device))
-        self.K = self.K_planes  # planes [4*m, D]; K_matrix(d) gives one drone's [4, m]
+        theta, K, st, stream = _lib.ptr(self.theta_planes), _lib.ptr(K_planes), _lib.ptr(status), _lib.stream_ptr(env.device)
+        if coupled:
+            qx = (_lib.C.c_double * (m * m))(*cross.reshape(-1).tolist())
+            _lib.call("mds_care_gains_coupled", env.dtype, m, q, r, qx, theta, K, st, E, N, stream)
+        else:
+            _lib.call("mds_care_gains", env.dtype, m, q, r, theta, K, st, D, stream)
+        self.K_planes, self.care_status, self._coupled = K_planes, status, coupled
+        # planes [4*m][D] (K_matrix(d) gives one drone's [4, m]) or, coupled, [N][4*m][D]: entry (j, i*m + k, e*N + r) = K_e[4r + i, m j + k]
+        self.K = self.K_planes
         return self.K
 
     def K_matrix(self, i=0, env_idx=0):

@@ -1,30 +1,42 @@
-// mds_care_tu.cu -- the Riccati solve of the 12-dim decentralised LQR when Q couples robots 0 and 1 of every environment
-// (decentralized_lqr.py:44-53: a cross block between their xy positions), and its launcher.
+// mds_care_tu.cu -- the batched continuous-time Riccati solve of the decentralised LQR, both kinds, and its launcher: one m x m
+// problem per drone (mds_care_gains), and the 12-dim case whose Q couples robots 0 and 1 of every environment
+// (mds_care_gains_coupled).
 //
-// A, B and R are block diagonal per drone and Q is kron(I_N, Q_d) apart from the cross block between robots 0 and 1, so the
-// block-diagonal X with blocks {0, 1}, {2}, ..., {N-1} satisfies the environment's Riccati equation block by block; its closed
-// loop is block diagonal and Hurwitz, so it is THE stabilising solution.  The 12N-state problem of an environment splits into
-// one 24-state pair problem (drones 0 and 1) and N - 2 independent 12-state problems; the gain is zero outside the blocks
-// {0, 1} x {0, 1} and {j} x {j}.  Both kinds run the method of care_gain_kernel (mds_sysid.cuh) in double, with state scaling
-// z = sqrt(diag Q) x (Q~ = I plus the scaled cross block in the pair problem), the determinant-scaled Newton iteration for the
-// matrix sign function of [[A~, -G~], [-Q~, -A~']], then W12 X~ = -(W11 + I), symmetrise, scale back, K = R^-1 B' X.
-// Results go straight to the robot-coupled [N][48][D] planes that mds_dlqr_ctrl (coupled = 1) and the fused learning
-// rollout read; a solved drone's entries for sources outside its problem are written as exact zeros.
+// compute_controller (decentralized_lqr_omega.py:185-204): K_d = R^-1 B_d' X_d with X_d the stabilising solution of
+// A'X + XA - X B R^-1 B' X + Q = 0 for every drone's learned (A_d, B_d) = theta_d.  The reference calls scipy
+// (solve_continuous_are: QZ on the balanced extended pencil) once per learning phase on the host; a swarm of distinct
+// learned models needs one solve per drone, so here ONE WARP solves one problem in shared memory, in double:
+//   * state scaling z = sqrt(Q) x (Q diagonal) -> Q~ = I, which equalises the Hamiltonian's blocks (the reference's
+//     Bryson weights span 1e-6 .. 1e6);
+//   * matrix sign function of H = [[A~, -G~], [-Q~, -A~']] by the determinant-scaled Newton iteration
+//     Z <- (c Z + (c Z)^-1) / 2, c = |det Z|^(-1/2n), each inverse a Gauss-Jordan sweep with partial pivoting over
+//     [Z | I]; 7-9 iterations to 1e-13;
+//   * X~ from W12 X~ = -(W11 + I) (W = sign H), symmetrised, scaled back, then K = R^-1 B' X.
+// Agreement with scipy on the reference's three parametrisations with perturbed / dense learned models: <= 2e-12 of max |K|.
+//
+// Robot-coupled Q (decentralized_lqr.py:44-53: a cross block between the xy positions of robots 0 and 1): A, B and R are block
+// diagonal per drone and Q is kron(I_N, Q_d) apart from that cross block, so the block-diagonal X with blocks {0, 1}, {2}, ...,
+// {N-1} satisfies the environment's Riccati equation block by block; its closed loop is block diagonal and Hurwitz, so it is
+// THE stabilising solution.  The 12N-state problem of an environment splits into one 24-state pair problem (drones 0 and 1,
+// Q~ = I plus the scaled cross block) and N - 2 independent 12-state problems; the gain is zero outside the blocks
+// {0, 1} x {0, 1} and {j} x {j}.  Results go straight to the robot-coupled [N][48][D] planes that mds_dlqr_ctrl (coupled = 1)
+// and the fused learning rollout read; a solved drone's entries for sources outside its problem are written as exact zeros.
+// The per-drone planes [4m][D] are that layout with a single source block (N = 1).
 #include "mds_care_launch.cuh"
 #include "mds_common.cuh"
 
 namespace mds {
 
-// S drones per problem: 1 (single) or 2 (pair).  One warp per problem; lane l owns the Hamiltonian rows l, l + 32 (48 rows of
-// the pair problem do not fit lane = row).  Shared memory per problem: Z [2n][2n], [Z | I] [2n][4n + 1] and B~ [n][4] doubles,
-// n = 12 S: 14 400 B (single; four problems per block, as care_gain_kernel) / 56 448 B (pair; one per block).
-template <int S> constexpr int care_cw_warps() { return S == 1 ? 4 : 1; }
-template <int S> constexpr int care_cw_doubles() { return (24 * S) * (24 * S) + (24 * S) * (48 * S + 1) + 12 * S * 4; }
+// S drones per problem: 1 (single) or 2 (pair).  One warp per problem; lane l owns the Hamiltonian rows l + 32 t (the 48 rows
+// of the pair problem do not fit lane = row).  Shared memory per problem: Z [2n][2n], [Z | I] [2n][4n + 1] and B~ [n][4]
+// doubles, n = M S: 14 400 B at M = 12 (single; four problems per block) / 56 448 B (pair; one per block).
+template <int S> constexpr int care_warps() { return S == 1 ? 4 : 1; }
+template <int M, int S> constexpr int care_doubles() { return (2 * M * S) * (2 * M * S) + (2 * M * S) * (4 * M * S + 1) + M * S * 4; }
 
 // Gauss-Jordan elimination with partial pivoting of the leading rows x rows block of a (row stride ld) to the identity, lane l
 // owning rows l + 32 t (t < R).  Columns left of the pivot are already zero in the rows that take part, so every sweep starts
 // at the pivot column.  Returns false on a vanishing pivot; *logdet += sum log |pivot|.
-template <int R> MDS_DEV bool warp_gauss_jordan_rows(double* a, int rows, int cols, int ld, int lane, double* logdet) {
+template <int R> MDS_DEV bool warp_gauss_jordan(double* a, int rows, int cols, int ld, int lane, double* logdet) {
   const unsigned full = 0xffffffffu;
   for (int k = 0; k < rows; ++k) {
     double best = -1.0;
@@ -64,45 +76,56 @@ template <int R> MDS_DEV bool warp_gauss_jordan_rows(double* a, int rows, int co
   return true;
 }
 
-// Problem p: S == 2 -> environment p, drones 0 and 1; S == 1 -> environment p / (N - 2), drone 2 + p % (N - 2).
-template <typename Real, int S>
-__global__ void __launch_bounds__(32 * care_cw_warps<S>()) care_coupled_kernel(CareCoupledP c, const Real* __restrict__ theta, Real* __restrict__ K,
-                                                                              int* __restrict__ status, int E, int N) {
-  constexpr int n = 12 * S, N2 = 2 * n, LD = 2 * N2 + 1, R = (N2 + 31) / 32, W = care_cw_warps<S>();
-  extern __shared__ __align__(16) unsigned char care_cw_smem[];
-  __shared__ double s_sq[12], s_rinv[4], s_cross[S == 2 ? 144 : 1];
+// M states per drone.  Problem p: S == 2 -> environment p, drones 0 and 1; S == 1 -> environment p / (N - first), drone
+// first + p % (N - first).  K is [N][4M][D], D = E N.
+// Register budget 72 (single) / 68 (pair): shared memory bounds residency (at most six 128-thread blocks per SM, at M = 9),
+// so neither costs occupancy.  Left to ptxas's own choice the M = 9, 10 kernels are held to 64 registers and the single
+// problems lose the schedule of the elimination sweep that loads a row's next element before storing the current one
+// (3 % slower at M = 12 on a B200); at 72 the fp64 pair kernel is 0.2 % slower than at 68.
+template <typename Real, int M, int S>
+__global__ void __maxnreg__(S == 1 ? 72 : 68) care_kernel(CareP c, const Real* __restrict__ theta, Real* __restrict__ K,
+                                                          int* __restrict__ status, int E, int N, int first) {
+  static_assert(S == 1 || M == 12, "the robot-coupled pair problem is the 12-dim model's");
+  constexpr int n = M * S, N2 = 2 * n, LD = 2 * N2 + 1, R = (N2 + 31) / 32, W = care_warps<S>();
+  extern __shared__ __align__(16) unsigned char care_smem[];
+  __shared__ double s_sq[M], s_rinv[4], s_cross[S == 2 ? M * M : 1];
   if (threadIdx.x == 0) {
 #pragma unroll
-    for (int i = 0; i < 12; ++i) s_sq[i] = c.sq[i];
+    for (int i = 0; i < M; ++i) s_sq[i] = c.sq[i];
 #pragma unroll
     for (int i = 0; i < 4; ++i) s_rinv[i] = c.rinv[i];
     if (S == 2)
-      for (int i = 0; i < 144; ++i) s_cross[i] = c.cross[i];
+      for (int i = 0; i < M * M; ++i) s_cross[i] = c.cross[i];
   }
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int per_env = S == 2 ? 1 : N - 2;
+  const int per_env = S == 2 ? 1 : N - first;
   const size_t p = (size_t)blockIdx.x * W + warp;
   if (p >= (size_t)E * per_env) return;  // whole warps leave together
-  const size_t e = p / per_env, D = (size_t)E * N;
-  const int n0 = S == 2 ? 0 : 2 + (int)(p % per_env);  // the problem's first drone in its environment
+  const size_t e = p / per_env;
+  const unsigned D = (unsigned)E * N;  // < 2^31 (the C ABI checks it); a 64-bit D costs the M = 9 kernels a spill
+  const int n0 = S == 2 ? 0 : first + (int)(p % per_env);  // the problem's first drone in its environment
   const size_t d0 = e * N + n0;
   const unsigned full = 0xffffffffu;
-  double* Z = reinterpret_cast<double*>(care_cw_smem) + (size_t)warp * care_cw_doubles<S>();
+  double* Z = reinterpret_cast<double*>(care_smem) + (size_t)warp * care_doubles<M, S>();
   double* Ag = Z + N2 * N2;
   double* Bs = Ag + N2 * LD;  // B~ [n][4] = sqrt(Q) B
-  // theta[i][j] of the problem's drone a: A[j][i] for i < 12, B[j][i-12] above
-  auto th = [&](int a, int i, int j) { return (double)theta[(size_t)(i * 12 + j) * D + d0 + a]; };
-  for (int s = lane; s < n; s += 32)
-    for (int i = 0; i < 4; ++i) Bs[s * 4 + i] = th(s / 12, 12 + i, s % 12) * s_sq[s % 12];
+  // theta[i][j] of the problem's drone a: A[j][i] for i < M, B[j][i-M] above
+  auto th = [&](int a, int i, int j) { return (double)theta[(size_t)(i * M + j) * D + d0 + a]; };
+  // state s of the problem: drone s / M within the problem (0 for S == 1), its state s % M
+  auto drone = [](int s) { return S == 1 ? 0 : s / M; };
+  for (int s = lane; s < n; s += 32) {
+    const int a = drone(s), k = s - a * M;
+    for (int i = 0; i < 4; ++i) Bs[s * 4 + i] = th(a, M + i, k) * s_sq[k];
+  }
   __syncwarp(full);
 #pragma unroll
   for (int t = 0; t < R; ++t) {
     const int row = lane + 32 * t;
     if (row < n) {  // rows [A~, -G~]: zero between the two drones of a pair
-      const int a = row / 12, k = row % 12;
+      const int a = drone(row), k = row - a * M;
       for (int cc = 0; cc < n; ++cc) {
-        const int b = cc / 12, l = cc % 12;
+        const int b = drone(cc), l = cc - b * M;
         double z = 0.0, g = 0.0;
         if (a == b) {
           z = th(a, l, k) * s_sq[k] / s_sq[l];
@@ -112,11 +135,11 @@ __global__ void __launch_bounds__(32 * care_cw_warps<S>()) care_coupled_kernel(C
         Z[row * N2 + n + cc] = -g;
       }
     } else if (row < N2) {  // rows [-Q~, -A~']
-      const int rr = row - n, a = rr / 12, k = rr % 12;
+      const int rr = row - n, a = drone(rr), k = rr - a * M;
       for (int cc = 0; cc < n; ++cc) {
-        const int b = cc / 12, l = cc % 12;
+        const int b = drone(cc), l = cc - b * M;
         double q = cc == rr ? 1.0 : 0.0;
-        if (S == 2 && a != b) q = a == 0 ? s_cross[k * 12 + l] : s_cross[l * 12 + k];
+        if (S == 2 && a != b) q = a == 0 ? s_cross[k * M + l] : s_cross[l * M + k];
         Z[row * N2 + cc] = -q;
         Z[row * N2 + n + cc] = a == b ? -th(a, k, l) * s_sq[l] / s_sq[k] : 0.0;
       }
@@ -134,7 +157,7 @@ __global__ void __launch_bounds__(32 * care_cw_warps<S>()) care_coupled_kernel(C
     }
     __syncwarp(full);
     double logdet = 0.0;
-    if (!warp_gauss_jordan_rows<R>(Ag, N2, 2 * N2, LD, lane, &logdet)) { ok = false; break; }
+    if (!warp_gauss_jordan<R>(Ag, N2, 2 * N2, LD, lane, &logdet)) { ok = false; break; }
     const double sc = exp(-logdet / (double)N2), isc = 1.0 / sc;
     double diff = 0.0, mx = 0.0;
 #pragma unroll
@@ -160,23 +183,23 @@ __global__ void __launch_bounds__(32 * care_cw_warps<S>()) care_coupled_kernel(C
       }
     __syncwarp(full);
     double ld = 0.0;
-    ok = warp_gauss_jordan_rows<1>(Ag, n, 2 * n, LD2, lane, &ld);
+    ok = warp_gauss_jordan<1>(Ag, n, 2 * n, LD2, lane, &ld);
     if (ok && lane < n) {  // column `lane` of the problem's K = R^-1 B' X, X[r][c] = sq_r (X~[r][c] + X~[c][r]) / 2 sq_c
-      const int b = lane / 12, l = lane % 12;
+      const int b = drone(lane), l = lane - b * M;
       for (int a = 0; a < S; ++a) {  // drone a's four rows, source drone b, its state l
         double kc[4] = {0.0, 0.0, 0.0, 0.0};
-        for (int k = 0; k < 12; ++k) {
-          const int r = 12 * a + k;
+        for (int k = 0; k < M; ++k) {
+          const int r = M * a + k;
           const double x = 0.5 * (Ag[r * LD2 + n + lane] + Ag[lane * LD2 + n + r]) * s_sq[l];  // times sq_r below, inside B~
           for (int i = 0; i < 4; ++i) kc[i] += Bs[r * 4 + i] * x;
         }
-        for (int i = 0; i < 4; ++i) K[(size_t)((n0 + b) * 48 + i * 12 + l) * D + d0 + a] = (Real)(s_rinv[i] * kc[i]);
+        for (int i = 0; i < 4; ++i) K[(size_t)((n0 + b) * 4 * M + i * M + l) * D + d0 + a] = (Real)(s_rinv[i] * kc[i]);
       }
     }
-    if (ok)  // the entries of the other source drones: plane (j * 48 + i * 12 + k), j outside the problem
+    if (ok)  // the entries of the other source drones: plane (j * 4M + i * M + k), j outside the problem
       for (int a = 0; a < S; ++a)
-        for (int q = lane; q < N * 48; q += 32)
-          if (q < n0 * 48 || q >= (n0 + S) * 48) K[(size_t)q * D + d0 + a] = Real(0);
+        for (int q = lane; q < N * 4 * M; q += 32)
+          if (q < n0 * 4 * M || q >= (n0 + S) * 4 * M) K[(size_t)q * D + d0 + a] = Real(0);
   } else {
     ok = false;
   }
@@ -184,24 +207,31 @@ __global__ void __launch_bounds__(32 * care_cw_warps<S>()) care_coupled_kernel(C
     for (int a = 0; a < S; ++a) status[d0 + a] = ok ? 0 : 1;
 }
 
-template <typename Real, int S>
-static cudaError_t launch_care_problems(const CareCoupledP& c, const Real* theta, Real* K, int* status, int E, int N, size_t problems, cudaStream_t cs) {
-  constexpr int W = care_cw_warps<S>();
-  const size_t smem = (size_t)care_cw_doubles<S>() * W * sizeof(double);
-  const cudaError_t ae = cudaFuncSetAttribute(care_coupled_kernel<Real, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+template <typename Real, int M, int S>
+static cudaError_t launch_care_problems(const CareP& c, const Real* theta, Real* K, int* status, int E, int N, int first, cudaStream_t cs) {
+  constexpr int W = care_warps<S>();
+  const size_t problems = (size_t)E * (S == 2 ? 1 : N - first);
+  const size_t smem = (size_t)care_doubles<M, S>() * W * sizeof(double);
+  const cudaError_t ae = cudaFuncSetAttribute(care_kernel<Real, M, S>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (ae != cudaSuccess) return ae;
-  care_coupled_kernel<Real, S><<<(unsigned)((problems + W - 1) / W), 32 * W, smem, cs>>>(c, theta, K, status, E, N);
+  care_kernel<Real, M, S><<<(unsigned)((problems + W - 1) / W), 32 * W, smem, cs>>>(c, theta, K, status, E, N, first);
   return cudaSuccess;
 }
 
 }  // namespace mds
 
 template <typename Real>
-cudaError_t launch_care_coupled(const mds::CareCoupledP& c, const Real* theta, Real* K, int* status, int E, int N, cudaStream_t cs) {
-  cudaError_t e = mds::launch_care_problems<Real, 2>(c, theta, K, status, E, N, (size_t)E, cs);
-  if (e == cudaSuccess && N > 2) e = mds::launch_care_problems<Real, 1>(c, theta, K, status, E, N, (size_t)E * (N - 2), cs);
-  return e;
+cudaError_t launch_care(const mds::CareP& c, int m, bool coupled, const Real* theta, Real* K, int* status, int E, int N, cudaStream_t cs) {
+  using namespace mds;
+  if (coupled) {
+    cudaError_t e = launch_care_problems<Real, 12, 2>(c, theta, K, status, E, N, 0, cs);
+    if (e == cudaSuccess && N > 2) e = launch_care_problems<Real, 12, 1>(c, theta, K, status, E, N, 2, cs);
+    return e;
+  }
+  if (m == 9) return launch_care_problems<Real, 9, 1>(c, theta, K, status, E, N, 0, cs);
+  if (m == 10) return launch_care_problems<Real, 10, 1>(c, theta, K, status, E, N, 0, cs);
+  return launch_care_problems<Real, 12, 1>(c, theta, K, status, E, N, 0, cs);
 }
 
-template cudaError_t launch_care_coupled<float>(const mds::CareCoupledP&, const float*, float*, int*, int, int, cudaStream_t);
-template cudaError_t launch_care_coupled<double>(const mds::CareCoupledP&, const double*, double*, int*, int, int, cudaStream_t);
+template cudaError_t launch_care<float>(const mds::CareP&, int, bool, const float*, float*, int*, int, int, cudaStream_t);
+template cudaError_t launch_care<double>(const mds::CareP&, int, bool, const double*, double*, int*, int, int, cudaStream_t);

@@ -524,40 +524,37 @@ static int rls_impl(const MdsRlsCfg* cfg, const Real* phi, const Real* xtp1, Rea
   if (ae != cudaSuccess) return cuda_fail("rls_update: shared-memory opt-in", ae);
   return check_launch("rls_update");
 }
+// The weights of both Riccati solves (mds_care_tu.cu): diagonal Q [m] and R [4], every entry positive; c gets sqrt(q) and 1 / r.
+static int care_weights(const char* what, int m, const double* q, const double* r, CareP* c) {
+  for (int i = 0; i < m; ++i) {
+    if (!(q[i] > 0.0)) return fail(MDS_ERR_ARG, "%s: Q must be diagonal and positive", what);
+    c->sq[i] = sqrt(q[i]);
+  }
+  for (int i = 0; i < 4; ++i) {
+    if (!(r[i] > 0.0)) return fail(MDS_ERR_ARG, "%s: R must be diagonal and positive", what);
+    c->rinv[i] = 1.0 / r[i];
+  }
+  return MDS_OK;
+}
 template <typename Real>
 static int care_impl(int m, const double* q, const double* r, const Real* theta, Real* K, int* status, int D, void* stream) {
   MDS_REQUIRE(q && r && theta && K && D > 0, "care_gains: bad argument");
   MDS_REQUIRE(m == 9 || m == 10 || m == 12, "care_gains: m must be 9, 10 or 12");
-  CareP c;
-  for (int i = 0; i < 12; ++i) c.sq[i] = 1.0;
-  for (int i = 0; i < m; ++i) { MDS_REQUIRE(q[i] > 0.0, "care_gains: Q must be diagonal and positive"); c.sq[i] = sqrt(q[i]); }
-  for (int i = 0; i < 4; ++i) { MDS_REQUIRE(r[i] > 0.0, "care_gains: R must be diagonal and positive"); c.rinv[i] = 1.0 / r[i]; }
-  const int blocks = (D + MDS_CARE_WARPS - 1) / MDS_CARE_WARPS;
-  cudaStream_t cs = (cudaStream_t)stream;
-  cudaError_t ae = cudaSuccess;
-#define MDS_LAUNCH_CARE(MM)                                                                                        \
-  do {                                                                                                             \
-    const size_t smem = (size_t)care_doubles_per_warp<MM>() * MDS_CARE_WARPS * sizeof(double);                     \
-    ae = cudaFuncSetAttribute(care_gain_kernel<Real, MM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-    if (ae == cudaSuccess) care_gain_kernel<Real, MM><<<blocks, 32 * MDS_CARE_WARPS, smem, cs>>>(c, theta, K, status, D); \
-  } while (0)
-  if (m == 9) MDS_LAUNCH_CARE(9);
-  else if (m == 10) MDS_LAUNCH_CARE(10);
-  else MDS_LAUNCH_CARE(12);
-#undef MDS_LAUNCH_CARE
+  CareP c{};
+  if (const int rc = care_weights("care_gains", m, q, r, &c)) return rc;
+  const cudaError_t ae = launch_care<Real>(c, m, false, theta, K, status, D, 1, (cudaStream_t)stream);
   if (ae != cudaSuccess) return cuda_fail("care_gains: shared-memory opt-in", ae);
   return check_launch("care_gains");
 }
-// The robot-coupled solve (mds_care_tu.cu): Q = kron(I_N, diag(q)) plus the cross block q_cross [m][m] between robots 0 and 1
+// The robot-coupled solve: Q = kron(I_N, diag(q)) plus the cross block q_cross [m][m] between robots 0 and 1
 template <typename Real>
 static int care_coupled_impl(int m, const double* q, const double* r, const double* q_cross, const Real* theta, Real* K, int* status, int E, int N,
                              void* stream) {
   MDS_REQUIRE(q && r && q_cross && theta && K, "care_gains_coupled: null pointer");
   MDS_REQUIRE(m == 12, "care_gains_coupled: m must be 12 (the robot-coupled weights are the torque-level model's)");
   MDS_REQUIRE(E >= 1 && N >= 2 && N <= MDS_MAX_DRONES_PER_ENV && (long long)E * N <= 0x7fffffffLL, "care_gains_coupled: bad E or N (N in [2, 32])");
-  CareCoupledP c;
-  for (int i = 0; i < 12; ++i) { MDS_REQUIRE(q[i] > 0.0, "care_gains_coupled: Q must be diagonal and positive"); c.sq[i] = sqrt(q[i]); }
-  for (int i = 0; i < 4; ++i) { MDS_REQUIRE(r[i] > 0.0, "care_gains_coupled: R must be diagonal and positive"); c.rinv[i] = 1.0 / r[i]; }
+  CareP c{};
+  if (const int rc = care_weights("care_gains_coupled", m, q, r, &c)) return rc;
   for (int k = 0; k < 12; ++k)
     for (int l = 0; l < 12; ++l) {
       MDS_REQUIRE(isfinite(q_cross[k * 12 + l]), "care_gains_coupled: q_cross must be finite");
@@ -582,7 +579,7 @@ static int care_coupled_impl(int m, const double* q, const double* r, const doub
     for (int i = k + 1; i < 12; ++i)
       for (int j = k + 1; j < 12; ++j) S[i][j] -= S[i][k] * S[k][j] / S[k][k];
   }
-  const cudaError_t ae = launch_care_coupled<Real>(c, theta, K, status, E, N, (cudaStream_t)stream);
+  const cudaError_t ae = launch_care<Real>(c, m, true, theta, K, status, E, N, (cudaStream_t)stream);
   if (ae != cudaSuccess) return cuda_fail("care_gains_coupled: shared-memory opt-in", ae);
   return check_launch("care_gains_coupled");
 }

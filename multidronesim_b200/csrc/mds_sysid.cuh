@@ -301,141 +301,3 @@ __global__ void __launch_bounds__(rls_threads<Real, M>()) rls_update_kernel(RlsP
 }
 
 }  // namespace mds
-
-// ================================================================== batched continuous-time Riccati solve
-// compute_controller (decentralized_lqr_omega.py:185-204): K_d = R^-1 B_d' X_d with X_d the stabilising solution of
-// A'X + XA - X B R^-1 B' X + Q = 0 for every drone's learned (A_d, B_d) = theta_d.  The reference calls scipy
-// (solve_continuous_are: QZ on the balanced extended pencil) once per learning phase on the host; a swarm of distinct
-// learned models needs one solve per drone, so here ONE WARP solves one drone's equation in shared memory, in double:
-//   * state scaling z = sqrt(Q) x (Q diagonal) -> Q~ = I, which equalises the Hamiltonian's blocks (the reference's
-//     Bryson weights span 1e-6 .. 1e6);
-//   * matrix sign function of H = [[A~, -G~], [-I, -A~']] by the determinant-scaled Newton iteration
-//     Z <- (c Z + (c Z)^-1) / 2, c = |det Z|^(-1/2m), each inverse a Gauss-Jordan sweep with partial pivoting over
-//     [Z | I] (lane = row); 7-9 iterations to 1e-13;
-//   * X~ from W12 X~ = -(W11 + I) (W = sign H), symmetrised, scaled back, then K = R^-1 B' X.
-// Agreement with scipy on the reference's three parametrisations with perturbed / dense learned models: <= 2e-12 of max |K|.
-namespace mds {
-
-struct CareP {
-  double sq[12];    // sqrt(q_ii)
-  double rinv[4];   // 1 / r_ii
-};
-
-// Gauss-Jordan elimination with partial pivoting on the rows x cols matrix a (row stride ld, rows <= 32, lane = row) until
-// its leading rows x rows block is the identity.  Returns false on a vanishing pivot; *logdet += sum log |pivot|.
-MDS_DEV bool warp_gauss_jordan(double* a, int rows, int cols, int ld, int lane, double* logdet) {
-  const unsigned full = 0xffffffffu;
-  for (int k = 0; k < rows; ++k) {
-    double best = (lane >= k && lane < rows) ? fabs(a[lane * ld + k]) : -1.0;
-    int who = lane;
-    for (int off = 16; off > 0; off >>= 1) {
-      const double ob = __shfl_xor_sync(full, best, off);
-      const int ow = __shfl_xor_sync(full, who, off);
-      if (ob > best || (ob == best && ow < who)) { best = ob; who = ow; }
-    }
-    if (!(best > 1e-300)) return false;
-    *logdet += log(best);
-    if (who != k)
-      for (int c = lane; c < cols; c += 32) { const double t = a[k * ld + c]; a[k * ld + c] = a[who * ld + c]; a[who * ld + c] = t; }
-    __syncwarp(full);
-    const double inv = 1.0 / a[k * ld + k];
-    __syncwarp(full);
-    for (int c = lane; c < cols; c += 32) a[k * ld + c] *= inv;
-    __syncwarp(full);
-    if (lane < rows && lane != k) {
-      const double f = a[lane * ld + k];
-      for (int c = 0; c < cols; ++c) a[lane * ld + c] -= f * a[k * ld + c];
-    }
-    __syncwarp(full);
-  }
-  return true;
-}
-
-#define MDS_CARE_WARPS 4
-template <int M> constexpr int care_doubles_per_warp() { return (2 * M) * (2 * M) + (2 * M) * (4 * M + 1) + M * 4; }
-
-template <typename Real, int M>
-__global__ void __launch_bounds__(32 * MDS_CARE_WARPS) care_gain_kernel(CareP c, const Real* __restrict__ theta, Real* __restrict__ K,
-                                                                        int* __restrict__ status, int D_) {
-  constexpr int N2 = 2 * M, LD = 2 * N2 + 1;
-  extern __shared__ __align__(16) unsigned char care_smem[];
-  __shared__ double s_sq[12], s_rinv[4];
-  if (threadIdx.x == 0) {
-#pragma unroll
-    for (int i = 0; i < M; ++i) s_sq[i] = c.sq[i];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) s_rinv[i] = c.rinv[i];
-  }
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const size_t d = (size_t)blockIdx.x * MDS_CARE_WARPS + warp, D = (size_t)D_;
-  if (d >= D) return;  // whole warps leave together
-  const unsigned full = 0xffffffffu;
-  double* Z = reinterpret_cast<double*>(care_smem) + (size_t)warp * care_doubles_per_warp<M>();
-  double* Ag = Z + N2 * N2;
-  double* Bs = Ag + N2 * LD;  // B~ [M][4] = sqrt(Q) B
-  auto th = [&](int i, int j) { return (double)theta[(size_t)(i * M + j) * D + d]; };  // theta[i][j]: A[j][i] for i < M, B[j][i-M] above
-  if (lane < M)
-    for (int k = 0; k < 4; ++k) Bs[lane * 4 + k] = th(M + k, lane) * s_sq[lane];
-  __syncwarp(full);
-  if (lane < M) {  // rows [A~, -G~]
-    const int r = lane;
-    for (int cc = 0; cc < M; ++cc) {
-      Z[r * N2 + cc] = th(cc, r) * s_sq[r] / s_sq[cc];
-      double g = 0.0;
-      for (int k = 0; k < 4; ++k) g += Bs[r * 4 + k] * s_rinv[k] * Bs[cc * 4 + k];
-      Z[r * N2 + M + cc] = -g;
-    }
-  } else if (lane < N2) {  // rows [-I, -A~']
-    const int r = lane - M;
-    for (int cc = 0; cc < M; ++cc) {
-      Z[lane * N2 + cc] = cc == r ? -1.0 : 0.0;
-      Z[lane * N2 + M + cc] = -th(r, cc) * s_sq[cc] / s_sq[r];
-    }
-  }
-  __syncwarp(full);
-  bool ok = true;
-  int it = 0;
-  for (; it < 60; ++it) {
-    if (lane < N2)
-      for (int cc = 0; cc < N2; ++cc) { Ag[lane * LD + cc] = Z[lane * N2 + cc]; Ag[lane * LD + N2 + cc] = cc == lane ? 1.0 : 0.0; }
-    __syncwarp(full);
-    double logdet = 0.0;
-    if (!warp_gauss_jordan(Ag, N2, 2 * N2, LD, lane, &logdet)) { ok = false; break; }
-    const double sc = exp(-logdet / (double)N2), isc = 1.0 / sc;
-    double diff = 0.0, mx = 0.0;
-    if (lane < N2)
-      for (int cc = 0; cc < N2; ++cc) {
-        const double z = Z[lane * N2 + cc], zn = 0.5 * (sc * z + isc * Ag[lane * LD + N2 + cc]);
-        diff = fmax(diff, fabs(zn - z)); mx = fmax(mx, fabs(zn));
-        Z[lane * N2 + cc] = zn;
-      }
-    for (int off = 16; off > 0; off >>= 1) { diff = fmax(diff, __shfl_xor_sync(full, diff, off)); mx = fmax(mx, __shfl_xor_sync(full, mx, off)); }
-    __syncwarp(full);
-    if (diff <= 1e-13 * mx) break;
-  }
-  if (ok && it < 60) {  // W12 X~ = -(W11 + I)
-    constexpr int LD2 = 2 * M + 1;
-    if (lane < M)
-      for (int cc = 0; cc < M; ++cc) {
-        Ag[lane * LD2 + cc] = Z[lane * N2 + M + cc];
-        Ag[lane * LD2 + M + cc] = -(Z[lane * N2 + cc] + (cc == lane ? 1.0 : 0.0));
-      }
-    __syncwarp(full);
-    double ld = 0.0;
-    ok = warp_gauss_jordan(Ag, M, 2 * M, LD2, lane, &ld);
-    if (ok && lane < M) {  // column `lane` of K = R^-1 B' X, X[r][c] = sq_r (X~[r][c] + X~[c][r]) / 2 sq_c
-      double kc[4] = {0.0, 0.0, 0.0, 0.0};
-      for (int r = 0; r < M; ++r) {
-        const double x = 0.5 * (Ag[r * LD2 + M + lane] + Ag[lane * LD2 + M + r]) * s_sq[lane];  // times sq_r below, inside B~
-        for (int i = 0; i < 4; ++i) kc[i] += Bs[r * 4 + i] * x;
-      }
-      for (int i = 0; i < 4; ++i) K[(size_t)(i * M + lane) * D + d] = (Real)(s_rinv[i] * kc[i]);
-    }
-  } else {
-    ok = false;
-  }
-  if (lane == 0 && status) status[d] = ok ? 0 : 1;
-}
-
-}  // namespace mds

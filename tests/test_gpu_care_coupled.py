@@ -1,7 +1,7 @@
 """mds_care_gains_coupled / DecentralizedLQR.compute_controller(solver="device") with the robot-coupled Q of the 12-dim model
 (decentralized_lqr.py:44-53): the device gain against the full 12N-state scipy solve of every environment, a structured scipy
 reference at N = 32, the reference's own coupled gain, failure reporting, the certainty-equivalence loop against the host
-solver, and the refusals (the C-ABI ones without a GPU)."""
+solver, and the refusals (the C-ABI ones, of mds_care_gains too, without a GPU)."""
 import ctypes
 
 import numpy as np
@@ -229,8 +229,8 @@ def test_coupled_refusals(case, lib_built):
 
 
 def test_coupled_c_argument_errors_do_not_need_a_gpu(lib_built):
-    """mds_care_gains_coupled validates every argument before it launches anything (the dummy device pointers are never
-    touched); every message starts with "care_gains_coupled: "."""
+    """mds_care_gains_coupled and mds_care_gains validate every argument before they launch anything (the dummy device
+    pointers are never touched); every message starts with "care_gains_coupled: " or "care_gains: "."""
     p = ctypes.c_void_p(64)
     arr = lambda vals: (ctypes.c_double * len(vals))(*vals)
     q = [1 / (np.pi / 10) ** 2] * 2 + [1 / (np.pi / 20) ** 2] + [4.0] * 3 + [1 / .15 ** 2] * 3 + [400.0] * 3
@@ -266,3 +266,27 @@ def test_coupled_c_argument_errors_do_not_need_a_gpu(lib_built):
         rc = call(**kw)
         e = lib_built.mds_last_error()
         assert rc == -1 and e.startswith(b"care_gains_coupled: ") and msg in e, (kw, e)
+
+    g32, g64 = lib_built.mds_care_gains_f32, lib_built.mds_care_gains_f64
+
+    def call_per_drone(m=9, qq=q, rr=r, theta=p, K=p, D=6, fn=g32):
+        return fn(m, arr(qq[:m]) if qq is not None else None, arr(rr), theta, K, None, D, None)
+
+    cases = [
+        (dict(m=11), b"m must be 9, 10 or 12"),
+        (dict(m=13, fn=g64), b"m must be 9, 10 or 12"),
+        (dict(m=8, fn=g64), b"m must be 9, 10 or 12"),
+        (dict(theta=None), b"bad argument"),
+        (dict(K=None, fn=g64), b"bad argument"),
+        (dict(qq=None), b"bad argument"),
+        (dict(D=0), b"bad argument"),
+        (dict(D=-4, fn=g64), b"bad argument"),
+        (dict(qq=q[:8] + [0.0]), b"Q must be diagonal and positive"),
+        (dict(m=10, qq=q[:9] + [float("nan")], fn=g64), b"Q must be diagonal and positive"),
+        (dict(m=12, qq=q[:11] + [-1.0]), b"Q must be diagonal and positive"),
+        (dict(rr=[1.0, 0.0, 1.0, 1.0], fn=g64), b"R must be diagonal and positive"),
+    ]
+    for kw, msg in cases:
+        rc = call_per_drone(**kw)
+        e = lib_built.mds_last_error()
+        assert rc == -1 and e.startswith(b"care_gains: ") and msg in e, (kw, e)
